@@ -1,8 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: 2-opt moves evaluated per second at n = 10 000.
 
-Contract (task prompt, section 4): `python bench.py --gpus N --steps K --warmup W` prints ONE JSON
-line on rank 0.
+`python bench.py --gpus N --steps K --warmup W` prints ONE JSON line on rank 0; exactly K steps
+are timed, after W (at least 3) untimed warm-up steps.  `--dump-outputs DIR` also writes what the
+timed path returned after its last step (the tour and the move that step applied) as DIR/*.npy, so
+that two builds can be compared output for output: the inputs depend on the arguments only.
 
 Workload (BASELINE.json configs[2], the config the metric is quoted on): 10 000 cities on the
 DIMACS-style 10^6 integer grid (splitmix64, seed 10000), TSPLIB nint distances, the int32
@@ -132,14 +134,13 @@ def bench_config(args, world: int) -> dict:
         "l2": (f"inputs larger than L2 ({4 * n * ld / 1e6:.0f} MB matrix, {4 * pairs_per_scan(n) / 1e6:.0f} MB read per "
                "scan, L2 126 MB); no flush") if args.path == "matrix" else
               "compute-bound path: 16 B per city of tour-ordered points, L2 state irrelevant",
-        "timed_region": f"chunks of {args.steps} steps, each after {args.warmup} untimed warm-up steps, repeated until "
-                        f">= {MIN_TIMED_MS:.0f} ms are timed; ms_per_step is the median chunk / {args.steps}",
+        "timed_region": f"{args.steps} steps after {args.warmup} untimed warm-up steps; ms_per_step is the timed "
+                        f"time / {args.steps}",
         "parallelism": f"independent instances x{world} (seed + rank), no data-path collective; the partitioned "
                        "cases (configs 4 and 5) are under `partitioned`",
     }
 
 
-MIN_TIMED_MS = 50.0   # a 20-step chunk is < 1 ms: repeat it until this much device time has been timed
 # an NN tour converges after ~1500 (10k) / ~170 (1k) moves: start a fresh session before that
 SESSION_CAPS = {"n10k": 1400, "n1k": 150, "n100k": 4000}
 SCAN_REPS = 200  # scan-kernel launches averaged for the roofline, whatever --steps is
@@ -276,6 +277,15 @@ def cpu_scan_rate(n: int, seed: int, path: str, dist: str, threads: int, budget_
     return scans * pairs_per_scan(n) / dt, scans, dt
 
 
+def dump_outputs(out_dir: str, tour, move) -> None:
+    """What a caller of the timed path receives after its last step, as float64 .npy files: the tour
+    (city indices in tour order) and the move that step applied, (delta, i, j); empty when the tour
+    had no improving move left."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "tour.npy"), np.asarray(tour, dtype=np.float64))
+    np.save(os.path.join(out_dir, "last_move.npy"), np.array(move[:3] if move else [], dtype=np.float64))
+
+
 def run_reference(args, rank: int, world: int):
     """--impl reference: the CPU port of the same step (scan + apply), all host threads."""
     if rank != 0:
@@ -284,26 +294,21 @@ def run_reference(args, rank: int, world: int):
     threads = os.cpu_count() or 1
     O, P = oracle_problem(n, seed, args.path, args.dist)
     tour = O.nn_tour(P, 3).copy()
-    budget = 150.0
-    done, t_all = 0, 0.0
-    t_start = time.perf_counter()
+    t_all = 0.0
     for k in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         mv = O.two_opt_best_scan(P, tour, nthreads=threads)
         if mv is not None:
             tour = O.swap_2opt(tour, mv[1] + 1, mv[2])
-        dt = time.perf_counter() - t0
         if k >= args.warmup:
-            done += 1
-            t_all += dt
-        if time.perf_counter() - t_start > budget and done >= 1:
-            break
-    value = done * pairs_per_scan(n) / t_all
-    sample = (f"{done} of {args.steps} requested full scan+apply steps of the n={n} workload "
-              f"(time-boxed to {budget:.0f} s)")
+            t_all += time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tour, mv)
+    value = args.steps * pairs_per_scan(n) / t_all
+    sample = f"{args.steps} full scan+apply steps of the n={n} workload"
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
-        "steps": done, "warmup": args.warmup, "ms_per_step": 1e3 * t_all / done, "higher_is_better": True,
+        "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * t_all / args.steps, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "int32" if args.dist == "nint" else "f32",
         "data": "synthetic",
         "config": bench_config(args, world),
@@ -484,74 +489,47 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     start = prob.nn_tour(3)  # the reference's `nn,2opt` pipeline
     path = paths[args.path]
 
-    # --- device-resident timing.  One CHUNK = exactly K timed steps after W untimed warm-up steps,
-    #     bracketed by barrier + synchronize on both sides and timed with CUDA events on the library's
-    #     stream.  A 20-step chunk lasts < 1 ms -- too short for NVML to sample and dominated by clock
-    #     ramp-up -- so the chunk is repeated (same session while the tour has moves left, else a fresh
-    #     one) until >= MIN_TIMED_MS of device time has been timed; the reported step time is the
-    #     MEDIAN chunk (max over ranks per chunk) / K.
+    # --- device-resident timing: exactly K = --steps timed steps, each stretch of them after W untimed
+    #     warm-up steps, bracketed by barrier + synchronize on both sides and timed with CUDA events on
+    #     the library's stream.  A tour runs out of improving moves after about SESSION_CAPS steps, so
+    #     a K larger than that is timed in pieces, each on a fresh session from the same start tour.
+    #     The reported step time is the timed device time (max over ranks) / K.
     cap = SESSION_CAPS[args.workload]
     sampler = ClockSampler(local_rank)
-    state = {"sess": None, "used": 0}
-
-    def session_for(steps_needed):
-        if state["sess"] is None or state["used"] + steps_needed > cap:
-            if state["sess"] is not None:
-                state["sess"].close()
-            state["sess"], state["used"] = prob.session(T.ALGO_TWO_OPT_BEST, start, path), 0
-        state["used"] += steps_needed
-        return state["sess"]
-
-    def timed_chunk():
-        """K timed steps (in pieces when K exceeds what one tour can supply); returns (ms, launches)."""
-        ms_c, launches_c, left = 0.0, 0, args.steps
-        while left > 0:
-            k = min(left, max(1, cap - args.warmup))
-            sess = session_for(args.warmup + k)
-            sess.enqueue(args.warmup)
-            barrier()
-            if rank == 0:
-                sampler.start()
-            l0 = ctx.launches
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            sess.enqueue(k)
-            e1.record()
-            barrier()
-            if rank == 0:
-                sampler.pause()
-            ms_c += e0.elapsed_time(e1)
-            launches_c += ctx.launches - l0
-            left -= k
-        return ms_c, launches_c
-
-    def rank_max(values):
-        if dist is None:
-            return list(values)
-        t = torch.tensor(list(values), device="cuda", dtype=torch.float64)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return [float(v) for v in t.tolist()]
-
-    first_ms, launches = timed_chunk()
-    first_ms = rank_max([first_ms])[0]
-    n_chunks = int(min(400, max(3, np.ceil(MIN_TIMED_MS / max(first_ms, 1e-3)))))
-    chunk_ms = [first_ms]
-    mine = []
-    for _ in range(n_chunks - 1):
-        ms_c, l_c = timed_chunk()
-        mine.append(ms_c)
-        launches += l_c
-    chunk_ms += rank_max(mine)
-    sess = state["sess"]
+    ms, launches, left, sess = 0.0, 0, args.steps, None
+    while left > 0:
+        k = min(left, max(1, cap - args.warmup))
+        if sess is not None:
+            sess.close()
+        sess = prob.session(T.ALGO_TWO_OPT_BEST, start, path)
+        sess.enqueue(args.warmup)
+        barrier()
+        if rank == 0:
+            sampler.start()
+        l0 = ctx.launches
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        sess.enqueue(k)
+        e1.record()
+        barrier()
+        if rank == 0:
+            sampler.pause()
+        ms += e0.elapsed_time(e1)
+        launches += ctx.launches - l0
+        left -= k
     real = int(sess.stats().moves)
-    if real < state["used"]:
-        raise SystemExit(f"bench invalid: the tour converged after {real} moves, fewer than the {state['used']} "
+    if real < args.warmup + k:
+        raise SystemExit(f"bench invalid: the tour converged after {real} moves, fewer than the {args.warmup + k} "
                          f"steps enqueued on it; lower SESSION_CAPS[{args.workload!r}]")
+    if dist is not None:
+        t_ms = torch.tensor([ms], device="cuda", dtype=torch.float64)
+        dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
+        ms = float(t_ms.item())
     clocks = sampler.stop() if rank == 0 else None
-    ms_chunk = float(np.median(chunk_ms))
-    ms = ms_chunk  # device time of K steps
     value = world * args.steps * P / (ms * 1e-3)
-    moves_applied = args.steps * len(chunk_ms)
+    moves_applied = args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sess.tour(), sess.log()[-1])
 
     # --- dominant kernel: average launch duration of the scan kernel (CUDA events, same stream)
     scan_ms = sess.time_scans(SCAN_REPS)
@@ -774,9 +752,7 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak",
-        "timed_chunks": len(chunk_ms), "timed_ms_total": float(sum(chunk_ms)),
-        "chunk_ms": {"median": ms_chunk, "min": float(min(chunk_ms)), "max": float(max(chunk_ms)),
-                     "first": float(chunk_ms[0])},
+        "timed_ms_total": ms,
         "vs_baseline": None, "dtype": "int32" if args.dist == "nint" else "f32", "data": "synthetic",
         "config": bench_config(args, world),
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
@@ -819,7 +795,11 @@ def main():
     ap.add_argument("--e2e-moves", type=int, default=-1, help="-1: to the local optimum")
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--cpu-budget", type=float, default=10.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed path's outputs after its last step "
+                    "as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.path == "recompute" and args.dist == "nint":
@@ -830,8 +810,6 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
-        if args.steps > 50:
-            args.steps = 50  # bounded sample: ~30 ms per CPU step
         run_reference(args, rank, world)
     else:
         run_ours(args, rank, world, local_rank)

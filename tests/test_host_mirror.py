@@ -27,8 +27,8 @@ def bins():
     return cli, build_host.SELFTEST
 
 
-def run(cmd, stdin=None):
-    p = subprocess.run(cmd, capture_output=True, text=True, input=stdin, timeout=600)
+def run(cmd, stdin=None, cwd=None):
+    p = subprocess.run(cmd, capture_output=True, text=True, input=stdin, timeout=600, cwd=cwd)
     return p.returncode, p.stdout, p.stderr
 
 
@@ -49,7 +49,7 @@ def test_cli_convert_discopt_fixture(bins, tmp_path):
     assert out.read_text() == ("NAME: tiny5_discopt\nTYPE: TSP\nCOMMENT: converted from DiscOpt dataset tiny5_discopt\n"
                                "DIMENSION: 5\nEDGE_WEIGHT_TYPE: EUC_2D\nNODE_COORD_SECTION\n"
                                "\t1 0 0\n\t2 10 0\n\t3 10 10\n\t4 0 10\n\t5 5 5\nEOF\n")
-    rc, _, _ = run([cli, "convert", "-i", "/nonexistent/file"])
+    rc, _, _ = run([cli, "convert", "-i", "/nonexistent/file"], cwd=tmp_path)  # default output: ./data/discopt
     assert rc != 0
     frac = tmp_path / "frac.txt"
     frac.write_text("3\n0.5 1e3\n\n-2.25 0.1\n7 8\n")
