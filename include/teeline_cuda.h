@@ -63,10 +63,15 @@ enum {
     TL_ALGO_TWO_OPT_BEST_CYCLIC = 2, /* Mode B incl. closing edge (two-opt-algo.ts:71-99)         */
     TL_ALGO_OR_OPT = 3,              /* or_opt.rs:80-184 (best-improvement, bit-exact)            */
     TL_ALGO_THREE_OPT = 4,           /* three_opt.rs:16-218 (best-improvement over triples, bit-exact) */
-    TL_ALGO_TWO_OPT_BEST_CACHED = 5  /* Mode B, the same moves and tour as TL_ALGO_TWO_OPT_BEST, but a step only
+    TL_ALGO_TWO_OPT_BEST_CACHED = 5, /* Mode B, the same moves and tour as TL_ALGO_TWO_OPT_BEST, but a step only
                                         re-evaluates the pairs the previous move changed (cached row minima):
                                         the fast way to the local optimum; stats.evals counts the pairs actually
                                         computed.  Not shardable, no tl_session_scan / time_scans. */
+    TL_ALGO_TWO_OPT_NEIGHBOR = 6     /* "Mode N": Mode B's move and delta over the pairs that create an edge to
+                                        one of a city's k nearest neighbours (see tl_problem_set_candidates):
+                                        a step costs O(n k) instead of O(n^2), for 10^5..10^6 cities.
+                                        Coordinate problems (F32_EXACT, NINT_I32), TL_PATH_AUTO / RECOMPUTE;
+                                        stats.evals counts the generated pairs.  Not shardable, not batched. */
 };
 
 /* where distances come from during the scan */
@@ -150,6 +155,20 @@ tl_status tl_dist_matrix_packed_i32(tl_problem *p, int32_t *out); /* NINT_I32 pr
  * (distance_matrix.rs:259-297, lin_kernighan.rs:12-27): out is n*k positions,
  * ascending distance, ties by lower position, rows padded with UINT32_MAX. */
 tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
+
+/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR, built on the device by tl_knn's kernel and kept with
+ * the problem (they depend on the instance only, like lin_kernighan::build_candidates,
+ * lin_kernighan.rs:12-27).  K[c] = the first k entries of tl_knn(k) for city c; padded slots
+ * (k > n-1) are skipped.  For every position i and slot s, with b = K[p_i][s], j = pos[b],
+ * lo = min(i, j), hi = max(i, j), the search generates the pairs (lo, hi) (the candidate edge is the
+ * move's first new edge) and (lo-1, hi-1) (its second new edge); a pair counts if it lies in Mode B's
+ * neighbourhood 0 <= i, i+2 <= j <= n-2.  A step applies the argmin of (delta, i, j) over them with
+ * strict '< 0', exactly as TL_ALGO_TWO_OPT_BEST; with k >= n-1 the moves are Mode B's.
+ * 1 <= k <= 32 (TL_ERR_INVALID otherwise); EXPLICIT problems: TL_ERR_UNSUPPORTED.  A session copies
+ * the lists when it is created, so later calls do not affect it.  Without a call, the first Mode N
+ * session builds TL_CANDIDATES_DEFAULT lists.  Memory is O(n k): nothing n^2 is allocated. */
+#define TL_CANDIDATES_DEFAULT 8
+tl_status tl_problem_set_candidates(tl_problem *p, uint32_t k);
 
 /* nearest_neighbor::solve (nearest_neighbor.rs:22-70), start at position 0. */
 tl_status tl_nn_tour(tl_problem *p, uint32_t k, uint32_t *tour_out);

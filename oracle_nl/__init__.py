@@ -1,0 +1,74 @@
+"""ctypes loader for the CPU ORACLE of candidate-list 2-opt (oracle_nl/libteeline_oracle_nl.so).
+
+TEST INFRASTRUCTURE ONLY, like `oracle`: tests and measurement scripts load it, the product package
+(teeline_b200/) never does.  Problems are `oracle.Problem` instances; the definition is in
+two_opt_nl.h and include/teeline_cuda.h (tl_problem_set_candidates).
+"""
+from __future__ import annotations
+
+import ctypes as C
+import os
+import subprocess
+
+import numpy as np
+
+import oracle as O
+
+_DIR = os.path.dirname(os.path.abspath(__file__))
+_SO = os.path.join(_DIR, "libteeline_oracle_nl.so")
+_ORACLE_DIR = os.path.dirname(os.path.abspath(O.__file__))
+
+
+def build(force: bool = False) -> str:
+    """Compile with gcc (oracle_nl/Makefile)."""
+    srcs = [os.path.join(_DIR, f) for f in ("two_opt_nl.c", "two_opt_nl.h", "Makefile")] + \
+        [os.path.join(_ORACLE_DIR, f) for f in ("teeline_oracle.c", "algos.inc", "teeline_oracle.h")]
+    stale = not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in srcs)
+    if force or stale:
+        subprocess.run(["make", "-C", _DIR, "-s"], check=True)
+    return _SO
+
+
+_lib = None
+
+
+def lib():
+    global _lib
+    if _lib is None:
+        build()
+        _lib = C.CDLL(_SO)
+    return _lib
+
+
+def _p(a):
+    return a.ctypes.data_as(C.c_void_p)
+
+
+def _cand(cand):
+    """n x k candidate positions as int32 (the GPU's UINT32_MAX padding becomes -1)."""
+    c = np.ascontiguousarray(cand)
+    if c.dtype == np.uint32:
+        c = c.view(np.int32)
+    c = np.ascontiguousarray(c, dtype=np.int32)
+    assert c.ndim == 2
+    return c
+
+
+def two_opt_nl_scan(p: O.Problem, tour, cand, nthreads: int = 1):
+    """One scan.  Returns (move or None, evals); move = (delta, i, j, 0, 0) as O.two_opt_best_scan."""
+    t = np.ascontiguousarray(tour, dtype=np.int32)
+    c = _cand(cand)
+    mv, ev = O.Move(), C.c_int64()
+    found = lib().tlo_two_opt_nl_scan(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int(nthreads), C.byref(mv),
+                                      C.byref(ev))
+    return (mv.astuple() if found else None), ev.value
+
+
+def two_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 1, log_cap: int = 0):
+    """Mode N to its local optimum (or max_moves).  Returns (tour, stats, moves) as O.two_opt_best."""
+    t = np.ascontiguousarray(tour, dtype=np.int32).copy()
+    c = _cand(cand)
+    st, log = O.Stats(), (O.Move * max(log_cap, 1))()
+    lib().tlo_two_opt_nl(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int64(max_moves), C.c_int(nthreads),
+                         C.byref(st), log, C.c_int64(log_cap))
+    return t, st, [log[m].astuple() for m in range(min(st.moves, log_cap))]

@@ -20,6 +20,8 @@ TL_OK = 0
 DIST_F32_EXACT, DIST_NINT_I32 = 0, 1
 ALGO_TWO_OPT_REF, ALGO_TWO_OPT_BEST, ALGO_TWO_OPT_BEST_CYCLIC, ALGO_OR_OPT, ALGO_THREE_OPT = 0, 1, 2, 3, 4
 ALGO_TWO_OPT_BEST_CACHED = 5
+ALGO_TWO_OPT_NEIGHBOR = 6
+CANDIDATES_DEFAULT = 8
 PATH_AUTO, PATH_MATRIX, PATH_RECOMPUTE = 0, 1, 2
 LEN_EXACT, LEN_FAST = 0, 1
 NCCL_ID_BYTES = 128
@@ -28,7 +30,7 @@ EXPORTS = [
     "tl_ctx_create", "tl_ctx_create_on_stream", "tl_ctx_destroy", "tl_ctx_sync", "tl_last_error",
     "tl_version", "tl_ctx_launch_count", "tl_nccl_unique_id", "tl_ctx_attach_nccl",
     "tl_problem_create_euc2d", "tl_problem_create_explicit", "tl_problem_destroy",
-    "tl_dist_matrix_packed", "tl_dist_matrix_packed_i32", "tl_knn", "tl_nn_tour", "tl_tour_lengths",
+    "tl_dist_matrix_packed", "tl_dist_matrix_packed_i32", "tl_knn", "tl_problem_set_candidates", "tl_nn_tour", "tl_tour_lengths",
     "tl_tour_lengths_i64", "tl_local_search", "tl_two_opt_batch", "tl_session_create",
     "tl_session_destroy", "tl_session_set_shard", "tl_session_scan", "tl_session_time_scans",
     "tl_session_enqueue",
@@ -105,6 +107,7 @@ def load():
     L.tl_dist_matrix_packed.argtypes = [C.c_void_p, C.c_void_p]
     L.tl_dist_matrix_packed_i32.argtypes = [C.c_void_p, C.c_void_p]
     L.tl_knn.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
+    L.tl_problem_set_candidates.argtypes = [C.c_void_p, C.c_uint32]
     L.tl_nn_tour.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
     L.tl_tour_lengths.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]
     L.tl_tour_lengths_i64.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]

@@ -80,6 +80,8 @@ struct tl_problem {
     float dmax = 0.0f;      // upper bound on any city-to-city distance (bounding-box diagonal, rounded up)
     float2 *d_xy = nullptr; // city-ordered coordinates (coordinate problems)
     float *d_tri = nullptr; // packed triangle (EXPLICIT problems)
+    uint32_t *d_cand = nullptr; // n x cand_k candidate lists for Mode N (tl_problem_set_candidates)
+    uint32_t cand_k = 0;
 };
 
 namespace tl {

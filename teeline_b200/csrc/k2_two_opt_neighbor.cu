@@ -1,0 +1,260 @@
+// k2_two_opt_neighbor.cu -- K2 candidate-list best-improvement 2-opt ("Mode N"), coordinate recompute.
+//
+// What it computes: Mode B's neighbourhood (0 <= i, i+2 <= j <= n-2, path[i+1..=j] reversed) and
+// delta, restricted to the pairs that create an edge to one of a city's k nearest neighbours.  For
+// every position i and candidate slot s, with b = K[p_i][s], j = pos[b], lo = min(i, j), hi = max(i, j):
+//   (lo, hi)         the candidate edge (p_lo, p_hi) is the move's first new edge
+//   (lo - 1, hi - 1) the candidate edge is its second new edge
+// A generated pair counts only inside the neighbourhood.  The step's move is the argmin of
+// (delta, i, j) over the generated pairs with strict '< 0' (better_2opt), as in Mode B; duplicates
+// carry the same key.  With k >= n-1 every Mode B pair is generated and the moves are Mode B's.
+//
+// How: a grid of resident CTAs walks the n*k (position, slot) items with a grid-stride loop.  Per
+// item: the record at i, the candidate, pos[b], then the records lo-1 .. hi+1; the two pairs share
+// d(p_lo, p_hi), so three distances cover both.  The last CTA (acq_rel ticket) reduces the per-CTA
+// records.  A short segment is reversed by that CTA; a long one is left as the pending move for the
+// apply grid that every step launches (apply_two_opt_kernel, pending_only), which leaves at once when
+// there is none.  The grid size cannot depend on the move: the host queues steps without reading back.
+// The records, pos[] and the candidate lists (16 + 4 + 4k bytes per city) fit L2 up to about 10^6
+// cities, so the scan is a chain of dependent L2 gathers.
+#include "kernels.cuh"
+#include "policy.cuh"
+#include "two_opt_apply.cuh"
+
+#include <math_constants.h>
+
+namespace tl {
+
+namespace {
+
+constexpr int THREADS = kNlThreads;
+constexpr int WARPS = THREADS / 32;
+
+// Pt records with the TSPLIB nint metric recomputed from the coordinates (bit-equal to K1's matrix
+// entries, as in the persistent Mode R kernel); the entering-edge length is stored as int32 bits.
+template <bool GRID>
+struct EucNintPol {
+    using V = int32_t;
+    using Rec = Pt;
+    Pt *pts;
+    __device__ __forceinline__ Rec load(uint32_t q) const { return pts[q]; }
+    static __device__ __forceinline__ V sp(const Rec &r) { return __float_as_int(r.sp); }
+    static __device__ __forceinline__ int32_t city(const Rec &r) { return r.city; }
+    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const
+    {
+        return GRID ? dist_nint_grid(a.x, a.y, b.x, b.y) : dist_nint(a.x, a.y, b.x, b.y);
+    }
+    __device__ __forceinline__ void store_id(uint32_t q, const Rec &from) const
+    {
+        pts[q].x = from.x;
+        pts[q].y = from.y;
+        pts[q].city = from.city;
+    }
+    __device__ __forceinline__ void store_sp(uint32_t q, V v) const { pts[q].sp = __int_as_float(v); }
+};
+
+// metric: 0 = f32 guarded fast sqrt, 1 = f32 IEEE sqrt, 2 = nint for integer coordinates, 3 = nint in f64
+#define TL_NL_DISPATCH(metric, pts, ...)                                      \
+    switch (metric) {                                                         \
+    case 0: { EucPol<true> P{pts}; __VA_ARGS__; } break;                      \
+    case 1: { EucPol<false> P{pts}; __VA_ARGS__; } break;                     \
+    case 2: { EucNintPol<true> P{pts}; __VA_ARGS__; } break;                  \
+    default: { EucNintPol<false> P{pts}; __VA_ARGS__; } break;                \
+    }
+
+// Tail of a fused step, run by the last CTA: reduce the per-CTA records, count the step's evaluated
+// pairs, then either reverse a short segment here and finish the step, or leave a long one pending.
+template <class Pol>
+__device__ __noinline__ void nl_tail(const Pol &P, uint32_t *pos, Best<typename Pol::V> *blockbest, DevState *state,
+                                     unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap)
+{
+    using V = typename Pol::V;
+    __shared__ Best<V> red[WARPS];
+    __shared__ unsigned long long red_cnt[WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    StateHeader hdr{};
+    if (threadIdx.x == 0) hdr = load_state_header(state);
+    Best<V> v{(V)0, 0xffffffffu, 0xffffffffu, 0u};
+    unsigned long long cnt = 0;
+    for (int c = threadIdx.x; c < (int)gridDim.x; c += blockDim.x) {
+        // L2 read: the records were written by other CTAs of this launch
+        const int4 raw = __ldcg(reinterpret_cast<const int4 *>(blockbest) + c);
+        const Best<V> o{Val<V>::from_bits(raw.x), (uint32_t)raw.y, (uint32_t)raw.z, (uint32_t)raw.w};
+        cnt += o.aux;
+        if (better_2opt(o.delta, o.i, o.j, v.delta, v.i, v.j)) v = o;
+    }
+    warp_argmin_2opt(v.delta, v.i, v.j);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
+    if (lane == 0) {
+        red[warp] = v;
+        red_cnt[warp] = cnt;
+    }
+    __syncthreads();
+    v = red[0];
+    cnt = red_cnt[0];
+#pragma unroll
+    for (int w = 1; w < WARPS; ++w) {
+        const Best<V> o = red[w];
+        cnt += red_cnt[w];
+        if (better_2opt(o.delta, o.i, o.j, v.delta, v.i, v.j)) v = o;
+    }
+    const bool found = v.i != 0xffffffffu;
+    const bool long_seg = found && (v.j - v.i) / 2 > (uint32_t)kNlCtaSwaps;
+    if (threadIdx.x == 0) {
+        state->computed += cnt;
+        // the pending move for this step's apply grid (none: the step is finished here)
+        blockbest[gridDim.x] = long_seg ? v : Best<V>{(V)0, 0xffffffffu, 0xffffffffu, 0u};
+        *ticket = 0u;
+    }
+    if (long_seg) return;
+    if (found) reverse_segment_inplace(P, v.i, v.j, nullptr, threadIdx.x, blockDim.x, false, V(), V(), pos);
+    if (threadIdx.x == 0) finish_best_step(state, hdr, found, (float)v.delta, v.i, v.j, log, log_cap);
+}
+
+template <class Pol>
+__global__ void __launch_bounds__(THREADS, kNlMinBlocks)
+    two_opt_nl_scan_kernel(Pol P, uint32_t *__restrict__ pos, const uint32_t *__restrict__ cand, uint32_t k,
+                           uint32_t n, Best<typename Pol::V> *blockbest, DevState *state, unsigned int *ticket,
+                           tl_move *__restrict__ log, uint64_t log_cap, int fuse_apply)
+{
+    using V = typename Pol::V;
+    using Rec = typename Pol::Rec;
+    griddep_launch_dependents();
+    griddep_wait(); // the previous step's move is applied and visible from here on
+    // uniform across the grid: only a step's tail or apply grid writes it, after every CTA has finished
+    if (*reinterpret_cast<const volatile int *>(&state->done)) return;
+
+    V best = (V)0;
+    uint32_t bi = 0xffffffffu, bj = 0xffffffffu, cnt = 0;
+    const uint64_t total = (uint64_t)n * k;
+    for (uint64_t t = (uint64_t)blockIdx.x * THREADS + threadIdx.x; t < total; t += (uint64_t)gridDim.x * THREADS) {
+        const uint32_t i = (uint32_t)(t / k), s = (uint32_t)(t - (uint64_t)i * k);
+        const uint32_t b = __ldg(&cand[(size_t)Pol::city(P.load(i)) * k + s]);
+        if (b == 0xffffffffu) continue; // padding: fewer than k other cities
+        const uint32_t j = pos[b];
+        const uint32_t lo = min(i, j), hi = max(i, j);
+        if (hi < lo + 2) continue; // the candidate edge is a tour edge: no pair
+        const bool first = hi <= n - 2, second = lo >= 1;
+        if (!first && !second) continue;
+        const Rec rlo = P.load(lo), rhi = P.load(hi);
+        const V shared = P.dist(rlo, rhi);
+        if (first) { // (lo, hi): new edges (p_lo, p_hi) and (p_lo+1, p_hi+1)
+            const Rec a = P.load(lo + 1), c = P.load(hi + 1);
+            const V d = Val<V>::sub(Val<V>::add(shared, P.dist(a, c)), Val<V>::add(Pol::sp(a), Pol::sp(c)));
+            ++cnt;
+            if (d < (V)0 && better_2opt(d, lo, hi, best, bi, bj)) {
+                best = d;
+                bi = lo;
+                bj = hi;
+            }
+        }
+        if (second) { // (lo-1, hi-1): new edges (p_lo-1, p_hi-1) and (p_lo, p_hi)
+            const Rec a = P.load(lo - 1), c = P.load(hi - 1);
+            const V d = Val<V>::sub(Val<V>::add(P.dist(a, c), shared), Val<V>::add(Pol::sp(rlo), Pol::sp(rhi)));
+            ++cnt;
+            if (d < (V)0 && better_2opt(d, lo - 1, hi - 1, best, bi, bj)) {
+                best = d;
+                bi = lo - 1;
+                bj = hi - 1;
+            }
+        }
+    }
+
+    __shared__ Best<V> red[WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    warp_argmin_2opt(best, bi, bj);
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if (lane == 0) red[warp] = Best<V>{best, bi, bj, cnt};
+    __syncthreads();
+    if (warp == 0) {
+        Best<V> v = lane < WARPS ? red[lane] : Best<V>{(V)0, 0xffffffffu, 0xffffffffu, 0u};
+        const uint32_t c = __reduce_add_sync(0xffffffffu, v.aux);
+        warp_argmin_2opt(v.delta, v.i, v.j);
+        v.aux = c; // 2-opt records carry the CTA's evaluated-pair count in aux
+        if (lane == 0) blockbest[blockIdx.x] = v;
+    }
+    if (!fuse_apply) return;
+    __shared__ unsigned int s_last;
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = (ticket_take_acq_rel(ticket) == gridDim.x - 1) ? 1u : 0u; // thread 0 wrote blockbest
+    __syncthreads();
+    if (!s_last) return;
+    nl_tail(P, pos, blockbest, state, ticket, log, log_cap);
+}
+
+// tour-ordered records (entering-edge length in the policy's metric) and pos[city] = position
+template <class Pol>
+__global__ void __launch_bounds__(256)
+    nl_init_kernel(Pol P, const float2 *__restrict__ xy, const uint32_t *__restrict__ tour, uint32_t n, uint32_t npad,
+                   uint32_t *__restrict__ pos)
+{
+    using V = typename Pol::V;
+    for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < npad; q += gridDim.x * blockDim.x) {
+        if (q < n) {
+            const uint32_t c = tour[q];
+            const float2 a = xy[c];
+            const Pt r{a.x, a.y, (int32_t)c, 0.0f};
+            P.store_id(q, r);
+            if (q == 0) {
+                P.store_sp(q, (V)0);
+            } else {
+                const float2 b = xy[tour[q - 1]];
+                P.store_sp(q, P.dist(Pt{b.x, b.y, 0, 0.0f}, r));
+            }
+            pos[c] = q;
+        } else { // padding: never part of a pair
+            P.store_id(q, Pt{0.0f, 0.0f, -1, 0.0f});
+            P.store_sp(q, Val<V>::neg_inf());
+        }
+    }
+}
+
+} // namespace
+
+void launch_nl_init(int metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
+                    uint32_t *pos, cudaStream_t st)
+{
+    const int grid = (int)((npad + 255) / 256);
+    TL_NL_DISPATCH(metric, pts, (nl_init_kernel<<<grid, 256, 0, st>>>(P, xy, tour, n, npad, pos)));
+}
+
+void launch_nl_scan(int metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
+                    DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
+                    cudaStream_t st)
+{
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)grid);
+    cfg.blockDim = dim3(THREADS);
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    const int fuse = fuse_apply ? 1 : 0;
+    TL_NL_DISPATCH(metric, pts,
+                   (cudaLaunchKernelEx(&cfg, two_opt_nl_scan_kernel<decltype(P)>, P, pos, cand, k, n,
+                                       reinterpret_cast<Best<typename decltype(P)::V> *>(blockbest), state, ticket,
+                                       log, (uint64_t)log_cap, fuse)));
+}
+
+void launch_nl_apply(int metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
+                     tl_move *log, uint64_t log_cap, int grid, cudaStream_t st)
+{
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)grid);
+    cfg.blockDim = dim3(256);
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    TL_NL_DISPATCH(metric, pts,
+                   (cudaLaunchKernelEx(&cfg, apply_two_opt_kernel<decltype(P)>, P,
+                                       reinterpret_cast<const Best<typename decltype(P)::V> *>(pending), 1, state,
+                                       ticket, log, (uint64_t)log_cap, pos, 1)));
+}
+
+} // namespace tl

@@ -596,7 +596,7 @@ void launch_apply_two_opt(const Src &src, const void *cand, int ncand, DevState 
 {
     TL_DISPATCH_POL(src, (apply_two_opt_kernel<<<grid, 256, 0, st>>>(
                              P, reinterpret_cast<const Best<typename decltype(P)::V> *>(cand), ncand, state,
-                             ticket, log, log_cap)));
+                             ticket, log, log_cap, nullptr, 0)));
 }
 
 void launch_extract_tour(const Src &src, uint32_t n, uint32_t *tour, cudaStream_t st)

@@ -255,6 +255,20 @@ void launch_two_opt_cached_step(const Src &src, uint32_t n, int cyclic, unsigned
                                 int *fullrows, DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap,
                                 int grid, cudaStream_t st);
 
+// K2 candidate-list 2-opt, "Mode N" (k2_two_opt_neighbor.cu).  metric: 0 = f32 fast sqrt, 1 = f32 IEEE
+// sqrt, 2 = nint for integer coordinates, 3 = nint in f64.  blockbest holds grid + 1 records: one per
+// CTA and, at [grid], the step's pending long move for the apply grid.
+constexpr int kNlThreads = 256;
+constexpr int kNlMinBlocks = 2;
+constexpr int kNlCtaSwaps = 2048; // segments of up to this many swapped pairs are reversed by the reducing CTA
+void launch_nl_init(int metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
+                    uint32_t *pos, cudaStream_t st);
+void launch_nl_scan(int metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
+                    DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
+                    cudaStream_t st);
+void launch_nl_apply(int metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
+                     tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
+
 // K2-batch: one CTA per tour, tour records in shared memory
 constexpr int kBatchR = 5;              // diagonals per thread group (odd => conflict-free LDS.128)
 constexpr int kBatchMaxSmem = 200 * 1024;

@@ -78,6 +78,14 @@ struct tl_session {
     DevBuf<CachedDesc> cdesc;
     DevBuf<int> fullrows;
 
+    // candidate-list 2-opt (TL_ALGO_TWO_OPT_NEIGHBOR): Pt records plus pos[] and the session's own
+    // copy of the problem's candidate lists
+    bool nl = false;
+    int nl_metric = 0;               // k2_two_opt_neighbor.cu: 0/1 f32 fast/IEEE sqrt, 2/3 nint grid/f64
+    DevBuf<uint32_t> pos;            // city -> position
+    DevBuf<uint32_t> nl_cand;        // n x nl_k
+    uint32_t nl_k = 0;
+
     DevBuf<BestF> cand; // shard_count * grid records (BestF and BestI have the same layout)
     DevBuf<DevState> state;
     DevBuf<unsigned int> ticket;
@@ -96,6 +104,7 @@ struct tl_session {
     double device_ms = 0.0;
 
     bool matrix() const { return path_used == TL_PATH_MATRIX; }
+    bool int_values() const { return nl ? nl_metric >= 2 : src.is_int(); }
 };
 
 namespace {
@@ -220,6 +229,15 @@ tl_status upload_three_geometry(tl_session *s)
 tl_status upload_geometry(tl_session *s)
 {
     if (s->algo == TL_ALGO_THREE_OPT) return upload_three_geometry(s);
+    if (s->nl) {
+        // resident CTAs walk the n*k (position, slot) items; one record per CTA plus the pending move
+        const int64_t blocks = ceil_div64((int64_t)s->n * s->nl_k, kNlThreads);
+        s->grid = (int)std::max<int64_t>(1, std::min<int64_t>(blocks, (int64_t)s->c->sm_count * kNlMinBlocks));
+        if (const char *cap = getenv("TL_MAX_GRID")) s->grid = std::max(1, std::min(s->grid, atoi(cap)));
+        TL_CUDA_TRY(s->cand.alloc((size_t)s->grid + 1));
+        TL_CUDA_TRY(cudaMemsetAsync(s->cand.p, 0xff, ((size_t)s->grid + 1) * sizeof(BestF), s->c->stream)); // no move pending
+        return TL_OK;
+    }
     if (s->algo == TL_ALGO_OR_OPT) {
         build_or_geometry(s);
         TL_CUDA_TRY(s->cand.alloc((size_t)s->grid * s->shard_count));
@@ -341,7 +359,11 @@ tl_status launch_scan(tl_session *s, bool fuse, bool exchange = true)
     const ShardComm *comm = (fused && s->shard_count > 1) ? &s->comm : nullptr;
     BestF *mine = s->cand.p + (size_t)s->shard_index * s->grid;
     cudaStream_t st = s->c->stream;
-    if (s->algo == TL_ALGO_THREE_OPT) {
+    if (s->nl) {
+        launch_nl_scan(s->nl_metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->cand.p, s->state.p,
+                       s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
+        s->c->launches++;
+    } else if (s->algo == TL_ALGO_THREE_OPT) {
         TL_CUDA_TRY(cudaMemsetAsync(s->or_ticket.p, 0, 4, st)); // re-arm the work queue
         launch_three_scan(s->src, s->n, s->band_first.p, s->or_item_begin, s->or_item_end, mine, s->state.p,
                           s->or_ticket.p, s->grid, st);
@@ -420,6 +442,12 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
         tl_status rc = launch_scan(s, true);
         if (rc != TL_OK) return rc;
         s->steps_since_permute++;
+        if (s->nl) { // a long segment left pending by the scan's last CTA (none: the grid leaves at once)
+            launch_nl_apply(s->nl_metric, s->pts.p, s->pos.p, s->cand.p + s->grid, s->state.p, s->ticket.p + 1,
+                            s->log.p, s->log_cap, apply_grid, st);
+            s->c->launches++;
+            continue;
+        }
         if (s->algo == TL_ALGO_OR_OPT) {
             launch_or_apply(s->src, s->tmp.p, s->n, s->cand.p, s->grid * s->shard_count, s->state.p, s->ticket.p,
                             s->log.p, s->log_cap, apply_grid, st);
@@ -510,7 +538,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     const bool cached = algo == TL_ALGO_TWO_OPT_BEST_CACHED; // Mode B with cached row minima: runs as Mode B
     if (cached) algo = TL_ALGO_TWO_OPT_BEST;
     if (algo != TL_ALGO_TWO_OPT_BEST && algo != TL_ALGO_TWO_OPT_BEST_CYCLIC && algo != TL_ALGO_TWO_OPT_REF &&
-        algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT) {
+        algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT && algo != TL_ALGO_TWO_OPT_NEIGHBOR) {
         set_error("tl_session_create: unknown algo %d", algo);
         return TL_ERR_INVALID;
     }
@@ -518,10 +546,17 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         set_error("tl_session_create: unknown path %d", path);
         return TL_ERR_INVALID;
     }
+    const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR;
+    if (nl && (path == TL_PATH_MATRIX || p->kind == PK_EXPLICIT)) {
+        // candidate 2-opt is for instances whose n^2 matrix is the problem; both metrics are recomputed
+        set_error(p->kind == PK_EXPLICIT ? "candidate 2-opt needs coordinates (EXPLICIT problem)"
+                                         : "candidate 2-opt recomputes distances: TL_PATH_MATRIX is not supported");
+        return TL_ERR_UNSUPPORTED;
+    }
     // AUTO: recompute for f32 coordinate problems (bit-identical to the matrix and no n^2 memory),
     // matrix for EXPLICIT problems (placeholder coordinates, tsplib.rs:257-262) and the nint metric
-    const bool want_matrix = path == TL_PATH_MATRIX || (path == TL_PATH_AUTO && p->kind != PK_EUC_F32);
-    if (!want_matrix && p->kind != PK_EUC_F32) {
+    const bool want_matrix = !nl && (path == TL_PATH_MATRIX || (path == TL_PATH_AUTO && p->kind != PK_EUC_F32));
+    if (!nl && !want_matrix && p->kind != PK_EUC_F32) {
         set_error(p->kind == PK_EXPLICIT ? "recompute path is illegal for EXPLICIT problems (no coordinates)"
                                          : "recompute path is not available for the NINT_I32 metric");
         return TL_ERR_UNSUPPORTED;
@@ -537,6 +572,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     s->c = c;
     s->algo = algo;
     s->cached = cached;
+    s->nl = nl;
     s->path_used = want_matrix ? TL_PATH_MATRIX : TL_PATH_RECOMPUTE;
     s->n = p->n;
     s->cyclic = algo == TL_ALGO_TWO_OPT_BEST_CYCLIC || algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT;
@@ -668,6 +704,26 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         if (const char *ev = getenv("TL_REPERMUTE_EVERY")) s->repermute_every = atoi(ev);
         if (cached) s->repermute_every = 0; // a cached step reads a few rows, not the triangle
         configure_matrix_pin(s, bytes);
+    } else if (nl) {
+        if (!s->trivial && !p->d_cand) {
+            tl_status rc = tl_problem_set_candidates(p, TL_CANDIDATES_DEFAULT);
+            if (rc != TL_OK) return fail(rc);
+        }
+        s->nl_k = s->trivial ? 0 : p->cand_k;
+        if (s->pts.alloc(s->npad) != cudaSuccess || s->pos.alloc(p->n) != cudaSuccess ||
+            s->nl_cand.alloc((size_t)p->n * s->nl_k) != cudaSuccess) {
+            set_error("tl_session_create: device allocation failed");
+            return fail(TL_ERR_NOMEM);
+        }
+        if (s->nl_k) { // the session's own copy: later tl_problem_set_candidates calls do not reach it
+            e = cudaMemcpyAsync(s->nl_cand.p, p->d_cand, (size_t)p->n * s->nl_k * 4, cudaMemcpyDeviceToDevice, c->stream);
+            if (e != cudaSuccess) { set_error("tl_session_create: %s", cudaGetErrorString(e)); return fail(TL_ERR_CUDA); }
+        }
+        s->nl_metric = p->kind == PK_EUC_NINT ? (p->grid_nint ? 2 : 3) : (p->fast_sqrt ? 0 : 1);
+        s->src.kind = p->fast_sqrt ? SRC_EUC_FAST : SRC_EUC_SAFE; // tl_session_tour reads the city fields only
+        s->src.pts = s->pts.p;
+        launch_nl_init(s->nl_metric, p->d_xy, d_tour.p, p->n, s->npad, s->pts.p, s->pos.p, c->stream);
+        c->launches++;
     } else {
         if (s->pts.alloc(s->npad) != cudaSuccess) { set_error("tl_session_create: device allocation failed"); return fail(TL_ERR_NOMEM); }
         s->src.kind = p->fast_sqrt ? SRC_EUC_FAST : SRC_EUC_SAFE;
@@ -744,6 +800,10 @@ tl_status tl_session_set_shard(tl_session *s, int32_t index, int32_t count)
         if (count > 1) { set_error("cached Mode B does not shard (a step touches a few rows)"); return TL_ERR_UNSUPPORTED; }
         return TL_OK;
     }
+    if (s->nl) {
+        if (count > 1) { set_error("candidate 2-opt does not shard"); return TL_ERR_UNSUPPORTED; }
+        return TL_OK;
+    }
     DeviceGuard g(s->c);
     s->shard_index = index;
     s->shard_count = count;
@@ -800,7 +860,7 @@ tl_status tl_session_scan(tl_session *s, tl_move *best, int32_t *found)
     if (was_done) { s->h.done = was_done; rc = push_state(s); if (rc != TL_OK) return rc; }
     bool any;
     const bool three = s->algo == TL_ALGO_THREE_OPT;
-    if (s->src.is_int()) {
+    if (s->int_values()) {
         std::vector<BestI> hi(hc.size());
         memcpy(hi.data(), hc.data(), hc.size() * sizeof(BestF));
         any = three ? reduce_host_three(hi, best) : reduce_host(hi, s->algo == TL_ALGO_OR_OPT, best);
@@ -956,7 +1016,7 @@ tl_status tl_session_stats(tl_session *s, tl_stats *stats)
     memset(stats, 0, sizeof *stats);
     stats->passes = s->algo == TL_ALGO_TWO_OPT_REF ? s->h.passes : s->h.scans;
     stats->moves = s->h.moves;
-    stats->evals = s->cached ? s->h.computed : stats->passes * s->pairs_per_scan;
+    stats->evals = (s->cached || s->nl) ? s->h.computed : stats->passes * s->pairs_per_scan;
     stats->launches = s->c->launches - s->launches0;
     stats->repermutes = s->repermutes;
     stats->device_ms = s->device_ms;

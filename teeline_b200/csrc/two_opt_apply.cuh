@@ -16,11 +16,14 @@ namespace tl {
 // known_e1: the caller already knows e1 = d(p_i, p_j) and the move's delta (integer metric only:
 // the matrix scan's winning thread held e1, and e2 = delta + (s_i + s_j) - e1 exactly), which
 // saves the two dependent matrix loads -- an HBM round trip on the fused step's critical path.
+// pos (nullable): city -> position map kept beside the records (candidate-list 2-opt); the thread that
+// stores a position's identity also stores that city's new position.
 template <class Pol>
 __device__ __forceinline__ void reverse_segment_inplace(const Pol &P, uint32_t mi, uint32_t mj, float *delta_out,
                                                         uint32_t tid, uint32_t nthreads, bool known_e1 = false,
                                                         typename Pol::V e1_in = typename Pol::V(),
-                                                        typename Pol::V delta_in = typename Pol::V())
+                                                        typename Pol::V delta_in = typename Pol::V(),
+                                                        uint32_t *pos = nullptr)
 {
     using V = typename Pol::V;
     using Rec = typename Pol::Rec;
@@ -71,6 +74,10 @@ __device__ __forceinline__ void reverse_segment_inplace(const Pol &P, uint32_t m
             }
             P.store_id(a, B[u]);
             P.store_id(b, A[u]);
+            if (pos) {
+                pos[B[u].city] = a;
+                pos[A[u].city] = b;
+            }
             if (t < nsp) { // mi+2+t <-> mj-t
                 P.store_sp(a + 1, Pol::sp(B[u]));
                 P.store_sp(b, sa[u]);
@@ -128,12 +135,16 @@ __device__ __forceinline__ unsigned int ticket_take_acq_rel(unsigned int *ticket
 // Stand-alone apply step for Mode B (sharded sessions and the matrix path): every block
 // reduces the candidate records redundantly (at most a few hundred), the grid reverses the
 // segment, the last block to finish updates the loop state.
+// Candidate-list 2-opt (k2_two_opt_neighbor.cu) passes its one pending long move with
+// pending_only = true: no move pending means the scan already finished the step, and the grid leaves.
 template <class Pol>
 __global__ void __launch_bounds__(256)
     apply_two_opt_kernel(Pol P, const Best<typename Pol::V> *__restrict__ cand, int ncand, DevState *state,
-                         unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap)
+                         unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap, uint32_t *pos,
+                         int pending_only)
 {
     using V = typename Pol::V;
+    griddep_wait(); // PDL launches only: the step's scan has finished and its writes are visible
     if (state->done) return;
     __shared__ Best<V> sred[8];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -152,8 +163,10 @@ __global__ void __launch_bounds__(256)
         if (better_2opt(o.delta, o.i, o.j, v.delta, v.i, v.j)) v = o;
     }
     const bool found = v.i != 0xffffffffu;
+    if (pending_only && !found) return; // uniform over the grid
     if (found)
-        reverse_segment_inplace(P, v.i, v.j, nullptr, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
+        reverse_segment_inplace(P, v.i, v.j, nullptr, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x,
+                                false, V(), V(), pos);
     __syncthreads();
     if (threadIdx.x == 0) {
         __threadfence();

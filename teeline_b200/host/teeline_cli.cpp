@@ -25,6 +25,7 @@ struct Args {
     std::optional<size_t> epochs, platoo_epochs, n_nearest, n_elite, num_ants;
     std::optional<float> mutation_probability, alpha, beta, evaporation_rate;
     uint64_t seed = 0; // extension: Philox key of the population solvers
+    uint32_t candidates = 0; // extension: k of `--mode neighbor` (0 = the library's default)
 };
 
 [[noreturn]] void die(const std::string &msg, int code = 1)
@@ -72,7 +73,15 @@ Args parse_args(int argc, char **argv)
         else if (s == "--evaporation-rate") a.evaporation_rate = std::strtof(next("--evaporation-rate").c_str(), nullptr);
         else if (s == "--num-ants") a.num_ants = std::strtoull(next("--num-ants").c_str(), nullptr, 10);
         else if (s == "--seed") a.seed = std::strtoull(next("--seed").c_str(), nullptr, 10);
-        else if (s == "--mode") a.mode = next("--mode");  // extension: ref | best | best_cyclic
+        else if (s == "--mode") a.mode = next("--mode");  // extension: ref | best | best_cyclic | neighbor
+        else if (s == "--candidates") { // extension: k nearest candidates of --mode neighbor, 1..32
+            const std::string v = next("--candidates");
+            char *end = nullptr;
+            const unsigned long long k = std::strtoull(v.c_str(), &end, 10);
+            if (v.empty() || *end || k < 1 || k > 32)
+                die("invalid value '" + v + "' for '--candidates <K>': must be an integer in 1..32", 2);
+            a.candidates = (uint32_t)k;
+        }
         else if (s == "--path") a.path = next("--path");  // extension: auto | matrix | recompute
         else if (!s.empty() && s[0] != '-' && a.cmd == "solve" && a.solver.empty()) a.solver = s;
         else die("unexpected argument '" + s + "' found", 2);
@@ -113,6 +122,7 @@ AppOptions options_from_args(const Args &a)
     o.cuda_seed = a.seed;
     o.cuda_mode = a.mode;
     o.cuda_path = a.path;
+    o.cuda_candidates = a.candidates;
     return o;
 }
 
@@ -244,6 +254,7 @@ int run_solvers()
     std::printf("  nn | nearest_neighbor        nearest-neighbour constructor (nearest_neighbor.rs)\n");
     std::printf("  2opt | two_opt               first-improvement 2-opt, bit-exact with two_opt.rs\n");
     std::printf("  2opt_best | two_opt_best     best-improvement 2-opt (extension)\n");
+    std::printf("  2opt --mode neighbor         candidate-list best-improvement 2-opt, --candidates K (extension)\n");
     std::printf("  or_opt | or-opt              Or-opt, bit-exact with or_opt.rs\n");
     std::printf("  3opt | three_opt             best-improvement 3-opt, bit-exact with three_opt.rs\n");
     std::printf("presets: fast (nn,2opt)\n");

@@ -456,12 +456,25 @@ Solution run_local_search(const TspProblem &problem, int algo, int path, const P
         m.total = 0.0f;
         (*tx)(m);
     }
-    std::vector<tl_move> log(tx ? (size_t)1 << 20 : 0);
+    // candidate 2-opt serves instances whose packed triangle cannot come to the host (2 TB at 10^6
+    // cities), and two_opt.rs's per-move progress value needs it: only the start and the result are sent
+    const bool replay = tx && algo != TL_ALGO_TWO_OPT_NEIGHBOR;
+    std::vector<tl_move> log(replay ? (size_t)1 << 20 : 0);
     tl_stats st{};
     std::vector<uint32_t> before = tour;
     check(tl_local_search(dm.impl->prob, algo, path, tour.data(), -1, &st, log.empty() ? nullptr : log.data(), log.size()),
           who);
-    if (tx) {
+    if (tx && !replay) {
+        ProgressMessage m;
+        m.kind = ProgressMessage::PathUpdate;
+        m.route = to_ids(tour, dm);
+        m.total = 0.0f;
+        (*tx)(m);
+        ProgressMessage done;
+        done.kind = ProgressMessage::Done;
+        (*tx)(done);
+    }
+    if (replay) {
         std::vector<uint32_t> cur = before;
         const size_t n = cur.size();
         for (size_t k = 0; k < std::min<size_t>(st.moves, log.size()); ++k) {
@@ -506,13 +519,16 @@ Solution run_local_search(const TspProblem &problem, int algo, int path, const P
 namespace two_opt {
 
 Solution solve_with(const TspProblem &problem, const std::string &mode, const std::string &path,
-                    const ProgressSender *progress_tx, const std::vector<size_t> *init_tour)
+                    const ProgressSender *progress_tx, const std::vector<size_t> *init_tour, uint32_t candidates)
 {
     int algo;
     if (mode.empty() || mode == "ref") algo = TL_ALGO_TWO_OPT_REF;
     else if (mode == "best") algo = TL_ALGO_TWO_OPT_BEST;
     else if (mode == "best_cyclic") algo = TL_ALGO_TWO_OPT_BEST_CYCLIC;
-    else throw std::runtime_error("unknown 2-opt mode `" + mode + "` (ref | best | best_cyclic)");
+    else if (mode == "neighbor") algo = TL_ALGO_TWO_OPT_NEIGHBOR;
+    else throw std::runtime_error("unknown 2-opt mode `" + mode + "` (ref | best | best_cyclic | neighbor)");
+    if (algo == TL_ALGO_TWO_OPT_NEIGHBOR && candidates)
+        check(tl_problem_set_candidates(problem.distances.impl->prob, candidates), "two_opt");
     const std::vector<size_t> start = init_tour ? *init_tour : ids_of(problem.cities); // two_opt.rs:18-20
     return run_local_search(problem, algo, path_code(path), progress_tx, start, "two_opt");
 }
@@ -682,7 +698,8 @@ Result<Solution> solve_with_context(Solvers solver, const TspProblem &problem, c
     case Solvers::TwoOpt:
         if (opts.cuda_mode.empty() && opts.cuda_path.empty())
             return Result<Solution>::ok(two_opt::solve(problem, h, tx, init_tour));
-        return Result<Solution>::ok(two_opt::solve_with(problem, opts.cuda_mode, opts.cuda_path, tx, init_tour));
+        return Result<Solution>::ok(
+            two_opt::solve_with(problem, opts.cuda_mode, opts.cuda_path, tx, init_tour, opts.cuda_candidates));
     case Solvers::TwoOptBest:
         return Result<Solution>::ok(two_opt::solve_with(problem, "best", opts.cuda_path, tx, init_tour));
     case Solvers::AntColony: { // mod.rs:1706-1711: options validated, then ant_colony::solve
@@ -1459,7 +1476,11 @@ Result<AppOptions> provide(const TomlTable &table, AppOptions base)
                 if (ckv.first == "mode" && s) base.cuda_mode = *s;
                 else if (ckv.first == "path" && s) base.cuda_path = *s;
                 else if (ckv.first == "seed" && iv) base.cuda_seed = (uint64_t)*iv;
-                else return Result<AppOptions>::err("config: unknown field `" + ckv.first + "` in [cuda] — valid: mode, path (strings), seed (integer)");
+                else if (ckv.first == "candidates" && iv) {
+                    if (*iv < 1 || *iv > 32) return Result<AppOptions>::err("config: [cuda] candidates must be in 1..32");
+                    base.cuda_candidates = (uint32_t)*iv;
+                }
+                else return Result<AppOptions>::err("config: unknown field `" + ckv.first + "` in [cuda] — valid: mode, path (strings), seed, candidates (integers)");
             }
         } else {
             return Result<AppOptions>::err("config: unknown field `" + key +

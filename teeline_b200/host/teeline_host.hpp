@@ -210,18 +210,22 @@ struct AppOptions { // mod.rs:1586-1596; only the sub-tables this path consumes 
     std::optional<AcoOptions> aco;
     std::optional<GAOptions> ga;
     // extension table [stage.cuda] (never required): mode = "ref"|"best", path = "auto"|"matrix"|"recompute",
-    // seed = <integer> (the population solvers' Philox key; the reference's RNG is unseeded)
+    // seed = <integer> (the population solvers' Philox key; the reference's RNG is unseeded),
+    // candidates = <integer> (mode "neighbor": k of the candidate lists, 1..32; 0 = TL_CANDIDATES_DEFAULT)
     std::string cuda_mode, cuda_path;
     uint64_t cuda_seed = 0;
+    uint32_t cuda_candidates = 0;
 };
 
 // ---- solvers (same free-function convention as the reference) ------------------------------------
 namespace two_opt {
 Solution solve(const TspProblem &problem, const HeuristicOptions &opts, const ProgressSender *progress_tx,
                const std::vector<size_t> *init_tour);
-// extension: best-improvement mode / explicit path selection ("ref"|"best", "auto"|"matrix"|"recompute")
+// extension: best-improvement mode / explicit path selection ("ref"|"best"|"best_cyclic"|"neighbor",
+// "auto"|"matrix"|"recompute"); candidates: k of mode "neighbor" (0 = the library's default)
 Solution solve_with(const TspProblem &problem, const std::string &mode, const std::string &path,
-                    const ProgressSender *progress_tx, const std::vector<size_t> *init_tour);
+                    const ProgressSender *progress_tx, const std::vector<size_t> *init_tour,
+                    uint32_t candidates = 0);
 }
 namespace or_opt {
 Solution solve(const TspProblem &problem, const HeuristicOptions &opts, const ProgressSender *progress_tx,
