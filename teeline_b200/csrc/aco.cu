@@ -64,7 +64,7 @@ extern "C" tl_status tl_aco(tl_problem *p, const tl_aco_options *o, const uint32
     if (e == cudaSuccess) e = cudaMemsetAsync(d_impr.p, 0, 8, st);
     if (e == cudaSuccess) e = cudaEventRecord(e0, st);
     // cost of the seed tour: the exact-order sum (distances.tour_length_by_pos)
-    launch_tour_lengths_f32(p->d_xy, p->d_tri, n, d_best.p, 1, p->fast_sqrt, false, d_cost1.p, c->sm_count, st);
+    launch_tour_lengths_f32(p->d_xy, p->d_tri, n, d_best.p, 1, p->metric == Metric::F32_FAST, false, d_cost1.p, c->sm_count, st);
     c->launches++;
     float best_cost = 0.0f;
     if (e == cudaSuccess) e = cudaMemcpyAsync(&best_cost, d_cost1.p, 4, cudaMemcpyDeviceToHost, st);
@@ -84,7 +84,7 @@ extern "C" tl_status tl_aco(tl_problem *p, const tl_aco_options *o, const uint32
         const float tau_min = tau0 * 1e-4f; // TAU_MIN_RATIO
         const float keep = 1.0f - o->evaporation_rate;
         launch_aco_fill(d_ph.p, nn, tau0, c->sm_count, st);
-        launch_aco_eta(p->d_xy, p->d_tri, n, p->fast_sqrt, o->beta, d_eta.p, c->sm_count, st);
+        launch_aco_eta(p->d_xy, p->d_tri, n, p->metric == Metric::F32_FAST, o->beta, d_eta.p, c->sm_count, st);
         c->launches += 2;
         if (init_tour) { // deposit_tour(best_pos_seed, best_cost), ant_colony.rs:176-178
             launch_aco_update(d_ph.p, n, nullptr, nullptr, 0, d_best.p, d_cost1.p, d_impr.p, st);
@@ -93,7 +93,7 @@ extern "C" tl_status tl_aco(tl_problem *p, const tl_aco_options *o, const uint32
         for (uint32_t epoch = 0; epoch < o->epochs && e == cudaSuccess; ++epoch) {
             launch_aco_weights(d_ph.p, d_eta.p, nn, o->alpha, d_w.p, c->sm_count, st);
             e = launch_aco_construct(d_w.p, d_eta.p, n, o->num_ants, epoch, o->seed, d_tours.p, st);
-            launch_tour_lengths_f32(p->d_xy, p->d_tri, n, d_tours.p, o->num_ants, p->fast_sqrt, false, d_costs.p,
+            launch_tour_lengths_f32(p->d_xy, p->d_tri, n, d_tours.p, o->num_ants, p->metric == Metric::F32_FAST, false, d_costs.p,
                                     c->sm_count, st);
             launch_aco_evaporate(d_ph.p, nn, keep, tau_min, c->sm_count, st);
             launch_aco_update(d_ph.p, n, d_tours.p, d_costs.p, o->num_ants, d_best.p, d_cost1.p, d_impr.p, st);

@@ -57,7 +57,7 @@ extern "C" tl_status tl_ga(tl_problem *p, const tl_ga_options *o, const uint32_t
     if (e == cudaSuccess) e = cudaEventRecord(e0, st);
     const uint32_t n_seeded = init_tour ? std::max(P / 5, 1u) : 0u; // from_cities_seeded (:207)
     if (e == cudaSuccess)
-        e = launch_ga_init(p->d_xy, p->d_tri, n, p->fast_sqrt, d_init.p, n_seeded, o->seed, d_pop[0].p, d_fit[0].p, st);
+        e = launch_ga_init(p->d_xy, p->d_tri, n, p->metric == Metric::F32_FAST, d_init.p, n_seeded, o->seed, d_pop[0].p, d_fit[0].p, st);
     c->launches++;
     // The Vec of individuals has L entries: n at first, and after every epoch elites + 2 * (n/2 - n_elite):
     // the reference's population SHRINKS by n_elite (+1 for odd n) in the first epoch and keeps that size
@@ -70,7 +70,7 @@ extern "C" tl_status tl_ga(tl_problem *p, const tl_ga_options *o, const uint32_t
         const uint32_t ne = std::min(o->n_elite, L);
         e = launch_ga_rank(d_fit[cur].p, L, d_order.p, d_sfit.p, st);
         if (e == cudaSuccess)
-            e = launch_ga_breed(p->d_xy, p->d_tri, n, p->fast_sqrt, L, ne, pairs, epoch, o->seed, o->mutation_probability,
+            e = launch_ga_breed(p->d_xy, p->d_tri, n, p->metric == Metric::F32_FAST, L, ne, pairs, epoch, o->seed, o->mutation_probability,
                                 d_pop[cur].p, d_order.p, d_sfit.p, d_pop[cur ^ 1].p, d_fit[cur ^ 1].p, d_mut.p, st);
         c->launches += 2;
         cur ^= 1;
@@ -83,7 +83,7 @@ extern "C" tl_status tl_ga(tl_problem *p, const tl_ga_options *o, const uint32_t
     unsigned long long mutations = 0;
     if (e == cudaSuccess && L > 0) {
         launch_ga_best(d_pop[cur].p, d_fit[cur].p, n, L, d_best.p, st);
-        launch_tour_lengths_f32(p->d_xy, p->d_tri, n, d_best.p, 1, p->fast_sqrt, false, d_cost.p, c->sm_count, st);
+        launch_tour_lengths_f32(p->d_xy, p->d_tri, n, d_best.p, 1, p->metric == Metric::F32_FAST, false, d_cost.p, c->sm_count, st);
         c->launches += 2;
         e = cudaEventRecord(e1, st);
         if (e == cudaSuccess) e = cudaMemcpyAsync(best_tour_out, d_best.p, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st);

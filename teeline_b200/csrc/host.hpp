@@ -7,9 +7,11 @@
 #include <new>
 #include <vector>
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -74,10 +76,10 @@ struct tl_problem {
     tl_ctx *ctx = nullptr;
     uint32_t n = 0;
     ProblemKind kind = PK_EUC_F32;
-    bool fast_sqrt = false; // coordinates guarantee dx^2+dy^2 in {0} U [2^-101, FLT_MAX]
-    bool grid_nint = false; // NINT problems: integer coordinates in the range of dist_nint_grid (common.cuh)
-    int nint_mode() const { return kind == PK_EUC_NINT ? (grid_nint ? 2 : 1) : 0; }
-    float dmax = 0.0f;      // upper bound on any city-to-city distance (bounding-box diagonal, rounded up)
+    tl::Metric metric = tl::Metric::F32_SAFE; // distance code of every kernel (api.cu); EXPLICIT problems keep F32_SAFE
+    // upper bound on any city-to-city distance (bounding-box diagonal, rounded up), set only when the
+    // coordinates are in the fast-sqrt domain (api.cu: coords_allow_fast_sqrt), else 0
+    float dmax = 0.0f;
     float2 *d_xy = nullptr; // city-ordered coordinates (coordinate problems)
     float *d_tri = nullptr; // packed triangle (EXPLICIT problems)
     uint32_t *d_cand = nullptr; // n x cand_k candidate lists for Mode N (tl_problem_set_candidates)
@@ -169,6 +171,14 @@ struct DevBuf {
     DevBuf(const DevBuf &) = delete;
     DevBuf &operator=(const DevBuf &) = delete;
 };
+
+// Margin of the screened scans (common.cuh: kScreenMarginScale), < 0 disables screening.  Screening
+// needs the fast-sqrt domain (dmax is 0 outside it) and a finite distance bound; TL_NO_SCREEN turns it off.
+inline float screen_margin(const tl_problem *p)
+{
+    const float m = p->dmax * kScreenMarginScale;
+    return (std::isfinite(m) && p->dmax >= kScreenMinDmax && !getenv("TL_NO_SCREEN")) ? m : -1.0f;
+}
 
 bool tour_is_permutation(const uint32_t *tour, uint32_t n);
 // K2-pop work decomposition (k2_two_opt_pop.cu): item count of one scan; fills band_first

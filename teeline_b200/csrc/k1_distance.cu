@@ -14,17 +14,15 @@
 
 namespace tl {
 
-// one matrix entry as raw bits: NINT = 0 f32 (FAST: guarded fast sqrt), 1 TSPLIB nint in double,
-// 2 TSPLIB nint for integer coordinates in 32-bit integer arithmetic (common.cuh: dist_nint_grid)
-template <bool FAST, int NINT>
+// one matrix entry as raw bits (f32 bits or int32)
+template <Metric M>
 __device__ __forceinline__ uint32_t k1_dist(const float2 a, const float2 b)
 {
-    if constexpr (NINT == 2)
-        return (uint32_t)dist_nint_grid(a.x, a.y, b.x, b.y);
-    else if constexpr (NINT == 1)
-        return (uint32_t)dist_nint(a.x, a.y, b.x, b.y);
+    const MetricValue<M> d = dist<M>(a.x, a.y, b.x, b.y);
+    if constexpr (metric_is_int(M))
+        return (uint32_t)d;
     else
-        return __float_as_uint(dist_f32<FAST>(a.x, a.y, b.x, b.y));
+        return __float_as_uint(d);
 }
 
 __device__ __forceinline__ void packed_index_to_pair(uint64_t t, uint32_t &hi, uint32_t &lo)
@@ -44,7 +42,7 @@ __device__ __forceinline__ void packed_index_to_pair(uint64_t t, uint32_t &hi, u
 // and 4 consecutive entries per lane cost 8 wavefronts per 8-byte load instead of 2.  The (hi, lo)
 // pair of T is found once with the closed form and then advanced incrementally (rows are longer
 // than 1024 almost everywhere, so the wrap loop runs 0-1 times).
-template <bool FAST, int NINT>
+template <Metric M>
 __global__ void __launch_bounds__(256) k1_packed_kernel(const float2 *__restrict__ xy, uint32_t n,
                                                         uint64_t total, uint64_t per_cta,
                                                         void *__restrict__ out)
@@ -67,7 +65,7 @@ __global__ void __launch_bounds__(256) k1_packed_kernel(const float2 *__restrict
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 // the reference evaluates cities[hi].distance(cities[lo])
-                o[32 * e + lane] = k1_dist<FAST, NINT>(ph, pl[e]);
+                o[32 * e + lane] = k1_dist<M>(ph, pl[e]);
             }
         } else {
 #pragma unroll 1
@@ -80,7 +78,7 @@ __global__ void __launch_bounds__(256) k1_packed_kernel(const float2 *__restrict
                     ++h;
                 }
                 const float2 ph = __ldg(&xy[h]), pl = __ldg(&xy[l]);
-                o[k] = k1_dist<FAST, NINT>(ph, pl);
+                o[k] = k1_dist<M>(ph, pl);
             }
         }
         // 1024 entries ahead: row hi holds hi entries
@@ -100,7 +98,7 @@ __global__ void __launch_bounds__(256) k1_packed_kernel(const float2 *__restrict
 // stores it with 128-bit stores, and stores its transpose, staged through shared memory, as tile
 // (bj, bi).  Half the arithmetic of the round-1 kernel (which was issue-bound for the nint metric:
 // 141 us for the 10k x 10k int32 matrix against a 61 us write floor) for the same bytes written.
-template <bool FAST, int NINT>
+template <Metric M>
 __global__ void __launch_bounds__(256) k1_square_kernel(const float2 *__restrict__ sxy, uint32_t n,
                                                         uint32_t ld, void *__restrict__ out)
 {
@@ -108,7 +106,7 @@ __global__ void __launch_bounds__(256) k1_square_kernel(const float2 *__restrict
     __shared__ uint32_t tile[64][65];
     const uint32_t tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
     const uint32_t col0 = blockIdx.x * 64 + tx * 4, row0 = blockIdx.y * 64 + ty * 4;
-    uint32_t *M = reinterpret_cast<uint32_t *>(out);
+    uint32_t *mat = reinterpret_cast<uint32_t *>(out);
     float2 c[4], r[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
@@ -123,12 +121,12 @@ __global__ void __launch_bounds__(256) k1_square_kernel(const float2 *__restrict
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
             const uint32_t cc = col0 + e;
-            const uint32_t d = k1_dist<FAST, NINT>(r[a], c[e]);
+            const uint32_t d = k1_dist<M>(r[a], c[e]);
             v[e] = (cc >= n || rr >= n || cc == rr) ? 0u : d;
             if (mirror) tile[ty * 4 + a][tx * 4 + e] = v[e];
         }
         if (rr < n && col0 < ld)
-            *reinterpret_cast<uint4 *>(M + (size_t)rr * ld + col0) = make_uint4(v[0], v[1], v[2], v[3]);
+            *reinterpret_cast<uint4 *>(mat + (size_t)rr * ld + col0) = make_uint4(v[0], v[1], v[2], v[3]);
     }
     if (!mirror) return;
     __syncthreads();
@@ -140,7 +138,7 @@ __global__ void __launch_bounds__(256) k1_square_kernel(const float2 *__restrict
         const uint32_t trow = blockIdx.x * 64 + ty * 4 + a;
         if (trow < n && tcol0 < ld) {
             const uint32_t lr = ty * 4 + a; // local column of the computed tile
-            *reinterpret_cast<uint4 *>(M + (size_t)trow * ld + tcol0) =
+            *reinterpret_cast<uint4 *>(mat + (size_t)trow * ld + tcol0) =
                 make_uint4(tile[tx * 4 + 0][lr], tile[tx * 4 + 1][lr], tile[tx * 4 + 2][lr], tile[tx * 4 + 3][lr]);
         }
     }
@@ -178,8 +176,7 @@ __global__ void __launch_bounds__(256) k1_square_from_packed_kernel(const uint32
 // ---------------------------------------------------------------------------
 // host launchers
 // ---------------------------------------------------------------------------
-void launch_k1_packed(const float2 *xy, uint32_t n, bool fast, int nint, void *out, int sm_count,
-                      cudaStream_t st)
+void launch_k1_packed(const float2 *xy, uint32_t n, Metric metric, void *out, int sm_count, cudaStream_t st)
 {
     const uint64_t total = (uint64_t)n * (n - 1) / 2;
     // a multiple of the SM count, at least 4 steps of 1024 entries per CTA when there is enough work
@@ -188,31 +185,16 @@ void launch_k1_packed(const float2 *xy, uint32_t n, bool fast, int nint, void *o
     if (per_cta < 4096) per_cta = 4096;
     blocks = (total + per_cta - 1) / per_cta;
     if (blocks == 0) blocks = 1;
-    if (nint == 2)
-        k1_packed_kernel<false, 2><<<(unsigned)blocks, 256, 0, st>>>(xy, n, total, per_cta, out);
-    else if (nint)
-        k1_packed_kernel<false, 1><<<(unsigned)blocks, 256, 0, st>>>(xy, n, total, per_cta, out);
-    else if (fast)
-        k1_packed_kernel<true, 0><<<(unsigned)blocks, 256, 0, st>>>(xy, n, total, per_cta, out);
-    else
-        k1_packed_kernel<false, 0><<<(unsigned)blocks, 256, 0, st>>>(xy, n, total, per_cta, out);
+    with_metric(metric, [&](auto M) { k1_packed_kernel<M><<<(unsigned)blocks, 256, 0, st>>>(xy, n, total, per_cta, out); });
 }
 
-void launch_k1_square(const float2 *sxy, uint32_t n, uint32_t ld, bool fast, int nint, void *out,
-                      cudaStream_t st)
+void launch_k1_square(const float2 *sxy, uint32_t n, uint32_t ld, Metric metric, void *out, cudaStream_t st)
 {
     // tiles of 64 x 64; the column blocks cover the padded width ld, the row blocks the n rows; the
     // grid is square so that every tile below the diagonal has a mirror above it
     const unsigned nb = (std::max(ld, n) + 63) / 64;
     dim3 grid(nb, nb);
-    if (nint == 2)
-        k1_square_kernel<false, 2><<<grid, 256, 0, st>>>(sxy, n, ld, out);
-    else if (nint)
-        k1_square_kernel<false, 1><<<grid, 256, 0, st>>>(sxy, n, ld, out);
-    else if (fast)
-        k1_square_kernel<true, 0><<<grid, 256, 0, st>>>(sxy, n, ld, out);
-    else
-        k1_square_kernel<false, 0><<<grid, 256, 0, st>>>(sxy, n, ld, out);
+    with_metric(metric, [&](auto M) { k1_square_kernel<M><<<grid, 256, 0, st>>>(sxy, n, ld, out); });
 }
 
 void launch_k1_square_from_packed(const uint32_t *tri, const int32_t *slot_city, uint32_t n,

@@ -18,7 +18,6 @@
 // The records, pos[] and the candidate lists (16 + 4 + 4k bytes per city) fit L2 up to about 10^6
 // cities, so the scan is a chain of dependent L2 gathers.
 #include "kernels.cuh"
-#include "policy.cuh"
 #include "two_opt_apply.cuh"
 
 #include <math_constants.h>
@@ -30,37 +29,26 @@ namespace {
 constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
 
-// Pt records with the TSPLIB nint metric recomputed from the coordinates (bit-equal to K1's matrix
-// entries, as in the persistent Mode R kernel); the entering-edge length is stored as int32 bits.
-template <bool GRID>
-struct EucNintPol {
-    using V = int32_t;
+// Pt records with distances recomputed from the coordinates in metric M (the nint metrics bit-equal to
+// K1's matrix entries, as in the persistent Mode R kernel); the entering-edge length is stored as the
+// bits of the metric's value type.
+template <Metric M>
+struct NlPol {
+    using V = MetricValue<M>;
     using Rec = Pt;
     Pt *pts;
     __device__ __forceinline__ Rec load(uint32_t q) const { return pts[q]; }
-    static __device__ __forceinline__ V sp(const Rec &r) { return __float_as_int(r.sp); }
+    static __device__ __forceinline__ V sp(const Rec &r) { return Val<V>::from_bits(__float_as_int(r.sp)); }
     static __device__ __forceinline__ int32_t city(const Rec &r) { return r.city; }
-    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const
-    {
-        return GRID ? dist_nint_grid(a.x, a.y, b.x, b.y) : dist_nint(a.x, a.y, b.x, b.y);
-    }
+    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const { return tl::dist<M>(a.x, a.y, b.x, b.y); }
     __device__ __forceinline__ void store_id(uint32_t q, const Rec &from) const
     {
         pts[q].x = from.x;
         pts[q].y = from.y;
         pts[q].city = from.city;
     }
-    __device__ __forceinline__ void store_sp(uint32_t q, V v) const { pts[q].sp = __int_as_float(v); }
+    __device__ __forceinline__ void store_sp(uint32_t q, V v) const { pts[q].sp = __int_as_float(Val<V>::bits(v)); }
 };
-
-// metric: 0 = f32 guarded fast sqrt, 1 = f32 IEEE sqrt, 2 = nint for integer coordinates, 3 = nint in f64
-#define TL_NL_DISPATCH(metric, pts, ...)                                      \
-    switch (metric) {                                                         \
-    case 0: { EucPol<true> P{pts}; __VA_ARGS__; } break;                      \
-    case 1: { EucPol<false> P{pts}; __VA_ARGS__; } break;                     \
-    case 2: { EucNintPol<true> P{pts}; __VA_ARGS__; } break;                  \
-    default: { EucNintPol<false> P{pts}; __VA_ARGS__; } break;                \
-    }
 
 // Tail of a fused step, run by the last CTA: reduce the per-CTA records, count the step's evaluated
 // pairs, then either reverse a short segment here and finish the step, or leave a long one pending.
@@ -212,14 +200,14 @@ __global__ void __launch_bounds__(256)
 
 } // namespace
 
-void launch_nl_init(int metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
+void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
                     uint32_t *pos, cudaStream_t st)
 {
     const int grid = (int)((npad + 255) / 256);
-    TL_NL_DISPATCH(metric, pts, (nl_init_kernel<<<grid, 256, 0, st>>>(P, xy, tour, n, npad, pos)));
+    with_metric(metric, [&](auto M) { nl_init_kernel<<<grid, 256, 0, st>>>(NlPol<M>{pts}, xy, tour, n, npad, pos); });
 }
 
-void launch_nl_scan(int metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
+void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
                     DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
                     cudaStream_t st)
 {
@@ -233,13 +221,15 @@ void launch_nl_scan(int metric, Pt *pts, uint32_t *pos, const uint32_t *cand, ui
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     const int fuse = fuse_apply ? 1 : 0;
-    TL_NL_DISPATCH(metric, pts,
-                   (cudaLaunchKernelEx(&cfg, two_opt_nl_scan_kernel<decltype(P)>, P, pos, cand, k, n,
-                                       reinterpret_cast<Best<typename decltype(P)::V> *>(blockbest), state, ticket,
-                                       log, (uint64_t)log_cap, fuse)));
+    with_metric(metric, [&](auto M) {
+        using Pol = NlPol<M>;
+        cudaLaunchKernelEx(&cfg, two_opt_nl_scan_kernel<Pol>, Pol{pts}, pos, cand, k, n,
+                           reinterpret_cast<Best<typename Pol::V> *>(blockbest), state, ticket, log, (uint64_t)log_cap,
+                           fuse);
+    });
 }
 
-void launch_nl_apply(int metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
+void launch_nl_apply(Metric metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
                      tl_move *log, uint64_t log_cap, int grid, cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
@@ -251,10 +241,11 @@ void launch_nl_apply(int metric, Pt *pts, uint32_t *pos, const void *pending, De
     cfg.stream = st;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    TL_NL_DISPATCH(metric, pts,
-                   (cudaLaunchKernelEx(&cfg, apply_two_opt_kernel<decltype(P)>, P,
-                                       reinterpret_cast<const Best<typename decltype(P)::V> *>(pending), 1, state,
-                                       ticket, log, (uint64_t)log_cap, pos, 1)));
+    with_metric(metric, [&](auto M) {
+        using Pol = NlPol<M>;
+        cudaLaunchKernelEx(&cfg, apply_two_opt_kernel<Pol>, Pol{pts}, reinterpret_cast<const Best<typename Pol::V> *>(pending),
+                           1, state, ticket, log, (uint64_t)log_cap, pos, 1);
+    });
 }
 
 } // namespace tl

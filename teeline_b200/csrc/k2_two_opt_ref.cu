@@ -186,14 +186,13 @@ __device__ __forceinline__ void cluster_barrier()
 // Tour records in shared memory as arrays (x, y, city, entering-edge length [, matrix slot]): a warp's
 // column loads and the reversal's stores touch consecutive words (conflict-free), and a load that
 // needs only some fields costs only those.  Same interface as EucPol / MatPol (policy.cuh).
-// METRIC: 0 = f32 guarded fast sqrt, 1 = f32 safe sqrt, 2 = TSPLIB nint for integer coordinates
-// (FP64-free, common.cuh: dist_nint_grid), 3 = TSPLIB nint in double.  The nint metrics belong to
-// matrix sessions: the kernel recomputes the matrix entries from the coordinates (bit-equal by K1's
-// construction) and carries every city's matrix slot along so that the Cs records can be restored.
-template <int METRIC>
+// Distances are recomputed in metric M.  The nint metrics belong to matrix sessions: the kernel
+// recomputes the matrix entries from the coordinates (bit-equal by K1's construction) and carries
+// every city's matrix slot along so that the Cs records can be restored.
+template <Metric M>
 struct SmemSoaPol {
-    static constexpr bool kInt = METRIC >= 2;
-    using V = typename std::conditional<kInt, int32_t, float>::type;
+    static constexpr bool kInt = metric_is_int(M);
+    using V = MetricValue<M>;
     struct Rec {
         float x, y;
         int32_t city, slot;
@@ -206,13 +205,7 @@ struct SmemSoaPol {
         return Rec{x[q], y[q], cty[q], kInt ? slt[q] : 0, Val<V>::from_bits(spl[q])};
     }
     static __device__ __forceinline__ V sp(const Rec &r) { return r.sp; }
-    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const
-    {
-        if constexpr (METRIC == 0) return dist_f32<true>(a.x, a.y, b.x, b.y);
-        else if constexpr (METRIC == 1) return dist_f32<false>(a.x, a.y, b.x, b.y);
-        else if constexpr (METRIC == 2) return dist_nint_grid(a.x, a.y, b.x, b.y);
-        else return dist_nint(a.x, a.y, b.x, b.y);
-    }
+    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const { return tl::dist<M>(a.x, a.y, b.x, b.y); }
     __device__ __forceinline__ void store_id(uint32_t q, const Rec &from) const
     {
         x[q] = from.x;
@@ -227,13 +220,13 @@ struct SmemSoaPol {
 // a warp loads the 32 column records once and evaluates RB pairs per lane.
 // key = (row in window) << 14 | column orders the window's pairs lexicographically; the cluster-wide
 // minimum key is the reference's next move.
-template <int METRIC, bool SCREEN>
+template <Metric M, bool SCREEN>
 __global__ void __launch_bounds__(kRefPThreads, 1)
     ref_persistent_kernel(Pt *__restrict__ pts, Cs *__restrict__ cs, const float2 *__restrict__ xy, uint32_t n,
                           DevState *state, tl_move *__restrict__ log, uint64_t log_cap, uint32_t max_steps,
                           float margin)
 {
-    using Pol = SmemSoaPol<METRIC>;
+    using Pol = SmemSoaPol<M>;
     using V = typename Pol::V;
     using Rec = typename Pol::Rec;
     constexpr bool kInt = Pol::kInt;
@@ -501,39 +494,27 @@ namespace tl {
 // The persistent form: one cluster of `csize` CTAs (16 needs the non-portable opt-in; 8 otherwise).
 namespace {
 using RefPFn = void (*)(Pt *, Cs *, const float2 *, uint32_t, DevState *, tl_move *, uint64_t, uint32_t, float);
-RefPFn refp_fn(int metric, bool screen)
+RefPFn refp_fn(Metric metric, bool screen)
 {
-    switch (metric) {
-    case 0: return screen ? ref_persistent_kernel<0, true> : ref_persistent_kernel<0, false>;
-    case 1: return ref_persistent_kernel<1, false>; // no screening outside the fast-sqrt domain
-    case 2: return screen ? ref_persistent_kernel<2, true> : ref_persistent_kernel<2, false>;
-    default: return screen ? ref_persistent_kernel<3, true> : ref_persistent_kernel<3, false>;
-    }
+    return with_metric(metric, [&](auto M) -> RefPFn {
+        if constexpr (M == Metric::F32_SAFE) return ref_persistent_kernel<M, false>; // no screening outside the fast-sqrt domain
+        else return screen ? ref_persistent_kernel<M, true> : ref_persistent_kernel<M, false>;
+    });
 }
-// 0/1: f32 coordinate sessions; 2/3: nint matrix sessions of coordinate problems (xy given); -1: none
-int refp_metric(const Src &src, const float2 *xy, int nint_mode)
-{
-    if (src.kind == SRC_EUC_FAST) return 0;
-    if (src.kind == SRC_EUC_SAFE) return 1;
-    if (src.kind == SRC_MAT_I32 && xy && nint_mode == 2) return 2;
-    if (src.kind == SRC_MAT_I32 && xy && nint_mode == 1) return 3;
-    return -1;
-}
-size_t refp_smem_bytes(int metric, uint32_t n) { return (size_t)((n + 3u) & ~3u) * (metric >= 2 ? 20 : 16); }
+size_t refp_smem_bytes(Metric metric, uint32_t n) { return (size_t)((n + 3u) & ~3u) * (metric_is_int(metric) ? 20 : 16); }
 } // namespace
 
 // Returns the cluster size this device can run for n records, 0 if the form does not apply.
-int ref_persistent_cluster_size(const Src &src, const float2 *xy, int nint_mode, uint32_t n)
+int ref_persistent_cluster_size(std::optional<Metric> metric, uint32_t n)
 {
-    const int metric = refp_metric(src, xy, nint_mode);
-    if (metric < 0 || n < 4 || n > (uint32_t)(metric >= 2 ? kRefPersistMaxNInt : kRefPersistMaxN)) return 0;
+    if (!metric || n < 4 || n > (uint32_t)(metric_is_int(*metric) ? kRefPersistMaxNInt : kRefPersistMaxN)) return 0;
     static int cached_size = -1; // every instantiation has the same shape; the answer for the largest n holds for every n
     if (cached_size >= 0) return cached_size;
     const size_t smem = (size_t)kRefPersistMaxN * 16;
     static_assert((size_t)kRefPersistMaxNInt * 20 <= (size_t)kRefPersistMaxN * 16, "one shared-memory opt-in for all");
     int best = 0;
     bool ok = true;
-    for (int m = 0; m < 4; ++m)
+    for (Metric m : kMetrics)
         for (int sc = 0; sc < 2; ++sc)
             ok = ok && cudaFuncSetAttribute((const void *)refp_fn(m, sc != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess &&
                  cudaFuncSetAttribute((const void *)refp_fn(m, sc != 0), cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
@@ -551,7 +532,7 @@ int ref_persistent_cluster_size(const Src &src, const float2 *xy, int nint_mode,
             cfg.attrs = attr;
             cfg.numAttrs = 1;
             int nclusters = 0;
-            if (cudaOccupancyMaxActiveClusters(&nclusters, (const void *)refp_fn(2, true), &cfg) == cudaSuccess && nclusters >= 1) {
+            if (cudaOccupancyMaxActiveClusters(&nclusters, (const void *)refp_fn(Metric::NINT_GRID, true), &cfg) == cudaSuccess && nclusters >= 1) {
                 best = cs;
                 break;
             }
@@ -570,10 +551,9 @@ int ref_persistent_cluster_size(const Src &src, const float2 *xy, int nint_mode,
 
 // screen_margin >= 0 (fast-sqrt domain only, common.cuh: kScreenMarginScale): screened distances first;
 // the nint metrics add the two roundings to integers (1.0) to it
-void launch_ref_persistent(const Src &src, const float2 *xy, int nint_mode, uint32_t n, DevState *state, tl_move *log,
+void launch_ref_persistent(const Src &src, const float2 *xy, Metric metric, uint32_t n, DevState *state, tl_move *log,
                            uint64_t log_cap, uint32_t max_steps, int csize, float screen_margin, cudaStream_t st)
 {
-    const int metric = refp_metric(src, xy, nint_mode);
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = (unsigned)csize;
@@ -586,8 +566,8 @@ void launch_ref_persistent(const Src &src, const float2 *xy, int nint_mode, uint
     cfg.stream = st;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    const bool screen = screen_margin >= 0.0f && metric != 1;
-    const float margin = screen ? (metric >= 2 ? screen_margin + 1.0009765625f : screen_margin) : -1.0f;
+    const bool screen = screen_margin >= 0.0f && metric != Metric::F32_SAFE;
+    const float margin = screen ? (metric_is_int(metric) ? screen_margin + 1.0009765625f : screen_margin) : -1.0f;
     cudaLaunchKernelEx(&cfg, refp_fn(metric, screen), src.pts, src.cs, xy, n, state, log, (uint64_t)log_cap, max_steps, margin);
 }
 

@@ -26,18 +26,9 @@ namespace {
 
 constexpr int kTile = 1024;
 
-// METRIC: 0 = f32 metric with the guarded fast sqrt, 1 = f32 metric with the IEEE-safe sqrt,
-// 2 = TSPLIB nint metric (converted to f32: exact while distances stay below 2^24), 3 = the same
-// integers from dist_nint_grid (integer coordinates, no FP64: common.cuh).
-template <int METRIC>
-__device__ __forceinline__ float metric(float x1, float y1, float x2, float y2)
-{
-    if (METRIC == 3) return (float)dist_nint_grid(x1, y1, x2, y2);
-    if (METRIC == 2) return (float)dist_nint(x1, y1, x2, y2);
-    return dist_f32<METRIC == 0>(x1, y1, x2, y2);
-}
-
-template <int METRIC, int K>
+// Distances are compared as f32: the nint metrics' integers are exact there while distances stay
+// below 2^24 (api.cu checks this for NINT problems).
+template <Metric M, int K>
 __global__ void __launch_bounds__(256)
     knn_kernel(const float2 *__restrict__ xy, uint32_t n, uint32_t k, uint32_t *__restrict__ out)
 {
@@ -82,14 +73,14 @@ __global__ void __launch_bounds__(256)
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     const float2 pc = tile[t + u];
-                    d[u] = metric<METRIC>(pq.x, pq.y, pc.x, pc.y);
+                    d[u] = (float)dist<M>(pq.x, pq.y, pc.x, pc.y);
                 }
 #pragma unroll
                 for (int u = 0; u < 4; ++u) offer(c0 + t + u, d[u]);
             }
             for (; t < cnt; ++t) {
                 const float2 pc = tile[t];
-                offer(c0 + t, metric<METRIC>(pq.x, pq.y, pc.x, pc.y));
+                offer(c0 + t, (float)dist<M>(pq.x, pq.y, pc.x, pc.y));
             }
         }
     }
@@ -145,7 +136,7 @@ __global__ void __launch_bounds__(256)
 // ballot per step, ~100 cycles), entries ks..kk-1 are looked up in global memory only when those
 // are all visited, and the other 31 warps wait at the barrier until a step needs the block-wide
 // argmin (every listed neighbour visited) -- 8.3 ms -> see profiles for n = 10 000.
-template <int METRIC>
+template <Metric M>
 __global__ void __launch_bounds__(1024)
     nn_tour_kernel(const float2 *__restrict__ xy, const float *__restrict__ tri, uint32_t n,
                    const uint32_t *__restrict__ knn, uint32_t kk, uint32_t ks, uint32_t *__restrict__ tour)
@@ -219,7 +210,7 @@ __global__ void __launch_bounds__(1024)
                     d = __ldg(&tri[hi * (hi - 1) / 2 + lo]);
                 } else {
                     const float2 p = xy[c];
-                    d = metric<METRIC>(pc.x, pc.y, p.x, p.y);
+                    d = (float)dist<M>(pc.x, pc.y, p.x, p.y);
                 }
                 if (bc == 0xffffffffu || d < bd) { bd = d; bc = c; } // c ascending within a thread
             }
@@ -252,7 +243,7 @@ __global__ void __launch_bounds__(1024)
     }
 }
 
-template <int METRIC>
+template <Metric M>
 void launch_knn_k(const float2 *xy, uint32_t n, uint32_t k, uint32_t *out, cudaStream_t st)
 {
     // one thread per query: a query's time is n candidates long whatever the grid, so small
@@ -260,18 +251,18 @@ void launch_knn_k(const float2 *xy, uint32_t n, uint32_t k, uint32_t *out, cudaS
     const int threads = n >= 148u * 256u ? 256 : (n >= 148u * 128u ? 128 : 64);
     const int grid = (int)((n + threads - 1) / threads);
     if (k <= 4)
-        knn_kernel<METRIC, 4><<<grid, threads, 0, st>>>(xy, n, k, out);
+        knn_kernel<M, 4><<<grid, threads, 0, st>>>(xy, n, k, out);
     else if (k <= 8)
-        knn_kernel<METRIC, 8><<<grid, threads, 0, st>>>(xy, n, k, out);
+        knn_kernel<M, 8><<<grid, threads, 0, st>>>(xy, n, k, out);
     else if (k <= 16)
-        knn_kernel<METRIC, 16><<<grid, threads, 0, st>>>(xy, n, k, out);
+        knn_kernel<M, 16><<<grid, threads, 0, st>>>(xy, n, k, out);
     else
-        knn_kernel<METRIC, 32><<<grid, threads, 0, st>>>(xy, n, k, out);
+        knn_kernel<M, 32><<<grid, threads, 0, st>>>(xy, n, k, out);
 }
 
 } // namespace
 
-void launch_knn(const float2 *xy, const float *tri, uint32_t n, uint32_t k, int metric_id, uint32_t *out,
+void launch_knn(const float2 *xy, const float *tri, uint32_t n, uint32_t k, Metric metric, uint32_t *out,
                 cudaStream_t st)
 {
     if (tri) {
@@ -284,14 +275,8 @@ void launch_knn(const float2 *xy, const float *tri, uint32_t n, uint32_t k, int 
             knn_packed_kernel<16><<<grid, 256, 0, st>>>(tri, n, k, out);
         else
             knn_packed_kernel<32><<<grid, 256, 0, st>>>(tri, n, k, out);
-    } else if (metric_id == 0) {
-        launch_knn_k<0>(xy, n, k, out, st);
-    } else if (metric_id == 1) {
-        launch_knn_k<1>(xy, n, k, out, st);
-    } else if (metric_id == 3) {
-        launch_knn_k<3>(xy, n, k, out, st);
     } else {
-        launch_knn_k<2>(xy, n, k, out, st);
+        with_metric(metric, [&](auto M) { launch_knn_k<M>(xy, n, k, out, st); });
     }
 }
 
@@ -310,26 +295,20 @@ static uint32_t nn_tour_heads(uint32_t n, uint32_t kk)
 
 cudaError_t nn_tour_configure()
 {
-    cudaError_t e = cudaFuncSetAttribute(nn_tour_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(nn_tour_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(nn_tour_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(nn_tour_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaError_t e = cudaSuccess;
+    for (Metric m : kMetrics)
+        if (e == cudaSuccess)
+            e = with_metric(m, [](auto M) { return cudaFuncSetAttribute(nn_tour_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
     return e;
 }
 
 void launch_nn_tour(const float2 *xy, const float *tri, uint32_t n, const uint32_t *knn, uint32_t kk,
-                    int metric_id, uint32_t *tour, cudaStream_t st)
+                    Metric metric, uint32_t *tour, cudaStream_t st)
 {
     const uint32_t ks = getenv("TL_NN_NO_HEADS") ? 0 : nn_tour_heads(n, kk);
     const size_t smem = nn_tour_smem_bytes(n) + (size_t)n * ks * 2;
-    if (metric_id == 0)
-        nn_tour_kernel<0><<<1, 1024, smem, st>>>(xy, tri, n, knn, kk, ks, tour);
-    else if (metric_id == 1)
-        nn_tour_kernel<1><<<1, 1024, smem, st>>>(xy, tri, n, knn, kk, ks, tour);
-    else if (metric_id == 3)
-        nn_tour_kernel<3><<<1, 1024, smem, st>>>(xy, tri, n, knn, kk, ks, tour);
-    else
-        nn_tour_kernel<2><<<1, 1024, smem, st>>>(xy, tri, n, knn, kk, ks, tour);
+    // EXPLICIT problems (F32_SAFE) pass tri: the kernel reads the triangle instead of recomputing
+    with_metric(metric, [&](auto M) { nn_tour_kernel<M><<<1, 1024, smem, st>>>(xy, tri, n, knn, kk, ks, tour); });
 }
 
 } // namespace tl

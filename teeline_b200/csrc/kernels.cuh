@@ -1,5 +1,6 @@
 // kernels.cuh -- kernel-side types and host launcher prototypes (internal).
 #pragma once
+#include <optional>
 #include <vector>
 
 #include "common.cuh"
@@ -85,11 +86,8 @@ struct Src {
 // ---------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------
-// nint: 0 = f32 metric, 1 = TSPLIB nint through f64, 2 = TSPLIB nint in 32-bit integers (integer coordinates)
-void launch_k1_packed(const float2 *xy, uint32_t n, bool fast, int nint, void *out, int sm_count,
-                      cudaStream_t st);
-void launch_k1_square(const float2 *sxy, uint32_t n, uint32_t ld, bool fast, int nint, void *out,
-                      cudaStream_t st);
+void launch_k1_packed(const float2 *xy, uint32_t n, Metric metric, void *out, int sm_count, cudaStream_t st);
+void launch_k1_square(const float2 *sxy, uint32_t n, uint32_t ld, Metric metric, void *out, cudaStream_t st);
 void launch_k1_square_from_packed(const uint32_t *tri, const int32_t *slot_city, uint32_t n,
                                   uint32_t ld, uint32_t *out, cudaStream_t st);
 
@@ -130,11 +128,12 @@ void launch_ref_step(const Src &src, uint32_t n, DevState *state, unsigned int *
                      uint64_t log_cap, int grid, cudaStream_t st);
 // persistent form: one thread-block cluster runs up to max_steps cursor steps from shared memory.
 // f32 coordinate sessions, and nint matrix sessions of coordinate problems (xy = city-ordered
-// coordinates, nint_mode as tl_problem::nint_mode(): the entries are recomputed, bit-equal to K1's)
+// coordinates: the entries are recomputed in the problem's metric, bit-equal to K1's).  metric: the
+// session's metric, none for sessions that read f32 matrix entries (f32 matrix, EXPLICIT)
 constexpr int kRefPersistMaxN = 14000;    // 16 bytes per position of the whole tour in one SM's shared memory
 constexpr int kRefPersistMaxNInt = 11000; // 20 bytes per position (the matrix slot travels with the city)
-int ref_persistent_cluster_size(const Src &src, const float2 *xy, int nint_mode, uint32_t n);
-void launch_ref_persistent(const Src &src, const float2 *xy, int nint_mode, uint32_t n, DevState *state, tl_move *log,
+int ref_persistent_cluster_size(std::optional<Metric> metric, uint32_t n);
+void launch_ref_persistent(const Src &src, const float2 *xy, Metric metric, uint32_t n, DevState *state, tl_move *log,
                            uint64_t log_cap, uint32_t max_steps, int csize, float screen_margin, cudaStream_t st);
 
 // K3 Or-opt (recompute path)
@@ -203,12 +202,13 @@ void launch_three_apply(const Src &src, void *tmp, uint32_t n, const void *cand,
                         cudaStream_t st);
 
 // K5 / N1
-void launch_knn(const float2 *xy, const float *tri, uint32_t n, uint32_t k, int metric_id, uint32_t *out,
+// tri non-null (EXPLICIT problems): distances from the packed triangle, else recomputed in `metric`
+void launch_knn(const float2 *xy, const float *tri, uint32_t n, uint32_t k, Metric metric, uint32_t *out,
                 cudaStream_t st);
 size_t nn_tour_smem_bytes(uint32_t n);
 cudaError_t nn_tour_configure();
 void launch_nn_tour(const float2 *xy, const float *tri, uint32_t n, const uint32_t *knn, uint32_t kk,
-                    int metric_id, uint32_t *tour, cudaStream_t st);
+                    Metric metric, uint32_t *tour, cudaStream_t st);
 
 // K2 matrix path
 constexpr int kMatR = 8;                 // diagonals per lane (strided by 32 => coalesced rows)
@@ -255,18 +255,18 @@ void launch_two_opt_cached_step(const Src &src, uint32_t n, int cyclic, unsigned
                                 int *fullrows, DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap,
                                 int grid, cudaStream_t st);
 
-// K2 candidate-list 2-opt, "Mode N" (k2_two_opt_neighbor.cu).  metric: 0 = f32 fast sqrt, 1 = f32 IEEE
-// sqrt, 2 = nint for integer coordinates, 3 = nint in f64.  blockbest holds grid + 1 records: one per
-// CTA and, at [grid], the step's pending long move for the apply grid.
+// K2 candidate-list 2-opt, "Mode N" (k2_two_opt_neighbor.cu): distances recomputed in the problem's
+// metric.  blockbest holds grid + 1 records: one per CTA and, at [grid], the step's pending long move
+// for the apply grid.
 constexpr int kNlThreads = 256;
 constexpr int kNlMinBlocks = 2;
 constexpr int kNlCtaSwaps = 2048; // segments of up to this many swapped pairs are reversed by the reducing CTA
-void launch_nl_init(int metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
+void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
                     uint32_t *pos, cudaStream_t st);
-void launch_nl_scan(int metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
+void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
                     DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
                     cudaStream_t st);
-void launch_nl_apply(int metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
+void launch_nl_apply(Metric metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
                      tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
 
 // K2-batch: one CTA per tour, tour records in shared memory

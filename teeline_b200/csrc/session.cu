@@ -81,7 +81,6 @@ struct tl_session {
     // candidate-list 2-opt (TL_ALGO_TWO_OPT_NEIGHBOR): Pt records plus pos[] and the session's own
     // copy of the problem's candidate lists
     bool nl = false;
-    int nl_metric = 0;               // k2_two_opt_neighbor.cu: 0/1 f32 fast/IEEE sqrt, 2/3 nint grid/f64
     DevBuf<uint32_t> pos;            // city -> position
     DevBuf<uint32_t> nl_cand;        // n x nl_k
     uint32_t nl_k = 0;
@@ -104,7 +103,13 @@ struct tl_session {
     double device_ms = 0.0;
 
     bool matrix() const { return path_used == TL_PATH_MATRIX; }
-    bool int_values() const { return nl ? nl_metric >= 2 : src.is_int(); }
+    bool int_values() const { return metric_is_int(p->metric); }
+    // the metric the persistent Mode R kernel recomputes distances in; none when the session reads f32
+    // matrix entries (f32 matrix and EXPLICIT sessions)
+    std::optional<Metric> recompute_metric() const
+    {
+        return src.kind == SRC_MAT_F32 ? std::nullopt : std::optional<Metric>(p->metric);
+    }
 };
 
 namespace {
@@ -121,12 +126,7 @@ void build_geometry(tl_session *s, std::vector<int32_t> &band_first_h)
     g.cyclic = s->cyclic;
     g.jmax = s->cyclic ? n - 1 : n - 2;
     g.kmax = n - 2;
-    // screening needs the fast-sqrt domain and a finite distance bound (common.cuh)
-    const float margin = s->p->dmax * kScreenMarginScale;
-    g.screen_margin = (s->p->fast_sqrt && std::isfinite(margin) && s->p->dmax >= kScreenMinDmax &&
-                       !getenv("TL_NO_SCREEN"))
-                          ? margin
-                          : -1.0f;
+    g.screen_margin = screen_margin(s->p);
     g.nbands = (g.kmax - 2) / bw + 1;
     auto H = [&](int b) { return g.jmax - (2 + b * bw) + 1; };
     // one work item per resident warp, times the shard count so that every rank of a sharded
@@ -278,20 +278,19 @@ void build_matrix(tl_session *s, const uint32_t *d_tour)
                                      s->M.p, st);
     } else {
         launch_gather_slots(p->d_xy, d_tour, s->cs.p, s->n, s->sxy.p, nullptr, st);
-        launch_k1_square(s->sxy.p, s->n, s->ld, p->fast_sqrt, p->nint_mode(), s->M.p, st);
+        launch_k1_square(s->sxy.p, s->n, s->ld, p->metric, s->M.p, st);
         if (getenv("TL_K1_TIMING")) { // tuning aid: warm kernel time (CUDA events, 20 back-to-back launches) on stderr
             cudaEvent_t e0, e1;
             cudaEventCreate(&e0);
             cudaEventCreate(&e1);
             cudaEventRecord(e0, st);
-            for (int r = 0; r < 20; ++r) launch_k1_square(s->sxy.p, s->n, s->ld, p->fast_sqrt, p->nint_mode(), s->M.p, st);
+            for (int r = 0; r < 20; ++r) launch_k1_square(s->sxy.p, s->n, s->ld, p->metric, s->M.p, st);
             cudaEventRecord(e1, st);
             cudaEventSynchronize(e1);
             float ms = 0.f;
             cudaEventElapsedTime(&ms, e0, e1);
-            fprintf(stderr, "[tl] k1_square n=%u %s: %.2f us per launch, %.1f GB/s written\n", s->n,
-                    p->kind == PK_EUC_NINT ? (p->grid_nint ? "nint-int32" : "nint-f64") : "f32", ms / 20 * 1e3,
-                    (double)s->n * s->ld * 4.0 / (ms / 20 * 1e-3) / 1e9);
+            fprintf(stderr, "[tl] k1_square n=%u %s: %.2f us per launch, %.1f GB/s written\n", s->n, metric_name(p->metric),
+                    ms / 20 * 1e3, (double)s->n * s->ld * 4.0 / (ms / 20 * 1e-3) / 1e9);
             cudaEventDestroy(e0);
             cudaEventDestroy(e1);
         }
@@ -360,7 +359,7 @@ tl_status launch_scan(tl_session *s, bool fuse, bool exchange = true)
     BestF *mine = s->cand.p + (size_t)s->shard_index * s->grid;
     cudaStream_t st = s->c->stream;
     if (s->nl) {
-        launch_nl_scan(s->nl_metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->cand.p, s->state.p,
+        launch_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->cand.p, s->state.p,
                        s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
         s->c->launches++;
     } else if (s->algo == TL_ALGO_THREE_OPT) {
@@ -404,11 +403,9 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
     if (s->algo == TL_ALGO_TWO_OPT_REF) {
         // coordinate problems whose records fit one SM's shared memory: the whole chain of `steps`
         // cursor steps in ONE launch of a thread-block cluster (k2_two_opt_ref.cu, persistent form)
-        if (const int csize = ref_persistent_cluster_size(s->src, s->p->d_xy, s->p->nint_mode(), s->n)) {
-            const float m = s->p->dmax * kScreenMarginScale;
-            const float margin = (s->p->fast_sqrt && std::isfinite(m) && s->p->dmax >= kScreenMinDmax && !getenv("TL_NO_SCREEN")) ? m : -1.0f;
-            launch_ref_persistent(s->src, s->p->d_xy, s->p->nint_mode(), s->n, s->state.p, s->log.p, s->log_cap, steps, csize,
-                                  margin, st);
+        if (const int csize = ref_persistent_cluster_size(s->recompute_metric(), s->n)) {
+            launch_ref_persistent(s->src, s->p->d_xy, s->p->metric, s->n, s->state.p, s->log.p, s->log_cap, steps, csize,
+                                  screen_margin(s->p), st);
             s->c->launches += 1;
             TL_CUDA_TRY(cudaGetLastError());
             return TL_OK;
@@ -443,7 +440,7 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
         if (rc != TL_OK) return rc;
         s->steps_since_permute++;
         if (s->nl) { // a long segment left pending by the scan's last CTA (none: the grid leaves at once)
-            launch_nl_apply(s->nl_metric, s->pts.p, s->pos.p, s->cand.p + s->grid, s->state.p, s->ticket.p + 1,
+            launch_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->cand.p + s->grid, s->state.p, s->ticket.p + 1,
                             s->log.p, s->log_cap, apply_grid, st);
             s->c->launches++;
             continue;
@@ -719,16 +716,16 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
             e = cudaMemcpyAsync(s->nl_cand.p, p->d_cand, (size_t)p->n * s->nl_k * 4, cudaMemcpyDeviceToDevice, c->stream);
             if (e != cudaSuccess) { set_error("tl_session_create: %s", cudaGetErrorString(e)); return fail(TL_ERR_CUDA); }
         }
-        s->nl_metric = p->kind == PK_EUC_NINT ? (p->grid_nint ? 2 : 3) : (p->fast_sqrt ? 0 : 1);
-        s->src.kind = p->fast_sqrt ? SRC_EUC_FAST : SRC_EUC_SAFE; // tl_session_tour reads the city fields only
+        s->src.kind = SRC_EUC_SAFE; // tl_session_tour reads the city fields only
         s->src.pts = s->pts.p;
-        launch_nl_init(s->nl_metric, p->d_xy, d_tour.p, p->n, s->npad, s->pts.p, s->pos.p, c->stream);
+        launch_nl_init(p->metric, p->d_xy, d_tour.p, p->n, s->npad, s->pts.p, s->pos.p, c->stream);
         c->launches++;
     } else {
         if (s->pts.alloc(s->npad) != cudaSuccess) { set_error("tl_session_create: device allocation failed"); return fail(TL_ERR_NOMEM); }
-        s->src.kind = p->fast_sqrt ? SRC_EUC_FAST : SRC_EUC_SAFE;
+        const bool fast = p->metric == Metric::F32_FAST;
+        s->src.kind = fast ? SRC_EUC_FAST : SRC_EUC_SAFE;
         s->src.pts = s->pts.p;
-        launch_build_pts(p->d_xy, d_tour.p, p->n, s->npad, s->cyclic, p->fast_sqrt, s->pts.p, c->stream);
+        launch_build_pts(p->d_xy, d_tour.p, p->n, s->npad, s->cyclic, fast, s->pts.p, c->stream);
         c->launches++;
     }
     memset(&s->h, 0, sizeof s->h);
@@ -948,7 +945,7 @@ tl_status tl_session_run(tl_session *s, int64_t max_moves)
         uint32_t batch = s->algo == TL_ALGO_TWO_OPT_REF ? 64 : 32;
         // Mode R, persistent form: a batch is one launch, so make it long (the kernel stops by itself
         // at convergence or at the move budget)
-        if (s->algo == TL_ALGO_TWO_OPT_REF && ref_persistent_cluster_size(s->src, s->p->d_xy, s->p->nint_mode(), s->n)) batch = 1u << 20;
+        if (s->algo == TL_ALGO_TWO_OPT_REF && ref_persistent_cluster_size(s->recompute_metric(), s->n)) batch = 1u << 20;
         if (budgeted) {
             batch = (uint32_t)std::min<int64_t>(256, budget);
             budget -= batch;
@@ -1136,6 +1133,7 @@ tl_status tl_two_opt_batch(tl_problem *p, int32_t algo, uint32_t *tours_inout, s
     DeviceGuard g(c);
     const uint32_t n = p->n;
     const bool cyclic = algo == TL_ALGO_TWO_OPT_BEST_CYCLIC;
+    const bool fast = p->metric == Metric::F32_FAST;
     const uint64_t launches0 = c->launches;
     DevBuf<uint32_t> d_t;
     DevBuf<float> d_len;
@@ -1160,9 +1158,7 @@ tl_status tl_two_opt_batch(tl_problem *p, int32_t algo, uint32_t *tours_inout, s
     DevBuf<int32_t> d_bands;
     DevBuf<unsigned long long> d_queue;
     if (e == cudaSuccess && n >= 4 && max_moves != 0) { // n < 4: nothing to scan, tours come back unchanged
-        const float m = p->dmax * kScreenMarginScale;
-        const float margin =
-            (p->fast_sqrt && std::isfinite(m) && p->dmax >= kScreenMinDmax && !getenv("TL_NO_SCREEN")) ? m : -1.0f;
+        const float margin = screen_margin(p);
         if (use_pop) {
             std::vector<int32_t> bf;
             int chunk = 0;
@@ -1179,11 +1175,11 @@ tl_status tl_two_opt_batch(tl_problem *p, int32_t algo, uint32_t *tours_inout, s
             }
             e = cudaMemcpyAsync(d_bands.p, bf.data(), bf.size() * 4, cudaMemcpyHostToDevice, st);
             if (e == cudaSuccess) e = cudaStreamSynchronize(st); // bf is a local
-            launch_pop_init(p->d_xy, d_t.p, n, npad, batch, cyclic, p->fast_sqrt, d_recs.p, d_ctl.p,
+            launch_pop_init(p->d_xy, d_t.p, n, npad, batch, cyclic, fast, d_recs.p, d_ctl.p,
                             reinterpret_cast<PopCounters *>(d_ctr.p), d_queue.p, qcap, c->sm_count, st);
             launch_two_opt_pop(d_recs.p, d_ctl.p, reinterpret_cast<PopCounters *>(d_ctr.p), n, npad, batch, cyclic,
                                max_moves, margin, chunk, (int)bf.size() - 1, nitems, d_bands.p, d_queue.p, qcap,
-                               p->fast_sqrt, c->sm_count, st);
+                               fast, c->sm_count, st);
             launch_pop_extract(d_recs.p, n, npad, batch, d_t.p, c->sm_count, st);
             c->launches += 3;
         } else {
@@ -1205,18 +1201,18 @@ tl_status tl_two_opt_batch(tl_problem *p, int32_t algo, uint32_t *tours_inout, s
                 // reported below
             } else if (cl > 1) { // fewer tours than CTA slots: a thread-block cluster per tour
                 e = launch_two_opt_batch_cluster(cfg, cl, p->d_xy, d_t.p, n, batch, cyclic, max_moves, margin, d_items.p,
-                                                 nitems, d_ctr.p, p->fast_sqrt, st);
+                                                 nitems, d_ctr.p, fast, st);
             } else {
-                const int grid = two_opt_batch_grid(cfg, n, batch, c->sm_count, p->fast_sqrt, margin >= 0.0f);
+                const int grid = two_opt_batch_grid(cfg, n, batch, c->sm_count, fast, margin >= 0.0f);
                 launch_two_opt_batch(cfg, p->d_xy, d_t.p, n, batch, cyclic, max_moves, margin, d_items.p, nitems, d_ctr.p,
-                                     grid, p->fast_sqrt, st);
+                                     grid, fast, st);
             }
             c->launches++;
         }
         if (e == cudaSuccess) e = cudaGetLastError();
     }
     if (e == cudaSuccess && lengths_out) {
-        launch_tour_lengths_f32(p->d_xy, nullptr, n, d_t.p, batch, p->fast_sqrt, false, d_len.p, c->sm_count, st);
+        launch_tour_lengths_f32(p->d_xy, nullptr, n, d_t.p, batch, fast, false, d_len.p, c->sm_count, st);
         c->launches++;
         e = cudaGetLastError();
     }
