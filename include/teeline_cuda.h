@@ -67,11 +67,17 @@ enum {
                                         re-evaluates the pairs the previous move changed (cached row minima):
                                         the fast way to the local optimum; stats.evals counts the pairs actually
                                         computed.  Not shardable, no tl_session_scan / time_scans. */
-    TL_ALGO_TWO_OPT_NEIGHBOR = 6     /* "Mode N": Mode B's move and delta over the pairs that create an edge to
+    TL_ALGO_TWO_OPT_NEIGHBOR = 6,    /* "Mode N": Mode B's move and delta over the pairs that create an edge to
                                         one of a city's k nearest neighbours (see tl_problem_set_candidates):
                                         a step costs O(n k) instead of O(n^2), for 10^5..10^6 cities.
                                         Coordinate problems (F32_EXACT, NINT_I32), TL_PATH_AUTO / RECOMPUTE;
                                         stats.evals counts the generated pairs.  Not shardable, not batched. */
+    TL_ALGO_OR_OPT_NEIGHBOR = 7      /* "Or-opt N": TL_ALGO_OR_OPT's move, delta, forbidden window and tie order
+                                        over the moves that create an edge between a segment endpoint and one
+                                        of its k nearest neighbours (see tl_problem_set_candidates): a step
+                                        costs O(n k) instead of O(n^2).  Same problems, paths and limits as
+                                        Mode N; n < 4 returns the identity order with no scan, as
+                                        TL_ALGO_OR_OPT does. */
 };
 
 /* where distances come from during the scan */
@@ -156,17 +162,34 @@ tl_status tl_dist_matrix_packed_i32(tl_problem *p, int32_t *out); /* NINT_I32 pr
  * ascending distance, ties by lower position, rows padded with UINT32_MAX. */
 tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
 
-/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR, built on the device by tl_knn's kernel and kept with
- * the problem (they depend on the instance only, like lin_kernighan::build_candidates,
- * lin_kernighan.rs:12-27).  K[c] = the first k entries of tl_knn(k) for city c; padded slots
- * (k > n-1) are skipped.  For every position i and slot s, with b = K[p_i][s], j = pos[b],
- * lo = min(i, j), hi = max(i, j), the search generates the pairs (lo, hi) (the candidate edge is the
- * move's first new edge) and (lo-1, hi-1) (its second new edge); a pair counts if it lies in Mode B's
- * neighbourhood 0 <= i, i+2 <= j <= n-2.  A step applies the argmin of (delta, i, j) over them with
- * strict '< 0', exactly as TL_ALGO_TWO_OPT_BEST; with k >= n-1 the moves are Mode B's.
+/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR and TL_ALGO_OR_OPT_NEIGHBOR, built on the device by
+ * tl_knn's kernel and kept with the problem (they depend on the instance only, like
+ * lin_kernighan::build_candidates, lin_kernighan.rs:12-27).  K[c] = the first k entries of tl_knn(k)
+ * for city c; padded slots (k > n-1) are skipped.
+ *
+ * Mode N: for every position i and slot s, with b = K[p_i][s], j = pos[b], lo = min(i, j),
+ * hi = max(i, j), the search generates the pairs (lo, hi) (the candidate edge is the move's first new
+ * edge) and (lo-1, hi-1) (its second new edge); a pair counts if it lies in Mode B's neighbourhood
+ * 0 <= i, i+2 <= j <= n-2.  A step applies the argmin of (delta, i, j) over them with strict '< 0',
+ * exactly as TL_ALGO_TWO_OPT_BEST; with k >= n-1 the moves are Mode B's.
+ *
+ * Or-opt N: with f = p_i, l = p_i+s-1, x = p_j, y = p_(j+1)%n, for every position q, c = p_q, slot t,
+ * b = K[c][t] and r = pos[b], the search generates the Or-opt moves (segment [i, i+s-1] inserted
+ * between x and y) whose new edge is (c, b):
+ *   (f, x) forward:  i = q,     j = r,           s = 1..3
+ *   (l, y) forward:  i = q-s+1, j = (r-1) mod n, s = 1..3
+ *   (l, x) reversed: i = q-s+1, j = r,           s = 2..3
+ *   (f, y) reversed: i = q,     j = (r-1) mod n, s = 2..3
+ * A move counts if it is legal for TL_ALGO_OR_OPT (n > s+1, 0 <= i, i+s <= n, j != prev(i), j outside
+ * [i, i+s-1]); its delta is TL_ALGO_OR_OPT's in the same rounding order, and a step applies the minimum
+ * of (delta, s, i, j, reversed) below Or-opt's threshold (-1e-3 in f32, 0 for NINT_I32), as
+ * TL_ALGO_OR_OPT's first-found scan does.  stats.evals counts the generated legal moves, forward and
+ * reversed separately, duplicates included.  With k >= n-1 every legal move is generated, so the moves
+ * are TL_ALGO_OR_OPT's.
+ *
  * 1 <= k <= 32 (TL_ERR_INVALID otherwise); EXPLICIT problems: TL_ERR_UNSUPPORTED.  A session copies
- * the lists when it is created, so later calls do not affect it.  Without a call, the first Mode N
- * session builds TL_CANDIDATES_DEFAULT lists.  Memory is O(n k): nothing n^2 is allocated. */
+ * the lists when it is created, so later calls do not affect it.  Without a call, the first session
+ * of either algorithm builds TL_CANDIDATES_DEFAULT lists.  Memory is O(n k): nothing n^2 is allocated. */
 #define TL_CANDIDATES_DEFAULT 8
 tl_status tl_problem_set_candidates(tl_problem *p, uint32_t k);
 

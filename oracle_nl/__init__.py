@@ -1,8 +1,8 @@
-"""ctypes loader for the CPU ORACLE of candidate-list 2-opt (oracle_nl/libteeline_oracle_nl.so).
+"""ctypes loader for the CPU ORACLES of candidate-list 2-opt and Or-opt (oracle_nl/libteeline_oracle_nl.so).
 
 TEST INFRASTRUCTURE ONLY, like `oracle`: tests and measurement scripts load it, the product package
-(teeline_b200/) never does.  Problems are `oracle.Problem` instances; the definition is in
-two_opt_nl.h and include/teeline_cuda.h (tl_problem_set_candidates).
+(teeline_b200/) never does.  Problems are `oracle.Problem` instances; the definitions are in
+two_opt_nl.h, or_opt_nl.h and include/teeline_cuda.h (tl_problem_set_candidates).
 """
 from __future__ import annotations
 
@@ -21,7 +21,7 @@ _ORACLE_DIR = os.path.dirname(os.path.abspath(O.__file__))
 
 def build(force: bool = False) -> str:
     """Compile with gcc (oracle_nl/Makefile)."""
-    srcs = [os.path.join(_DIR, f) for f in ("two_opt_nl.c", "two_opt_nl.h", "Makefile")] + \
+    srcs = [os.path.join(_DIR, f) for f in ("two_opt_nl.c", "two_opt_nl.h", "or_opt_nl.c", "or_opt_nl.h", "Makefile")] + \
         [os.path.join(_ORACLE_DIR, f) for f in ("teeline_oracle.c", "algos.inc", "teeline_oracle.h")]
     stale = not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in srcs)
     if force or stale:
@@ -71,4 +71,24 @@ def two_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 1,
     st, log = O.Stats(), (O.Move * max(log_cap, 1))()
     lib().tlo_two_opt_nl(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int64(max_moves), C.c_int(nthreads),
                          C.byref(st), log, C.c_int64(log_cap))
+    return t, st, [log[m].astuple() for m in range(min(st.moves, log_cap))]
+
+
+def or_opt_nl_scan(p: O.Problem, tour, cand, nthreads: int = 1):
+    """One Or-opt N scan.  Returns (move or None, evals); move = (delta, i, j, seg_len, reversed)."""
+    t = np.ascontiguousarray(tour, dtype=np.int32)
+    c = _cand(cand)
+    mv, ev = O.Move(), C.c_int64()
+    found = lib().tlo_or_opt_nl_scan(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int(nthreads), C.byref(mv),
+                                     C.byref(ev))
+    return (mv.astuple() if found else None), ev.value
+
+
+def or_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 1, log_cap: int = 0):
+    """Or-opt N to its local optimum (or max_moves).  Returns (tour, stats, moves) as O.or_opt."""
+    t = np.ascontiguousarray(tour, dtype=np.int32).copy()
+    c = _cand(cand)
+    st, log = O.Stats(), (O.Move * max(log_cap, 1))()
+    lib().tlo_or_opt_nl(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int64(max_moves), C.c_int(nthreads),
+                        C.byref(st), log, C.c_int64(log_cap))
     return t, st, [log[m].astuple() for m in range(min(st.moves, log_cap))]

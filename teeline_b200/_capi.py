@@ -21,6 +21,7 @@ DIST_F32_EXACT, DIST_NINT_I32 = 0, 1
 ALGO_TWO_OPT_REF, ALGO_TWO_OPT_BEST, ALGO_TWO_OPT_BEST_CYCLIC, ALGO_OR_OPT, ALGO_THREE_OPT = 0, 1, 2, 3, 4
 ALGO_TWO_OPT_BEST_CACHED = 5
 ALGO_TWO_OPT_NEIGHBOR = 6
+ALGO_OR_OPT_NEIGHBOR = 7
 CANDIDATES_DEFAULT = 8
 PATH_AUTO, PATH_MATRIX, PATH_RECOMPUTE = 0, 1, 2
 LEN_EXACT, LEN_FAST = 0, 1

@@ -29,27 +29,6 @@ namespace {
 constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
 
-// Pt records with distances recomputed from the coordinates in metric M (the nint metrics bit-equal to
-// K1's matrix entries, as in the persistent Mode R kernel); the entering-edge length is stored as the
-// bits of the metric's value type.
-template <Metric M>
-struct NlPol {
-    using V = MetricValue<M>;
-    using Rec = Pt;
-    Pt *pts;
-    __device__ __forceinline__ Rec load(uint32_t q) const { return pts[q]; }
-    static __device__ __forceinline__ V sp(const Rec &r) { return Val<V>::from_bits(__float_as_int(r.sp)); }
-    static __device__ __forceinline__ int32_t city(const Rec &r) { return r.city; }
-    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const { return tl::dist<M>(a.x, a.y, b.x, b.y); }
-    __device__ __forceinline__ void store_id(uint32_t q, const Rec &from) const
-    {
-        pts[q].x = from.x;
-        pts[q].y = from.y;
-        pts[q].city = from.city;
-    }
-    __device__ __forceinline__ void store_sp(uint32_t q, V v) const { pts[q].sp = __int_as_float(Val<V>::bits(v)); }
-};
-
 // Tail of a fused step, run by the last CTA: reduce the per-CTA records, count the step's evaluated
 // pairs, then either reverse a short segment here and finish the step, or leave a long one pending.
 template <class Pol>
@@ -171,26 +150,28 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     nl_tail(P, pos, blockbest, state, ticket, log, log_cap);
 }
 
-// tour-ordered records (entering-edge length in the policy's metric) and pos[city] = position
-template <class Pol>
+// tour-ordered records (entering-edge length in the policy's metric) and pos[city] = position.
+// CYCLIC (Or-opt N, which reads the closing edge): position 0 carries d(p_n-1, p_0) as its entering
+// edge and position n is a copy of position 0, as launch_build_pts(..., cyclic) lays them out for K3.
+template <bool CYCLIC, class Pol>
 __global__ void __launch_bounds__(256)
     nl_init_kernel(Pol P, const float2 *__restrict__ xy, const uint32_t *__restrict__ tour, uint32_t n, uint32_t npad,
                    uint32_t *__restrict__ pos)
 {
     using V = typename Pol::V;
     for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < npad; q += gridDim.x * blockDim.x) {
-        if (q < n) {
-            const uint32_t c = tour[q];
+        if (q < n || (CYCLIC && q == n)) {
+            const uint32_t c = tour[CYCLIC && q == n ? 0 : q];
             const float2 a = xy[c];
             const Pt r{a.x, a.y, (int32_t)c, 0.0f};
             P.store_id(q, r);
-            if (q == 0) {
+            if (q == 0 && !CYCLIC) {
                 P.store_sp(q, (V)0);
             } else {
-                const float2 b = xy[tour[q - 1]];
+                const float2 b = xy[tour[CYCLIC && q == 0 ? n - 1 : q - 1]];
                 P.store_sp(q, P.dist(Pt{b.x, b.y, 0, 0.0f}, r));
             }
-            pos[c] = q;
+            if (!CYCLIC || q < n) pos[c] = q;
         } else { // padding: never part of a pair
             P.store_id(q, Pt{0.0f, 0.0f, -1, 0.0f});
             P.store_sp(q, Val<V>::neg_inf());
@@ -200,11 +181,16 @@ __global__ void __launch_bounds__(256)
 
 } // namespace
 
-void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
-                    uint32_t *pos, cudaStream_t st)
+void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, bool cyclic,
+                    Pt *pts, uint32_t *pos, cudaStream_t st)
 {
     const int grid = (int)((npad + 255) / 256);
-    with_metric(metric, [&](auto M) { nl_init_kernel<<<grid, 256, 0, st>>>(NlPol<M>{pts}, xy, tour, n, npad, pos); });
+    with_metric(metric, [&](auto M) {
+        if (cyclic)
+            nl_init_kernel<true><<<grid, 256, 0, st>>>(NlPol<M>{pts}, xy, tour, n, npad, pos);
+        else
+            nl_init_kernel<false><<<grid, 256, 0, st>>>(NlPol<M>{pts}, xy, tour, n, npad, pos);
+    });
 }
 
 void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,

@@ -261,13 +261,24 @@ void launch_two_opt_cached_step(const Src &src, uint32_t n, int cyclic, unsigned
 constexpr int kNlThreads = 256;
 constexpr int kNlMinBlocks = 2;
 constexpr int kNlCtaSwaps = 2048; // segments of up to this many swapped pairs are reversed by the reducing CTA
-void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, Pt *pts,
-                    uint32_t *pos, cudaStream_t st);
+// cyclic: Or-opt N's records (position 0 carries the closing edge, position n is the wrap copy)
+void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, bool cyclic,
+                    Pt *pts, uint32_t *pos, cudaStream_t st);
 void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
                     DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
                     cudaStream_t st);
 void launch_nl_apply(Metric metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
                      tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
+
+// K3 candidate-list Or-opt, "Or-opt N" (k3_or_opt_neighbor.cu): Mode N's records (cyclic), pos[] and
+// lists.  blockbest holds grid + 1 records as in Mode N, blockcnt the grid per-CTA candidate counts;
+// tmp stages the relocated span (npad records).
+constexpr int kOrNlCtaSpan = 4096; // relocated spans of up to this many positions are moved by the reducing CTA
+void launch_or_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *tmp,
+                       void *blockbest, unsigned long long *blockcnt, DevState *state, unsigned int *ticket, tl_move *log,
+                       uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st);
+void launch_or_nl_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32_t n, const void *pending,
+                        DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
 
 // K2-batch: one CTA per tour, tour records in shared memory
 constexpr int kBatchR = 5;              // diagonals per thread group (odd => conflict-free LDS.128)

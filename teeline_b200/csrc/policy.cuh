@@ -4,7 +4,8 @@
 //   EucPol<FAST> : distances recomputed from tour-ordered coordinates (16-byte Pt records)
 //   MatPol<V>    : distances read from the slot-ordered n x ld matrix in HBM through the
 //                  tour-ordered Cs records (slot, entering-edge length, city), V = float | int32
-// Both are bit-identical for EUC_2D f32 problems (SURVEY.md section 0); MatPol also serves
+//   NlPol<M>     : the candidate-list searches' Pt records, distances recomputed in metric M
+// EucPol and MatPol are bit-identical for EUC_2D f32 problems (SURVEY.md section 0); MatPol also serves
 // EXPLICIT matrices and the TSPLIB nint metric.
 #pragma once
 
@@ -113,6 +114,28 @@ template <class Pol>
 struct L2Pol : Pol {
     __device__ __forceinline__ explicit L2Pol(const Pol &p) : Pol(p) {}
     __device__ __forceinline__ typename Pol::Rec load(uint32_t q) const { return Pol::load_l2(q); }
+};
+
+// NlPol<M> (candidate-list searches, k2_two_opt_neighbor.cu and k3_or_opt_neighbor.cu): Pt records with
+// distances recomputed from the coordinates in metric M (the nint metrics bit-equal to
+// K1's matrix entries, as in the persistent Mode R kernel); the entering-edge length is stored as the
+// bits of the metric's value type.
+template <Metric M>
+struct NlPol {
+    using V = MetricValue<M>;
+    using Rec = Pt;
+    Pt *pts;
+    __device__ __forceinline__ Rec load(uint32_t q) const { return pts[q]; }
+    static __device__ __forceinline__ V sp(const Rec &r) { return Val<V>::from_bits(__float_as_int(r.sp)); }
+    static __device__ __forceinline__ int32_t city(const Rec &r) { return r.city; }
+    __device__ __forceinline__ V dist(const Rec &a, const Rec &b) const { return tl::dist<M>(a.x, a.y, b.x, b.y); }
+    __device__ __forceinline__ void store_id(uint32_t q, const Rec &from) const
+    {
+        pts[q].x = from.x;
+        pts[q].y = from.y;
+        pts[q].city = from.city;
+    }
+    __device__ __forceinline__ void store_sp(uint32_t q, V v) const { pts[q].sp = __int_as_float(Val<V>::bits(v)); }
 };
 
 } // namespace tl

@@ -58,7 +58,7 @@ struct tl_session {
     uint64_t repermutes = 0;
     MatPin pin;                  // matrix path: L2 residency of part of a matrix larger than L2
 
-    DevBuf<unsigned char> tmp;     // Or-opt: relocated range staging (npad records of 16 B)
+    DevBuf<unsigned char> tmp;     // Or-opt, Or-opt N: relocated range staging (npad records of 16 B)
     DevBuf<unsigned char> rowinfo; // Or-opt: per-row removal gains (npad x 16 B)
     DevBuf<unsigned int> or_ticket; // Or-opt: work queue of the scan kernel
     int or_chunk = 0, or_items_per_cb = 0, or_item_begin = 0, or_item_end = 0;
@@ -78,12 +78,13 @@ struct tl_session {
     DevBuf<CachedDesc> cdesc;
     DevBuf<int> fullrows;
 
-    // candidate-list 2-opt (TL_ALGO_TWO_OPT_NEIGHBOR): Pt records plus pos[] and the session's own
-    // copy of the problem's candidate lists
+    // candidate-list searches (TL_ALGO_TWO_OPT_NEIGHBOR, TL_ALGO_OR_OPT_NEIGHBOR): Pt records plus pos[]
+    // and the session's own copy of the problem's candidate lists
     bool nl = false;
     DevBuf<uint32_t> pos;            // city -> position
     DevBuf<uint32_t> nl_cand;        // n x nl_k
     uint32_t nl_k = 0;
+    DevBuf<unsigned long long> nl_cnt; // Or-opt N: per-CTA counts of evaluated candidates
 
     DevBuf<BestF> cand; // shard_count * grid records (BestF and BestI have the same layout)
     DevBuf<DevState> state;
@@ -236,6 +237,7 @@ tl_status upload_geometry(tl_session *s)
         if (const char *cap = getenv("TL_MAX_GRID")) s->grid = std::max(1, std::min(s->grid, atoi(cap)));
         TL_CUDA_TRY(s->cand.alloc((size_t)s->grid + 1));
         TL_CUDA_TRY(cudaMemsetAsync(s->cand.p, 0xff, ((size_t)s->grid + 1) * sizeof(BestF), s->c->stream)); // no move pending
+        if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR) TL_CUDA_TRY(s->nl_cnt.alloc((size_t)s->grid));
         return TL_OK;
     }
     if (s->algo == TL_ALGO_OR_OPT) {
@@ -358,7 +360,11 @@ tl_status launch_scan(tl_session *s, bool fuse, bool exchange = true)
     const ShardComm *comm = (fused && s->shard_count > 1) ? &s->comm : nullptr;
     BestF *mine = s->cand.p + (size_t)s->shard_index * s->grid;
     cudaStream_t st = s->c->stream;
-    if (s->nl) {
+    if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR) {
+        launch_or_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->tmp.p, s->cand.p,
+                          s->nl_cnt.p, s->state.p, s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
+        s->c->launches++;
+    } else if (s->nl) {
         launch_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->cand.p, s->state.p,
                        s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
         s->c->launches++;
@@ -439,6 +445,12 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
         tl_status rc = launch_scan(s, true);
         if (rc != TL_OK) return rc;
         s->steps_since_permute++;
+        if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR) { // a long span left pending by the scan's last CTA
+            launch_or_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->tmp.p, s->n, s->cand.p + s->grid, s->state.p,
+                               s->ticket.p + 1, s->log.p, s->log_cap, apply_grid, st);
+            s->c->launches += 2;
+            continue;
+        }
         if (s->nl) { // a long segment left pending by the scan's last CTA (none: the grid leaves at once)
             launch_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->cand.p + s->grid, s->state.p, s->ticket.p + 1,
                             s->log.p, s->log_cap, apply_grid, st);
@@ -535,7 +547,8 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     const bool cached = algo == TL_ALGO_TWO_OPT_BEST_CACHED; // Mode B with cached row minima: runs as Mode B
     if (cached) algo = TL_ALGO_TWO_OPT_BEST;
     if (algo != TL_ALGO_TWO_OPT_BEST && algo != TL_ALGO_TWO_OPT_BEST_CYCLIC && algo != TL_ALGO_TWO_OPT_REF &&
-        algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT && algo != TL_ALGO_TWO_OPT_NEIGHBOR) {
+        algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT && algo != TL_ALGO_TWO_OPT_NEIGHBOR &&
+        algo != TL_ALGO_OR_OPT_NEIGHBOR) {
         set_error("tl_session_create: unknown algo %d", algo);
         return TL_ERR_INVALID;
     }
@@ -543,11 +556,11 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         set_error("tl_session_create: unknown path %d", path);
         return TL_ERR_INVALID;
     }
-    const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR;
+    const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR || algo == TL_ALGO_OR_OPT_NEIGHBOR;
     if (nl && (path == TL_PATH_MATRIX || p->kind == PK_EXPLICIT)) {
-        // candidate 2-opt is for instances whose n^2 matrix is the problem; both metrics are recomputed
-        set_error(p->kind == PK_EXPLICIT ? "candidate 2-opt needs coordinates (EXPLICIT problem)"
-                                         : "candidate 2-opt recomputes distances: TL_PATH_MATRIX is not supported");
+        // candidate-list searches are for instances whose n^2 matrix is the problem; both metrics are recomputed
+        set_error(p->kind == PK_EXPLICIT ? "candidate-list search needs coordinates (EXPLICIT problem)"
+                                         : "candidate-list search recomputes distances: TL_PATH_MATRIX is not supported");
         return TL_ERR_UNSUPPORTED;
     }
     // AUTO: recompute for f32 coordinate problems (bit-identical to the matrix and no n^2 memory),
@@ -656,6 +669,10 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         set_error("tl_session_create: device allocation failed");
         return fail(TL_ERR_NOMEM);
     }
+    if (algo == TL_ALGO_OR_OPT_NEIGHBOR && s->tmp.alloc((size_t)s->npad * 16) != cudaSuccess) {
+        set_error("tl_session_create: device allocation failed");
+        return fail(TL_ERR_NOMEM);
+    }
     if (cached && !s->trivial) {
         if (s->rowkey.alloc(p->n) != cudaSuccess || s->cdesc.alloc(1) != cudaSuccess || s->fullrows.alloc(p->n) != cudaSuccess) {
             set_error("tl_session_create: device allocation failed");
@@ -669,9 +686,10 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         if (ce != cudaSuccess) { set_error("tl_session_create: %s", cudaGetErrorString(ce)); return fail(TL_ERR_CUDA); }
     }
     // or_opt::solve and three_opt::solve ignore the seed and return identity order when n < 4
-    // (or_opt.rs:31-34, three_opt.rs:25-28)
+    // (or_opt.rs:31-34, three_opt.rs:25-28); so does Or-opt N
+    const bool or_like = algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT || algo == TL_ALGO_OR_OPT_NEIGHBOR;
     std::vector<uint32_t> ident;
-    if ((algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT) && s->trivial) {
+    if (or_like && s->trivial) {
         ident.resize(p->n);
         for (uint32_t k = 0; k < p->n; ++k) ident[k] = k;
         tour = ident.data();
@@ -718,7 +736,8 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         }
         s->src.kind = SRC_EUC_SAFE; // tl_session_tour reads the city fields only
         s->src.pts = s->pts.p;
-        launch_nl_init(p->metric, p->d_xy, d_tour.p, p->n, s->npad, s->pts.p, s->pos.p, c->stream);
+        launch_nl_init(p->metric, p->d_xy, d_tour.p, p->n, s->npad, algo == TL_ALGO_OR_OPT_NEIGHBOR, s->pts.p, s->pos.p,
+                       c->stream);
         c->launches++;
     } else {
         if (s->pts.alloc(s->npad) != cudaSuccess) { set_error("tl_session_create: device allocation failed"); return fail(TL_ERR_NOMEM); }
@@ -739,7 +758,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         // loop runs one empty pass for n == 3 and is skipped for n < 3 (two_opt.rs:17,29 underflow)
         s->h.done = 1;
         s->h.converged = 1;
-        s->h.scans = (algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT) ? 0 : 1;
+        s->h.scans = or_like ? 0 : 1;
         s->h.passes = (p->n == 3) ? 1 : 0;
     }
     tl_status rc = push_state(s); // also waits for d_tour's consumers
@@ -798,7 +817,7 @@ tl_status tl_session_set_shard(tl_session *s, int32_t index, int32_t count)
         return TL_OK;
     }
     if (s->nl) {
-        if (count > 1) { set_error("candidate 2-opt does not shard"); return TL_ERR_UNSUPPORTED; }
+        if (count > 1) { set_error("candidate-list searches do not shard"); return TL_ERR_UNSUPPORTED; }
         return TL_OK;
     }
     DeviceGuard g(s->c);
@@ -857,12 +876,13 @@ tl_status tl_session_scan(tl_session *s, tl_move *best, int32_t *found)
     if (was_done) { s->h.done = was_done; rc = push_state(s); if (rc != TL_OK) return rc; }
     bool any;
     const bool three = s->algo == TL_ALGO_THREE_OPT;
+    const bool or_opt = s->algo == TL_ALGO_OR_OPT || s->algo == TL_ALGO_OR_OPT_NEIGHBOR;
     if (s->int_values()) {
         std::vector<BestI> hi(hc.size());
         memcpy(hi.data(), hc.data(), hc.size() * sizeof(BestF));
-        any = three ? reduce_host_three(hi, best) : reduce_host(hi, s->algo == TL_ALGO_OR_OPT, best);
+        any = three ? reduce_host_three(hi, best) : reduce_host(hi, or_opt, best);
     } else {
-        any = three ? reduce_host_three(hc, best) : reduce_host(hc, s->algo == TL_ALGO_OR_OPT, best);
+        any = three ? reduce_host_three(hc, best) : reduce_host(hc, or_opt, best);
     }
     *found = any ? 1 : 0;
     return TL_OK;
