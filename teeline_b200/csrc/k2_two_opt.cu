@@ -22,7 +22,7 @@
 // work 15 flop/move, ~0 bytes/move (DESIGN.md section 4).
 #include "kernels.cuh"
 #include "policy.cuh"
-#include "two_opt_apply.cuh"
+#include "apply.cuh"
 
 #include <math_constants.h>
 
@@ -344,15 +344,7 @@ void launch_scan_recompute(Pt *pts, const ScanGeom &g, const int32_t *band_first
     sc.world = 1;
     if (shard) sc = *shard;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(WARPS * 32);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
+    const cudaLaunchConfig_t cfg = pdl_config(grid, WARPS * 32, smem, attr, st);
     const int fuse = fuse_apply ? 1 : 0;
     auto kern = (fast && g.screen_margin >= 0.0f) ? two_opt_scan_recompute_kernel<true, true>
                 : fast                           ? two_opt_scan_recompute_kernel<true, false>

@@ -22,7 +22,7 @@
 // screened delta is re-evaluated exactly is shared by all threads working on the tour.
 // Argmin: (delta, i, j) lexicographic as ONE 64-bit key, two REDUX and one shared-memory atomicMin per
 // warp -- independent of which thread saw a candidate first.  Apply: the in-place reversal of
-// two_opt_apply.cuh on the shared-memory records.
+// apply.cuh on the shared-memory records.
 //
 // CLUSTER PER TOUR (two_opt_batch_cluster_kernel): when the batch has fewer tours than the GPU has
 // CTA slots -- BASELINE config 5 sharded over 8 GPUs leaves 128 tours for 148 SMs -- a tour is a
@@ -39,7 +39,7 @@
 // tour).  Algorithmic work 15 flop/move as for the single-tour recompute kernel.
 #include "kernels.cuh"
 #include "policy.cuh"
-#include "two_opt_apply.cuh"
+#include "apply.cuh"
 
 #include <cooperative_groups.h>
 #include <math_constants.h>

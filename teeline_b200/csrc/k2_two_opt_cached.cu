@@ -29,7 +29,7 @@
 // place and writes the next description.
 #include "kernels.cuh"
 #include "policy.cuh"
-#include "two_opt_apply.cuh"
+#include "apply.cuh"
 
 #include <cstdlib>
 
@@ -344,14 +344,8 @@ void launch_two_opt_cached_step(const Src &src, uint32_t n, int cyclic, unsigned
                                 int grid, cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = getenv("TL_CACHED_NO_PDL") ? 0 : 1; // experiment: plain stream order between steps
+    cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
+    if (getenv("TL_CACHED_NO_PDL")) cfg.numAttrs = 0; // experiment: plain stream order between steps
     TL_DISPATCH_POL(src, (cudaLaunchKernelEx(&cfg, two_opt_cached_step_kernel<decltype(P)>, P, (int)n, cyclic, rowkey, desc,
                                              fullrows, state, ticket, log, (uint64_t)log_cap)));
 }

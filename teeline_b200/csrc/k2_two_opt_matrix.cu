@@ -18,7 +18,7 @@
 // Roofline: HBM bandwidth, 4 B per move (DESIGN.md section 4).
 #include "kernels.cuh"
 #include "policy.cuh"
-#include "two_opt_apply.cuh"
+#include "apply.cuh"
 
 #include <type_traits>
 
@@ -535,9 +535,7 @@ void launch_scan_matrix(const Src &src, const ScanGeom &g, const int32_t *band_f
     sc.world = 1;
     if (shard) sc = *shard;
     cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    int nattr = 1;
+    cudaLaunchConfig_t cfg = pdl_config(grid, WARPS * 32, smem, attr, st);
     if (pin.window_bytes > 0) { // driver-managed residency: persisting window over the first matrix rows
         attr[1].id = cudaLaunchAttributeAccessPolicyWindow;
         attr[1].val.accessPolicyWindow.base_ptr = const_cast<void *>(src.M);
@@ -545,15 +543,8 @@ void launch_scan_matrix(const Src &src, const ScanGeom &g, const int32_t *band_f
         attr[1].val.accessPolicyWindow.hitRatio = pin.window_hit_ratio;
         attr[1].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
         attr[1].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        nattr = 2;
+        cfg.numAttrs = 2;
     }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(WARPS * 32);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = nattr;
     const int fuse = fuse_apply ? 1 : 0;
     const int pin_rows = pin.hint_rows;
     static const int pf_default = [] {

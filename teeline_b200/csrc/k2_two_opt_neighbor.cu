@@ -17,8 +17,8 @@
 // there is none.  The grid size cannot depend on the move: the host queues steps without reading back.
 // The records, pos[] and the candidate lists (16 + 4 + 4k bytes per city) fit L2 up to about 10^6
 // cities, so the scan is a chain of dependent L2 gathers.
+#include "apply.cuh"
 #include "kernels.cuh"
-#include "two_opt_apply.cuh"
 
 #include <math_constants.h>
 
@@ -48,24 +48,15 @@ __device__ __noinline__ void nl_tail(const Pol &P, uint32_t *pos, Best<typename 
         const int4 raw = __ldcg(reinterpret_cast<const int4 *>(blockbest) + c);
         const Best<V> o{Val<V>::from_bits(raw.x), (uint32_t)raw.y, (uint32_t)raw.z, (uint32_t)raw.w};
         cnt += o.aux;
-        if (better_2opt(o.delta, o.i, o.j, v.delta, v.i, v.j)) v = o;
+        if (TwoOptOrder::better(o, v)) v = o;
     }
-    warp_argmin_2opt(v.delta, v.i, v.j);
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
-    if (lane == 0) {
-        red[warp] = v;
-        red_cnt[warp] = cnt;
-    }
-    __syncthreads();
-    v = red[0];
-    cnt = red_cnt[0];
+    if (lane == 0) red_cnt[warp] = cnt;
+    v = block_argmin<WARPS, TwoOptOrder>(v, red); // its barrier publishes red_cnt too
+    cnt = 0;
 #pragma unroll
-    for (int w = 1; w < WARPS; ++w) {
-        const Best<V> o = red[w];
-        cnt += red_cnt[w];
-        if (better_2opt(o.delta, o.i, o.j, v.delta, v.i, v.j)) v = o;
-    }
+    for (int w = 0; w < WARPS; ++w) cnt += red_cnt[w];
     const bool found = v.i != 0xffffffffu;
     const bool long_seg = found && (v.j - v.i) / 2 > (uint32_t)kNlCtaSwaps;
     if (threadIdx.x == 0) {
@@ -198,14 +189,7 @@ void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand,
                     cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(THREADS);
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
+    const cudaLaunchConfig_t cfg = pdl_config(grid, THREADS, 0, attr, st);
     const int fuse = fuse_apply ? 1 : 0;
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
@@ -219,14 +203,7 @@ void launch_nl_apply(Metric metric, Pt *pts, uint32_t *pos, const void *pending,
                      tl_move *log, uint64_t log_cap, int grid, cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
+    const cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
         cudaLaunchKernelEx(&cfg, apply_two_opt_kernel<Pol>, Pol{pts}, reinterpret_cast<const Best<typename Pol::V> *>(pending),

@@ -23,7 +23,7 @@
 //                 move, screened like K2-B) -> publish the warp's best candidate with ONE 64-bit
 //                 atomicMin on (order-preserving delta bits << 32 | i*n + j) -> count the item done.
 //   the worker that completes the LAST item of a scan applies the move: reverses the segment in
-//   the tour's global records (two_opt_apply.cuh), bumps the move count and pushes the tour back
+//   the tour's global records (apply.cuh), bumps the move count and pushes the tour back
 //   into the FIFO (or retires it when nothing improves / the move budget is spent).
 //   (First version: per-tour tickets that idle workers polled, 32 tours per round -- the polling
 //   storm of ~3500 warps on a few KB of L2 made a step take 340 us; profiles/r02d.)
@@ -37,7 +37,7 @@
 // Roofline: FP32 issue, ~0.5 B/move of L2 traffic for staging; 15 flop/move as for K2-B.
 #include "host.hpp"
 #include "policy.cuh"
-#include "two_opt_apply.cuh"
+#include "apply.cuh"
 
 #include <math_constants.h>
 

@@ -31,7 +31,7 @@
 // kernel's, which changes what is evaluated speculatively, never which move comes next.
 #include "kernels.cuh"
 #include "policy.cuh"
-#include "two_opt_apply.cuh"
+#include "apply.cuh"
 
 #include <cooperative_groups.h>
 #include <type_traits>
@@ -463,14 +463,7 @@ void launch_ref_step(const Src &src, uint32_t n, DevState *state, unsigned int *
                      uint64_t log_cap, int grid, cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
+    const cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
     TL_DISPATCH_POL(src, (cudaLaunchKernelEx(&cfg, ref_step_kernel<decltype(P)>, P, n, state, ticket, log,
                                              (uint64_t)log_cap)));
 }

@@ -21,6 +21,7 @@
 // diagonal, so warps take a masked copy of the step there and the mask-free copy elsewhere.
 //
 // Roofline: FP32 issue; ~6.5 issued instructions per candidate.
+#include "apply.cuh"
 #include "kernels.cuh"
 #include "or_opt_rank.cuh"
 #include "policy.cuh"
@@ -264,104 +265,6 @@ __global__ void __launch_bounds__(WARPS * 32, kOrMinBlocks)
     }
 }
 
-// ---- relocation (apply_relocation, or_opt.rs:172-184) --------------------------------------------
-
-template <typename V>
-__device__ __forceinline__ OrMove reduce_or_candidates(const Best<V> *__restrict__ cand, int ncand, Best<V> *sred)
-{
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    Best<V> v{(V)0, kNone, kNone, 0u};
-    for (int c = threadIdx.x; c < ncand; c += blockDim.x) {
-        const Best<V> o = cand[c];
-        if (better_or(o, v)) v = o;
-    }
-    warp_argmin_or(v);
-    if (lane == 0) sred[warp] = v;
-    __syncthreads();
-    v = sred[0];
-    for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
-        if (better_or(sred[w], v)) v = sred[w];
-    return or_move_of(v);
-}
-
-template <class Pol>
-__global__ void __launch_bounds__(256)
-    or_apply_gather_kernel(Pol P, typename Pol::Rec *__restrict__ tmp,
-                           const Best<typename Pol::V> *__restrict__ cand, int ncand,
-                           const DevState *__restrict__ state)
-{
-    if (state->done) return;
-    __shared__ Best<typename Pol::V> sred[8];
-    const OrMove m = reduce_or_candidates(cand, ncand, sred);
-    if (!m.found) return;
-    for (uint32_t q = m.lo + blockIdx.x * blockDim.x + threadIdx.x; q <= m.hi; q += gridDim.x * blockDim.x)
-        tmp[q - m.lo] = P.load(or_source(m, q));
-}
-
-template <class Pol>
-__global__ void __launch_bounds__(256)
-    or_apply_scatter_kernel(Pol P, const typename Pol::Rec *__restrict__ tmp, uint32_t n,
-                            const Best<typename Pol::V> *__restrict__ cand, int ncand, DevState *state,
-                            unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap)
-{
-    using Rec = typename Pol::Rec;
-    if (state->done) return;
-    __shared__ Best<typename Pol::V> sred[8];
-    const OrMove m = reduce_or_candidates(cand, ncand, sred);
-    if (m.found) {
-        // record now at position q (q in 0..n): relocated range from tmp, everything else unchanged
-        auto newpt = [&](uint32_t q) -> Rec {
-            const uint32_t qq = q == n ? 0u : q;
-            return (qq >= m.lo && qq <= m.hi) ? tmp[qq - m.lo] : P.load(qq);
-        };
-        // positions lo .. hi+1 get a new record and/or a new entering edge; every read of a
-        // relocated position goes to tmp, so the in-place writes below cannot race with them
-        for (uint32_t q = m.lo + blockIdx.x * blockDim.x + threadIdx.x; q <= m.hi + 1; q += gridDim.x * blockDim.x) {
-            if (q < 1 || q > n) continue;
-            Rec p = newpt(q);
-            const Rec b = newpt(q - 1);
-            const typename Pol::V e = P.dist(b, p);
-            if (q <= m.hi) {
-                Pol::set_sp(p, e);
-                P.store(q, p);
-            } else {
-                P.store_sp(q, e); // hi+1: same city (or the wrap copy), new entering edge
-            }
-        }
-        // closing edge and the wrap copy at position n
-        if (blockIdx.x == 0 && threadIdx.x == 0 && (m.lo == 0 || m.hi >= n - 1)) {
-            Rec p0 = newpt(0);
-            const Rec last = newpt(n - 1);
-            Pol::set_sp(p0, P.dist(last, p0));
-            P.store(n, p0);
-            if (m.lo == 0) {
-                P.store(0, p0);
-            } else {
-                P.store_sp(0, Pol::sp(p0));
-            }
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const unsigned int tk = atomicAdd(ticket, 1u);
-        if (tk == gridDim.x - 1) {
-            *ticket = 0u;
-            state->scans += 1;
-            if (m.found) {
-                const unsigned long long mv = state->moves;
-                if (log && mv < log_cap) log[mv] = tl_move{m.delta, m.i, m.j, (uint8_t)m.s, (uint8_t)m.rev, 0};
-                state->moves = mv + 1;
-                if (state->max_moves >= 0 && (long long)(mv + 1) >= state->max_moves) state->done = 1;
-            } else {
-                state->done = 1;
-                state->converged = 1;
-            }
-            __threadfence();
-        }
-    }
-}
-
 } // namespace
 
 size_t or_scan_smem_bytes()
@@ -404,8 +307,9 @@ void launch_or_apply(const Src &src, void *tmp, uint32_t n, const void *cand, in
         using PolT = decltype(P);
         auto *t = reinterpret_cast<typename PolT::Rec *>(tmp);
         auto *c = reinterpret_cast<const Best<typename PolT::V> *>(cand);
-        or_apply_gather_kernel<<<grid, 256, 0, st>>>(P, t, c, ncand, state);
-        or_apply_scatter_kernel<<<grid, 256, 0, st>>>(P, t, n, c, ncand, state, ticket, log, log_cap);
+        relocate_gather_kernel<PolT, OrMove><<<grid, 256, 0, st>>>(P, t, c, ncand, state);
+        relocate_scatter_kernel<PolT, OrMove><<<grid, 256, 0, st>>>(P, t, n, c, ncand, state, ticket, log, log_cap,
+                                                                    nullptr, 0);
     });
 }
 

@@ -34,9 +34,9 @@
 // barrier, scatter); a longer one is left pending for the gather and scatter grids that every step
 // launches, which leave at once when nothing is pending.  The grid size cannot depend on the move: the
 // host queues steps without reading back.
+#include "apply.cuh"
 #include "kernels.cuh"
 #include "or_opt_rank.cuh"
-#include "two_opt_apply.cuh"
 
 namespace tl {
 
@@ -45,67 +45,6 @@ namespace {
 constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
 constexpr uint32_t kNone = 0xffffffffu;
-
-// loop state and log after an Or-opt N step (one thread)
-__device__ __forceinline__ void finish_or_step(DevState *state, const StateHeader &h, const OrMove &m,
-                                               tl_move *__restrict__ log, uint64_t log_cap)
-{
-    const unsigned long long mv = h.h0.x;
-    const long long max_moves = h.h1.x;
-    state->scans = h.h0.y + 1;
-    if (m.found) {
-        if (log && mv < log_cap) log[mv] = tl_move{m.delta, m.i, m.j, (uint8_t)m.s, (uint8_t)m.rev, 0};
-        state->moves = mv + 1;
-        if (max_moves >= 0 && (long long)(mv + 1) >= max_moves) state->done = 1;
-    } else {
-        state->done = 1;
-        state->converged = 1;
-    }
-}
-
-// apply_relocation in two phases with a barrier between them (block or grid): first copy the new
-// occupants of [lo, hi] to tmp ...
-template <class Pol>
-__device__ __forceinline__ void or_gather(const Pol &P, Pt *__restrict__ tmp, const OrMove &m, uint32_t tid,
-                                          uint32_t nthreads)
-{
-    for (uint32_t q = m.lo + tid; q <= m.hi; q += nthreads) tmp[q - m.lo] = P.load(or_source(m, q));
-}
-
-// ... then write them back with the entering edges of lo .. hi+1 and their pos[] entries; thread 0 of
-// the group rewrites the closing edge and the wrap copy at position n.  Every read of a relocated
-// position goes to tmp, so the in-place writes cannot race with them.
-template <class Pol>
-__device__ __forceinline__ void or_scatter(const Pol &P, const Pt *__restrict__ tmp, uint32_t n, const OrMove &m,
-                                           uint32_t *__restrict__ pos, uint32_t tid, uint32_t nthreads)
-{
-    using V = typename Pol::V;
-    auto newpt = [&](uint32_t q) -> Pt {
-        const uint32_t qq = q == n ? 0u : q;
-        return (qq >= m.lo && qq <= m.hi) ? tmp[qq - m.lo] : P.load(qq);
-    };
-    for (uint32_t q = m.lo + tid; q <= m.hi + 1; q += nthreads) {
-        if (q < 1 || q > n) continue;
-        const Pt p = newpt(q), b = newpt(q - 1);
-        const V e = P.dist(b, p);
-        if (q <= m.hi) {
-            P.store_id(q, p);
-            pos[p.city] = q;
-        }
-        P.store_sp(q, e); // hi+1: same city (or the wrap copy), new entering edge
-    }
-    if (tid == 0 && (m.lo == 0 || m.hi >= n - 1)) {
-        const Pt p0 = newpt(0), last = newpt(n - 1);
-        const V e = P.dist(last, p0);
-        if (m.lo == 0) {
-            P.store_id(0, p0);
-            pos[p0.city] = 0;
-        }
-        P.store_sp(0, e);
-        P.store_id(n, p0);
-        P.store_sp(n, e);
-    }
-}
 
 // Tail of a fused step, run by the last CTA: reduce the per-CTA records, count the step's evaluated
 // candidates, then either relocate a short span here and finish the step, or leave a long one pending.
@@ -129,22 +68,14 @@ __device__ __noinline__ void or_nl_tail(const Pol &P, uint32_t n, uint32_t *pos,
         cnt += __ldcg(blockcnt + c);
         if (better_or(o, v)) v = o;
     }
-    warp_argmin_or(v);
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
-    if (lane == 0) {
-        red[warp] = v;
-        red_cnt[warp] = cnt;
-    }
-    __syncthreads();
-    v = red[0];
-    cnt = red_cnt[0];
+    if (lane == 0) red_cnt[warp] = cnt;
+    v = block_argmin<WARPS, OrMove>(v, red); // its barrier publishes red_cnt too
+    cnt = 0;
 #pragma unroll
-    for (int w = 1; w < WARPS; ++w) {
-        cnt += red_cnt[w];
-        if (better_or(red[w], v)) v = red[w];
-    }
-    const OrMove m = or_move_of(v);
+    for (int w = 0; w < WARPS; ++w) cnt += red_cnt[w];
+    const OrMove m = OrMove::of(v);
     const bool long_span = m.found && m.hi - m.lo + 1 > (uint32_t)kOrNlCtaSpan;
     if (threadIdx.x == 0) {
         state->computed += cnt;
@@ -154,11 +85,11 @@ __device__ __noinline__ void or_nl_tail(const Pol &P, uint32_t n, uint32_t *pos,
     }
     if (long_span) return;
     if (m.found) {
-        or_gather(P, tmp, m, threadIdx.x, blockDim.x);
+        relocate_gather(P, tmp, m, threadIdx.x, blockDim.x);
         __syncthreads();
-        or_scatter(P, tmp, n, m, pos, threadIdx.x, blockDim.x);
+        relocate_scatter(P, tmp, n, m, pos, threadIdx.x, blockDim.x);
     }
-    if (threadIdx.x == 0) finish_or_step(state, hdr, m, log, log_cap);
+    if (threadIdx.x == 0) finish_step(state, hdr, m.found, m.entry(), log, log_cap);
 }
 
 template <class Pol>
@@ -267,55 +198,6 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     or_nl_tail(P, n, pos, tmp, blockbest, blockcnt, state, ticket, log, log_cap);
 }
 
-// the apply grids of a step whose span the scan left pending: gather, then scatter and finish the step
-template <class Pol>
-__global__ void __launch_bounds__(256)
-    or_nl_gather_kernel(Pol P, Pt *__restrict__ tmp, const Best<typename Pol::V> *__restrict__ pending,
-                        const DevState *__restrict__ state)
-{
-    griddep_wait(); // the step's scan has finished and its writes are visible
-    if (state->done) return;
-    const OrMove m = or_move_of(*pending);
-    if (!m.found) return; // the scan's last CTA finished the step
-    or_gather(P, tmp, m, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
-}
-
-template <class Pol>
-__global__ void __launch_bounds__(256)
-    or_nl_scatter_kernel(Pol P, const Pt *__restrict__ tmp, uint32_t n, const Best<typename Pol::V> *__restrict__ pending,
-                         uint32_t *__restrict__ pos, DevState *state, unsigned int *ticket, tl_move *__restrict__ log,
-                         uint64_t log_cap)
-{
-    griddep_wait(); // the gather grid has finished
-    if (state->done) return;
-    const OrMove m = or_move_of(*pending);
-    if (!m.found) return; // uniform over the grid
-    or_scatter(P, tmp, n, m, pos, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const unsigned int tk = atomicAdd(ticket, 1u);
-        if (tk == gridDim.x - 1) { // last block: everyone has read `state` by now
-            *ticket = 0u;
-            finish_or_step(state, load_state_header(state), m, log, log_cap);
-            __threadfence();
-        }
-    }
-}
-
-cudaLaunchConfig_t pdl_config(int grid, int threads, cudaLaunchAttribute *attr, cudaStream_t st)
-{
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3((unsigned)threads);
-    cfg.stream = st;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cfg;
-}
-
 } // namespace
 
 void launch_or_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *tmp,
@@ -323,7 +205,7 @@ void launch_or_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *ca
                        uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t cfg = pdl_config(grid, THREADS, attr, st);
+    const cudaLaunchConfig_t cfg = pdl_config(grid, THREADS, 0, attr, st);
     const int fuse = fuse_apply ? 1 : 0;
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
@@ -337,14 +219,14 @@ void launch_or_nl_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32
                         DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid, cudaStream_t st)
 {
     cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t cfg = pdl_config(grid, 256, attr, st);
+    const cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
         const auto *pend = reinterpret_cast<const Best<typename Pol::V> *>(pending);
-        cudaLaunchKernelEx(&cfg, or_nl_gather_kernel<Pol>, Pol{pts}, reinterpret_cast<Pt *>(tmp), pend,
+        cudaLaunchKernelEx(&cfg, relocate_gather_kernel<Pol, OrMove>, Pol{pts}, reinterpret_cast<Pt *>(tmp), pend, 1,
                            (const DevState *)state);
-        cudaLaunchKernelEx(&cfg, or_nl_scatter_kernel<Pol>, Pol{pts}, (const Pt *)tmp, n, pend, pos, state, ticket, log,
-                           (uint64_t)log_cap);
+        cudaLaunchKernelEx(&cfg, relocate_scatter_kernel<Pol, OrMove>, Pol{pts}, (const Pt *)tmp, n, pend, 1, state,
+                           ticket, log, (uint64_t)log_cap, pos, 1);
     });
 }
 

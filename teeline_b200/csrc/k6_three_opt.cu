@@ -23,6 +23,7 @@
 // Work items are pulled from a global ticket (row i of the triangle has ~(n-i)^2/2 triples).
 //
 // Roofline: FP32 issue (2 exact distances + 14 adds + min tree per triple, ~50 instructions).
+#include "apply.cuh"
 #include "kernels.cuh"
 #include "policy.cuh"
 
@@ -45,6 +46,14 @@ __device__ __forceinline__ bool better_three(V s1, uint32_t i1, uint32_t j1, uin
     if (i1 != i2) return i1 < i2;
     if (j1 != j2) return j1 < j2;
     return (a1 >> 3) < (a2 >> 3);
+}
+// record form; a record with i == kNone is "no candidate" and only loses
+template <typename V>
+__device__ __forceinline__ bool better_three(const Best<V> &a, const Best<V> &b)
+{
+    if (a.i == kNone) return false;
+    if (b.i == kNone) return true;
+    return better_three(a.delta, a.i, a.j, a.aux, b.delta, b.i, b.j, b.aux);
 }
 
 // staged per-k entry: the record of F = p[k+1], d_EF, and the two j-independent distances
@@ -178,46 +187,32 @@ __global__ void __launch_bounds__(WARPS * 32, kThreeMinBlocks)
 
 // ---- apply_3opt (three_opt.rs:182-218) -------------------------------------------------------------
 
+// the move of a record, with the span [lo, hi] = [i+1, k] it rebuilds (lo >= 1, hi <= n-1): the Move of
+// the relocation apply step (apply.cuh)
 struct ThreeMove {
     bool found;
     float savings;
-    uint32_t i, j, k, kase;
-};
+    uint32_t i, j, k, kase, lo, hi;
 
-template <typename V>
-__device__ __forceinline__ ThreeMove reduce_three_candidates(const Best<V> *__restrict__ cand, int ncand, Best<V> *sred)
-{
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    Best<V> v{(V)0, kNone, kNone, 0u};
-    for (int c = threadIdx.x; c < ncand; c += blockDim.x) {
-        const Best<V> o = cand[c];
-        if (o.i != kNone && (v.i == kNone || better_three(o.delta, o.i, o.j, o.aux, v.delta, v.i, v.j, v.aux))) v = o;
+    template <typename V>
+    static __device__ __forceinline__ ThreeMove of(const Best<V> &v)
+    {
+        ThreeMove m;
+        m.found = v.i != kNone;
+        m.savings = (float)v.delta;
+        m.i = v.i;
+        m.j = v.j;
+        m.k = v.aux >> 3;
+        m.kase = v.aux & 7u;
+        m.lo = m.i + 1;
+        m.hi = m.k;
+        return m;
     }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        Best<V> o;
-        o.delta = __shfl_xor_sync(0xffffffffu, v.delta, off);
-        o.i = __shfl_xor_sync(0xffffffffu, v.i, off);
-        o.j = __shfl_xor_sync(0xffffffffu, v.j, off);
-        o.aux = __shfl_xor_sync(0xffffffffu, v.aux, off);
-        if (o.i != kNone && (v.i == kNone || better_three(o.delta, o.i, o.j, o.aux, v.delta, v.i, v.j, v.aux))) v = o;
-    }
-    if (lane == 0) sred[warp] = v;
-    __syncthreads();
-    v = sred[0];
-    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) {
-        const Best<V> o = sred[w];
-        if (o.i != kNone && (v.i == kNone || better_three(o.delta, o.i, o.j, o.aux, v.delta, v.i, v.j, v.aux))) v = o;
-    }
-    ThreeMove m;
-    m.found = v.i != kNone;
-    m.savings = (float)v.delta;
-    m.i = v.i;
-    m.j = v.j;
-    m.k = v.aux >> 3;
-    m.kase = v.aux & 7u;
-    return m;
-}
+    template <typename V>
+    static __device__ __forceinline__ bool better(const Best<V> &a, const Best<V> &b) { return better_three(a, b); }
+    __device__ __forceinline__ uint32_t source(uint32_t q) const;
+    __device__ __forceinline__ tl_move entry() const { return tl_move{-savings, i, j, (uint8_t)kase, 0, 0, k}; }
+};
 
 // new occupant of position q in [i+1, k], as an old position: the middle is rebuilt from
 // seg1 = p[i+1..=j] and seg2 = p[j+1..=k] (cases 4-7 put seg2 first; odd cases reverse seg1,
@@ -235,69 +230,7 @@ __device__ __forceinline__ uint32_t three_source(const ThreeMove &m, uint32_t q)
     return m.i + 1 + (rev1 ? l1 - 1 - u : u);
 }
 
-template <class Pol>
-__global__ void __launch_bounds__(256)
-    three_apply_gather_kernel(Pol P, typename Pol::Rec *__restrict__ tmp, const Best<typename Pol::V> *__restrict__ cand,
-                              int ncand, const DevState *__restrict__ state)
-{
-    if (state->done) return;
-    __shared__ Best<typename Pol::V> sred[8];
-    const ThreeMove m = reduce_three_candidates(cand, ncand, sred);
-    if (!m.found) return;
-    for (uint32_t q = m.i + 1 + blockIdx.x * blockDim.x + threadIdx.x; q <= m.k; q += gridDim.x * blockDim.x)
-        tmp[q - (m.i + 1)] = P.load(three_source(m, q));
-}
-
-template <class Pol>
-__global__ void __launch_bounds__(256)
-    three_apply_scatter_kernel(Pol P, const typename Pol::Rec *__restrict__ tmp, uint32_t n,
-                               const Best<typename Pol::V> *__restrict__ cand, int ncand, DevState *state,
-                               unsigned int *ticket, unsigned int *work_ticket, tl_move *__restrict__ log,
-                               uint64_t log_cap)
-{
-    using Rec = typename Pol::Rec;
-    if (state->done) return;
-    __shared__ Best<typename Pol::V> sred[8];
-    const ThreeMove m = reduce_three_candidates(cand, ncand, sred);
-    if (m.found) {
-        const uint32_t lo = m.i + 1, hi = m.k; // positions that get a new occupant; lo >= 1, hi <= n-1
-        auto newpt = [&](uint32_t q) -> Rec { return (q >= lo && q <= hi) ? tmp[q - lo] : P.load(q); };
-        // positions lo .. hi+1 get a new record and/or a new entering edge; reads of relocated
-        // positions go to tmp, so the in-place writes cannot race with them
-        for (uint32_t q = lo + blockIdx.x * blockDim.x + threadIdx.x; q <= hi + 1; q += gridDim.x * blockDim.x) {
-            Rec p = (q == n) ? P.load(0) : newpt(q); // hi+1 == n: the wrap copy of position 0
-            const Rec b = newpt(q - 1);
-            const typename Pol::V e = P.dist(b, p);
-            if (q <= hi) {
-                Pol::set_sp(p, e);
-                P.store(q, p);
-            } else {
-                P.store_sp(q, e);              // same city (or the wrap copy), new entering edge
-                if (q == n) P.store_sp(0, e);  // position 0 carries the closing edge too
-            }
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const unsigned int tk = atomicAdd(ticket, 1u);
-        if (tk == gridDim.x - 1) {
-            *ticket = 0u;
-            *work_ticket = 0u; // re-arm the scan's work queue
-            state->scans += 1;
-            if (m.found) {
-                const unsigned long long mv = state->moves;
-                if (log && mv < log_cap) log[mv] = tl_move{-m.savings, m.i, m.j, (uint8_t)m.kase, 0, 0, m.k};
-                state->moves = mv + 1;
-                if (state->max_moves >= 0 && (long long)(mv + 1) >= state->max_moves) state->done = 1;
-            } else {
-                state->done = 1;
-                state->converged = 1;
-            }
-            __threadfence();
-        }
-    }
-}
+__device__ __forceinline__ uint32_t ThreeMove::source(uint32_t q) const { return three_source(*this, q); }
 
 } // namespace
 
@@ -310,15 +243,15 @@ void launch_three_scan(const Src &src, uint32_t n, const int32_t *row_first, int
 }
 
 void launch_three_apply(const Src &src, void *tmp, uint32_t n, const void *cand, int ncand, DevState *state,
-                        unsigned int *ticket, unsigned int *work_ticket, tl_move *log, uint64_t log_cap, int grid,
-                        cudaStream_t st)
+                        unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid, cudaStream_t st)
 {
     TL_DISPATCH_POL(src, {
         using PolT = decltype(P);
         auto *t = reinterpret_cast<typename PolT::Rec *>(tmp);
         auto *c = reinterpret_cast<const Best<typename PolT::V> *>(cand);
-        three_apply_gather_kernel<<<grid, 256, 0, st>>>(P, t, c, ncand, state);
-        three_apply_scatter_kernel<<<grid, 256, 0, st>>>(P, t, n, c, ncand, state, ticket, work_ticket, log, log_cap);
+        relocate_gather_kernel<PolT, ThreeMove><<<grid, 256, 0, st>>>(P, t, c, ncand, state);
+        relocate_scatter_kernel<PolT, ThreeMove><<<grid, 256, 0, st>>>(P, t, n, c, ncand, state, ticket, log, log_cap,
+                                                                       nullptr, 0);
     });
 }
 

@@ -86,6 +86,22 @@ struct Src {
 // ---------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------
+// Launch configuration with programmatic dependent launch (common.cuh: griddep_wait) in attr[0].  A
+// caller that needs more attributes sets attr[1..] and raises numAttrs.
+inline cudaLaunchConfig_t pdl_config(int grid, int threads, size_t smem, cudaLaunchAttribute *attr, cudaStream_t st)
+{
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)grid);
+    cfg.blockDim = dim3((unsigned)threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cfg;
+}
+
 void launch_k1_packed(const float2 *xy, uint32_t n, Metric metric, void *out, int sm_count, cudaStream_t st);
 void launch_k1_square(const float2 *sxy, uint32_t n, uint32_t ld, Metric metric, void *out, cudaStream_t st);
 void launch_k1_square_from_packed(const uint32_t *tri, const int32_t *slot_city, uint32_t n,
@@ -198,8 +214,7 @@ constexpr int kThreeMinBlocks = 4;
 void launch_three_scan(const Src &src, uint32_t n, const int32_t *row_first, int item_begin, int item_end,
                        void *blockbest, const DevState *state, unsigned int *work_ticket, int grid, cudaStream_t st);
 void launch_three_apply(const Src &src, void *tmp, uint32_t n, const void *cand, int ncand, DevState *state,
-                        unsigned int *ticket, unsigned int *work_ticket, tl_move *log, uint64_t log_cap, int grid,
-                        cudaStream_t st);
+                        unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
 
 // K5 / N1
 // tri non-null (EXPLICIT problems): distances from the packed triangle, else recomputed in `metric`

@@ -3,6 +3,7 @@
 #pragma once
 
 #include "common.cuh"
+#include "../../include/teeline_cuda.h"
 
 namespace tl {
 
@@ -43,25 +44,30 @@ __device__ __forceinline__ void warp_argmin_or(Best<V> &v)
 // ---- relocation (apply_relocation, or_opt.rs:172-184) --------------------------------------------
 
 // the move with its relocated span [lo, hi]: every position outside it keeps its record
+// (the Move of the relocation apply step, apply.cuh)
 struct OrMove {
     bool found;
     float delta;
     uint32_t i, j, s, rev, lo, hi;
-};
 
-template <typename V>
-__device__ __forceinline__ OrMove or_move_of(const Best<V> &v)
-{
-    OrMove m;
-    m.found = v.i != 0xffffffffu;
-    m.delta = (float)v.delta;
-    m.i = v.i;
-    m.j = v.j;
-    m.s = (v.aux >> 1) + 1;
-    m.rev = v.aux & 1u;
-    if (m.j >= m.i + m.s) { m.lo = m.i; m.hi = m.j; } else { m.lo = m.j + 1; m.hi = m.i + m.s - 1; }
-    return m;
-}
+    template <typename V>
+    static __device__ __forceinline__ OrMove of(const Best<V> &v)
+    {
+        OrMove m;
+        m.found = v.i != 0xffffffffu;
+        m.delta = (float)v.delta;
+        m.i = v.i;
+        m.j = v.j;
+        m.s = (v.aux >> 1) + 1;
+        m.rev = v.aux & 1u;
+        if (m.j >= m.i + m.s) { m.lo = m.i; m.hi = m.j; } else { m.lo = m.j + 1; m.hi = m.i + m.s - 1; }
+        return m;
+    }
+    template <typename V>
+    static __device__ __forceinline__ bool better(const Best<V> &a, const Best<V> &b) { return better_or(a, b); }
+    __device__ __forceinline__ uint32_t source(uint32_t q) const;
+    __device__ __forceinline__ tl_move entry() const { return tl_move{delta, i, j, (uint8_t)s, (uint8_t)rev, 0}; }
+};
 
 // new occupant of position q in [lo, hi] after the relocation, as an old position
 __device__ __forceinline__ uint32_t or_source(const OrMove &m, uint32_t q)
@@ -78,5 +84,7 @@ __device__ __forceinline__ uint32_t or_source(const OrMove &m, uint32_t q)
     }
     return q - m.s;
 }
+
+__device__ __forceinline__ uint32_t OrMove::source(uint32_t q) const { return or_source(*this, q); }
 
 } // namespace tl

@@ -136,6 +136,8 @@ struct NlPol {
         pts[q].city = from.city;
     }
     __device__ __forceinline__ void store_sp(uint32_t q, V v) const { pts[q].sp = __int_as_float(Val<V>::bits(v)); }
+    static __device__ __forceinline__ void set_sp(Rec &r, V v) { r.sp = __int_as_float(Val<V>::bits(v)); }
+    __device__ __forceinline__ void store(uint32_t q, const Rec &r) const { pts[q] = r; }
 };
 
 } // namespace tl

@@ -465,7 +465,7 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
         }
         if (s->algo == TL_ALGO_THREE_OPT) {
             launch_three_apply(s->src, s->tmp.p, s->n, s->cand.p, s->grid * s->shard_count, s->state.p, s->ticket.p,
-                               s->or_ticket.p, s->log.p, s->log_cap, apply_grid, st);
+                               s->log.p, s->log_cap, apply_grid, st);
             s->c->launches += 2;
             continue;
         }

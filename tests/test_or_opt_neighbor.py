@@ -273,9 +273,10 @@ def test_gpu_both_relocation_routes(ctx):
     prob.set_candidates(8)
     opt, st, _ = prob.local_search(T.ALGO_OR_OPT_NEIGHBOR, prob.nn_tour(3))
     assert st.converged == 1
-    # carry single cities far from their place: Or-opt N brings them back over long spans
+    # carry single cities far from their place: Or-opt N brings them back over long spans; the last two
+    # spans start at position 0 and end at n-1, so the apply grids rewrite the closing edge and the wrap copy
     tour = opt.astype(np.int64).tolist()
-    for src, dst in ((1000, 9000), (2000, 2300), (7000, 100), (5000, 5050), (3000, 8800)):
+    for src, dst in ((1000, 9000), (2000, 2300), (7000, 100), (5000, 5050), (3000, 8800), (6000, 0), (4000, 9999)):
         c = tour.pop(src)
         tour.insert(dst, c)
     got_t, got_m = gpu_vs_oracle(ctx, x, y, "f32", 8, np.array(tour, dtype=np.uint32), prob=prob)
