@@ -72,12 +72,18 @@ enum {
                                         a step costs O(n k) instead of O(n^2), for 10^5..10^6 cities.
                                         Coordinate problems (F32_EXACT, NINT_I32), TL_PATH_AUTO / RECOMPUTE;
                                         stats.evals counts the generated pairs.  Not shardable, not batched. */
-    TL_ALGO_OR_OPT_NEIGHBOR = 7      /* "Or-opt N": TL_ALGO_OR_OPT's move, delta, forbidden window and tie order
+    TL_ALGO_OR_OPT_NEIGHBOR = 7,     /* "Or-opt N": TL_ALGO_OR_OPT's move, delta, forbidden window and tie order
                                         over the moves that create an edge between a segment endpoint and one
                                         of its k nearest neighbours (see tl_problem_set_candidates): a step
                                         costs O(n k) instead of O(n^2).  Same problems, paths and limits as
                                         Mode N; n < 4 returns the identity order with no scan, as
                                         TL_ALGO_OR_OPT does. */
+    TL_ALGO_THREE_OPT_NEIGHBOR = 8   /* "3-opt N": TL_ALGO_THREE_OPT's triples, costs, case choice and tie order
+                                        over the triples that the first two candidate edges of a sequential
+                                        3-exchange generate (see tl_problem_set_candidates): a step costs
+                                        O(n k^2) instead of O(n^3).  Same problems, paths and limits as Or-opt N;
+                                        n < 4 returns the identity order with no scan, as TL_ALGO_THREE_OPT
+                                        does. */
 };
 
 /* where distances come from during the scan */
@@ -162,7 +168,8 @@ tl_status tl_dist_matrix_packed_i32(tl_problem *p, int32_t *out); /* NINT_I32 pr
  * ascending distance, ties by lower position, rows padded with UINT32_MAX. */
 tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
 
-/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR and TL_ALGO_OR_OPT_NEIGHBOR, built on the device by
+/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR, TL_ALGO_OR_OPT_NEIGHBOR and TL_ALGO_THREE_OPT_NEIGHBOR, built
+ * on the device by
  * tl_knn's kernel and kept with the problem (they depend on the instance only, like
  * lin_kernighan::build_candidates, lin_kernighan.rs:12-27).  K[c] = the first k entries of tl_knn(k)
  * for city c; padded slots (k > n-1) are skipped.
@@ -187,9 +194,25 @@ tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
  * reversed separately, duplicates included.  With k >= n-1 every legal move is generated, so the moves
  * are TL_ALGO_OR_OPT's.
  *
+ * 3-opt N: cut edge e (0 <= e <= n-1) joins p_e and p_(e+1)%n; TL_ALGO_THREE_OPT's triple (i, j, k) with
+ * i < j < k removes edges i, j and k.  Following the first two candidate edges of a sequential
+ * 3-exchange, for every position q, c = p_q:
+ *   1. every slot s1 with b = K[c][s1] not padding, r = pos[b];
+ *   2. each e2 in {(r-1) mod n, r}; t = the other endpoint of edge e2: p_(r+1)%n when e2 = r, p_(r-1)%n
+ *      otherwise;
+ *   3. every slot s2 with b' = K[t][s2] not padding, r' = pos[b'];
+ *   4. each e1 in {(q-1) mod n, q} and e3 in {(r'-1) mod n, r'}: if e1, e2 and e3 are distinct, sorted
+ *      into i < j < k, the triple counts unless i = 0 and k = n-1 (TL_ALGO_THREE_OPT's skip).
+ * At most 8 triples per (q, s1, s2), 8 n k^2 per step.  Evaluation is TL_ALGO_THREE_OPT's: orig and
+ * cost1..cost7 are its left-to-right sums in the metric's value type, the triple's case is the first
+ * minimal cost among those below orig, and savings = orig - cost.  A step applies the counted triple with
+ * the largest savings > 0, ties to the lowest (i, j, k); duplicates carry the same key.  stats.evals
+ * counts every counted triple, duplicates included.  With k >= n-1 every triple is generated (q = i+1,
+ * b = p_j, e2 = j, t = p_j+1, b' = p_k, e1 = i, e3 = k), so the moves are TL_ALGO_THREE_OPT's.
+ *
  * 1 <= k <= 32 (TL_ERR_INVALID otherwise); EXPLICIT problems: TL_ERR_UNSUPPORTED.  A session copies
  * the lists when it is created, so later calls do not affect it.  Without a call, the first session
- * of either algorithm builds TL_CANDIDATES_DEFAULT lists.  Memory is O(n k): nothing n^2 is allocated. */
+ * of any of these algorithms builds TL_CANDIDATES_DEFAULT lists.  Memory is O(n k): nothing n^2 is allocated. */
 #define TL_CANDIDATES_DEFAULT 8
 tl_status tl_problem_set_candidates(tl_problem *p, uint32_t k);
 

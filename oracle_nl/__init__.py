@@ -1,8 +1,8 @@
-"""ctypes loader for the CPU ORACLES of candidate-list 2-opt and Or-opt (oracle_nl/libteeline_oracle_nl.so).
+"""ctypes loader for the CPU ORACLES of candidate-list 2-opt, Or-opt and 3-opt (oracle_nl/libteeline_oracle_nl.so).
 
 TEST INFRASTRUCTURE ONLY, like `oracle`: tests and measurement scripts load it, the product package
 (teeline_b200/) never does.  Problems are `oracle.Problem` instances; the definitions are in
-two_opt_nl.h, or_opt_nl.h and include/teeline_cuda.h (tl_problem_set_candidates).
+two_opt_nl.h, or_opt_nl.h, three_opt_nl.h and include/teeline_cuda.h (tl_problem_set_candidates).
 """
 from __future__ import annotations
 
@@ -21,7 +21,8 @@ _ORACLE_DIR = os.path.dirname(os.path.abspath(O.__file__))
 
 def build(force: bool = False) -> str:
     """Compile with gcc (oracle_nl/Makefile)."""
-    srcs = [os.path.join(_DIR, f) for f in ("two_opt_nl.c", "two_opt_nl.h", "or_opt_nl.c", "or_opt_nl.h", "Makefile")] + \
+    srcs = [os.path.join(_DIR, f) for f in ("two_opt_nl.c", "two_opt_nl.h", "or_opt_nl.c", "or_opt_nl.h", "three_opt_nl.c",
+                                         "three_opt_nl.h", "Makefile")] + \
         [os.path.join(_ORACLE_DIR, f) for f in ("teeline_oracle.c", "algos.inc", "teeline_oracle.h")]
     stale = not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in srcs)
     if force or stale:
@@ -92,3 +93,36 @@ def or_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 1, 
     lib().tlo_or_opt_nl(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int64(max_moves), C.c_int(nthreads),
                         C.byref(st), log, C.c_int64(log_cap))
     return t, st, [log[m].astuple() for m in range(min(st.moves, log_cap))]
+
+
+def three_opt_nl_eval(p: O.Problem, tour, i: int, j: int, k: int):
+    """The evaluation of the triple i < j < k on tour: (delta = -savings, case), or None when no case improves."""
+    t = np.ascontiguousarray(tour, dtype=np.int32)
+    s, kase = C.c_double(), C.c_int32()
+    ok = lib().tlo_three_opt_nl_eval(p.ref, _p(t), C.c_int32(i), C.c_int32(j), C.c_int32(k), C.byref(s),
+                                     C.byref(kase))
+    return (-s.value, kase.value) if ok else None
+
+
+def three_opt_nl_scan(p: O.Problem, tour, cand, nthreads: int = 1):
+    """One 3-opt N scan.  Returns (move or None, evals); move = (delta = -savings, i, j, k, case) as
+    O.three_opt_find_best."""
+    t = np.ascontiguousarray(tour, dtype=np.int32)
+    c = _cand(cand)
+    mv, k, ev = O.Move(), C.c_int32(), C.c_int64()
+    found = lib().tlo_three_opt_nl_scan(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int(nthreads), C.byref(mv),
+                                        C.byref(k), C.byref(ev))
+    return ((mv.delta, mv.i, mv.j, k.value, mv.seg_len) if found else None), ev.value
+
+
+def three_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 1, log_cap: int = 0):
+    """3-opt N to its local optimum (or max_moves).  Returns (tour, stats, moves) as O.three_opt, with
+    moves = (delta, i, j, k, case)."""
+    t = np.ascontiguousarray(tour, dtype=np.int32).copy()
+    c = _cand(cand)
+    st, log = O.Stats(), (O.Move * max(log_cap, 1))()
+    ks = np.zeros(max(log_cap, 1), dtype=np.int32)
+    lib().tlo_three_opt_nl(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int64(max_moves), C.c_int(nthreads),
+                           C.byref(st), log, _p(ks), C.c_int64(log_cap))
+    mv = [(log[m].delta, log[m].i, log[m].j, int(ks[m]), log[m].seg_len) for m in range(min(st.moves, log_cap))]
+    return t, st, mv

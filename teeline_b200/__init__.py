@@ -15,7 +15,7 @@ import numpy as np
 
 from . import _capi as capi
 from ._capi import (ALGO_OR_OPT, ALGO_OR_OPT_NEIGHBOR, ALGO_THREE_OPT, ALGO_TWO_OPT_BEST, ALGO_TWO_OPT_BEST_CACHED, ALGO_TWO_OPT_BEST_CYCLIC,
-                    ALGO_TWO_OPT_NEIGHBOR, ALGO_TWO_OPT_REF, CANDIDATES_DEFAULT,
+                    ALGO_THREE_OPT_NEIGHBOR, ALGO_TWO_OPT_NEIGHBOR, ALGO_TWO_OPT_REF, CANDIDATES_DEFAULT,
                     DIST_F32_EXACT, DIST_NINT_I32, LEN_EXACT, LEN_FAST, PATH_AUTO, PATH_MATRIX,
                     PATH_RECOMPUTE, Move, Stats, TeelineError)
 
@@ -128,8 +128,8 @@ class Problem:
         return out
 
     def set_candidates(self, k: int = CANDIDATES_DEFAULT):
-        """tl_problem_set_candidates: the k-nearest candidate lists that later ALGO_TWO_OPT_NEIGHBOR and
-        ALGO_OR_OPT_NEIGHBOR sessions of this problem search (1 <= k <= 32)."""
+        """tl_problem_set_candidates: the k-nearest candidate lists that later ALGO_TWO_OPT_NEIGHBOR,
+        ALGO_OR_OPT_NEIGHBOR and ALGO_THREE_OPT_NEIGHBOR sessions of this problem search (1 <= k <= 32)."""
         capi.check(self._lib.tl_problem_set_candidates(self.h, k))
 
     def nn_tour(self, k: int = 3) -> np.ndarray:
@@ -161,7 +161,7 @@ class Problem:
         log = (Move * max(log_cap, 1))()
         capi.check(self._lib.tl_local_search(self.h, algo, path, capi.ptr(t), max_moves, C.byref(st),
                                              log if log_cap else None, log_cap))
-        three = algo == ALGO_THREE_OPT
+        three = algo in (ALGO_THREE_OPT, ALGO_THREE_OPT_NEIGHBOR)
         moves = [log[k].astuple3() if three else log[k].astuple() for k in range(min(int(st.moves), log_cap))]
         return t, st, moves
 
@@ -234,7 +234,7 @@ class Session:
         capi.check(self._lib.tl_session_scan(self.h, C.byref(mv), C.byref(found)))
         if not found.value:
             return None
-        return mv.astuple3() if self.algo == ALGO_THREE_OPT else mv.astuple()
+        return mv.astuple3() if self.algo in (ALGO_THREE_OPT, ALGO_THREE_OPT_NEIGHBOR) else mv.astuple()
 
     def time_scans(self, reps: int) -> float:
         """Average scan-kernel launch duration in ms (CUDA events on the context's stream)."""
@@ -262,7 +262,7 @@ class Session:
         log = (Move * max(cap, 1))()
         got = C.c_size_t()
         capi.check(self._lib.tl_session_log(self.h, log, cap, C.byref(got)))
-        three = self.algo == ALGO_THREE_OPT
+        three = self.algo in (ALGO_THREE_OPT, ALGO_THREE_OPT_NEIGHBOR)
         return [log[k].astuple3() if three else log[k].astuple() for k in range(got.value)]
 
     def close(self):

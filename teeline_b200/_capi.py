@@ -22,6 +22,7 @@ ALGO_TWO_OPT_REF, ALGO_TWO_OPT_BEST, ALGO_TWO_OPT_BEST_CYCLIC, ALGO_OR_OPT, ALGO
 ALGO_TWO_OPT_BEST_CACHED = 5
 ALGO_TWO_OPT_NEIGHBOR = 6
 ALGO_OR_OPT_NEIGHBOR = 7
+ALGO_THREE_OPT_NEIGHBOR = 8
 CANDIDATES_DEFAULT = 8
 PATH_AUTO, PATH_MATRIX, PATH_RECOMPUTE = 0, 1, 2
 LEN_EXACT, LEN_FAST = 0, 1

@@ -292,6 +292,56 @@ __device__ __forceinline__ void relocate_scatter(const Pol &P, const typename Po
     }
 }
 
+// Tail of a fused candidate-list relocation step (Or-opt N, 3-opt N), run by the scan's last CTA of
+// WARPS warps: reduce the per-CTA records blockbest[0 .. grid) in Move's order, add the per-CTA counts of
+// evaluated candidates to state->computed, then either relocate a span of at most kOrNlCtaSpan positions
+// here through tmp and finish the step, or leave a longer one pending in blockbest[grid] for the apply
+// grids (relocate_gather_kernel / relocate_scatter_kernel with pending_only).
+template <int WARPS, class Move, class Pol>
+__device__ __noinline__ void relocate_step_tail(const Pol &P, uint32_t n, uint32_t *pos, typename Pol::Rec *tmp,
+                                                Best<typename Pol::V> *blockbest, const unsigned long long *blockcnt,
+                                                DevState *state, unsigned int *ticket, tl_move *__restrict__ log,
+                                                uint64_t log_cap)
+{
+    using V = typename Pol::V;
+    __shared__ Best<V> red[WARPS];
+    __shared__ unsigned long long red_cnt[WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    StateHeader hdr{};
+    if (threadIdx.x == 0) hdr = load_state_header(state);
+    Best<V> v{(V)0, 0xffffffffu, 0xffffffffu, 0u};
+    unsigned long long cnt = 0;
+    for (int c = threadIdx.x; c < (int)gridDim.x; c += blockDim.x) {
+        // L2 reads: the records were written by other CTAs of this launch
+        const int4 raw = __ldcg(reinterpret_cast<const int4 *>(blockbest) + c);
+        const Best<V> o{Val<V>::from_bits(raw.x), (uint32_t)raw.y, (uint32_t)raw.z, (uint32_t)raw.w};
+        cnt += __ldcg(blockcnt + c);
+        if (Move::better(o, v)) v = o;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
+    if (lane == 0) red_cnt[warp] = cnt;
+    v = block_argmin<WARPS, Move>(v, red); // its barrier publishes red_cnt too
+    cnt = 0;
+#pragma unroll
+    for (int w = 0; w < WARPS; ++w) cnt += red_cnt[w];
+    const Move m = Move::of(v);
+    const bool long_span = m.found && m.hi - m.lo + 1 > (uint32_t)kOrNlCtaSpan;
+    if (threadIdx.x == 0) {
+        state->computed += cnt;
+        // the pending move for this step's apply grids (none: the step is finished here)
+        blockbest[gridDim.x] = long_span ? v : Best<V>{(V)0, 0xffffffffu, 0xffffffffu, 0u};
+        *ticket = 0u;
+    }
+    if (long_span) return;
+    if (m.found) {
+        relocate_gather(P, tmp, m, threadIdx.x, blockDim.x);
+        __syncthreads();
+        relocate_scatter(P, tmp, n, m, pos, threadIdx.x, blockDim.x);
+    }
+    if (threadIdx.x == 0) finish_step(state, hdr, m.found, m.entry(), log, log_cap);
+}
+
 // The two apply grids of a relocating search, with the contract of apply_two_opt_kernel: every block
 // reduces cand[0 .. ncand); with pending_only (Or-opt N's one pending record) no move means the scan
 // already finished the step.  The gather grid writes nothing else, so it needs no pending_only.

@@ -46,52 +46,6 @@ constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
 constexpr uint32_t kNone = 0xffffffffu;
 
-// Tail of a fused step, run by the last CTA: reduce the per-CTA records, count the step's evaluated
-// candidates, then either relocate a short span here and finish the step, or leave a long one pending.
-template <class Pol>
-__device__ __noinline__ void or_nl_tail(const Pol &P, uint32_t n, uint32_t *pos, Pt *tmp, Best<typename Pol::V> *blockbest,
-                                        const unsigned long long *blockcnt, DevState *state, unsigned int *ticket,
-                                        tl_move *__restrict__ log, uint64_t log_cap)
-{
-    using V = typename Pol::V;
-    __shared__ Best<V> red[WARPS];
-    __shared__ unsigned long long red_cnt[WARPS];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    StateHeader hdr{};
-    if (threadIdx.x == 0) hdr = load_state_header(state);
-    Best<V> v{(V)0, kNone, kNone, 0u};
-    unsigned long long cnt = 0;
-    for (int c = threadIdx.x; c < (int)gridDim.x; c += blockDim.x) {
-        // L2 reads: the records were written by other CTAs of this launch
-        const int4 raw = __ldcg(reinterpret_cast<const int4 *>(blockbest) + c);
-        const Best<V> o{Val<V>::from_bits(raw.x), (uint32_t)raw.y, (uint32_t)raw.z, (uint32_t)raw.w};
-        cnt += __ldcg(blockcnt + c);
-        if (better_or(o, v)) v = o;
-    }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
-    if (lane == 0) red_cnt[warp] = cnt;
-    v = block_argmin<WARPS, OrMove>(v, red); // its barrier publishes red_cnt too
-    cnt = 0;
-#pragma unroll
-    for (int w = 0; w < WARPS; ++w) cnt += red_cnt[w];
-    const OrMove m = OrMove::of(v);
-    const bool long_span = m.found && m.hi - m.lo + 1 > (uint32_t)kOrNlCtaSpan;
-    if (threadIdx.x == 0) {
-        state->computed += cnt;
-        // the pending move for this step's apply grids (none: the step is finished here)
-        blockbest[gridDim.x] = long_span ? v : Best<V>{(V)0, kNone, kNone, 0u};
-        *ticket = 0u;
-    }
-    if (long_span) return;
-    if (m.found) {
-        relocate_gather(P, tmp, m, threadIdx.x, blockDim.x);
-        __syncthreads();
-        relocate_scatter(P, tmp, n, m, pos, threadIdx.x, blockDim.x);
-    }
-    if (threadIdx.x == 0) finish_step(state, hdr, m.found, m.entry(), log, log_cap);
-}
-
 template <class Pol>
 __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     or_nl_scan_kernel(Pol P, uint32_t *__restrict__ pos, const uint32_t *__restrict__ cand, uint32_t k, uint32_t n,
@@ -195,7 +149,7 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     if (threadIdx.x == 0) s_last = (ticket_take_acq_rel(ticket) == gridDim.x - 1) ? 1u : 0u; // thread 0 wrote blockbest
     __syncthreads();
     if (!s_last) return;
-    or_nl_tail(P, n, pos, tmp, blockbest, blockcnt, state, ticket, log, log_cap);
+    relocate_step_tail<WARPS, OrMove>(P, n, pos, tmp, blockbest, blockcnt, state, ticket, log, log_cap);
 }
 
 } // namespace

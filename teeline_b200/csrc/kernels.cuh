@@ -295,6 +295,15 @@ void launch_or_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *ca
 void launch_or_nl_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32_t n, const void *pending,
                         DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
 
+// K6 candidate-list 3-opt, "3-opt N" (k6_three_opt_neighbor.cu): Or-opt N's records, pos[], lists,
+// buffers and relocation routes; its records carry the savings, as K6's do.
+void launch_three_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *tmp,
+                          void *blockbest, unsigned long long *blockcnt, DevState *state, unsigned int *ticket,
+                          tl_move *log, uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st);
+void launch_three_nl_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32_t n, const void *pending,
+                           DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid,
+                           cudaStream_t st);
+
 // K2-batch: one CTA per tour, tour records in shared memory
 constexpr int kBatchR = 5;              // diagonals per thread group (odd => conflict-free LDS.128)
 constexpr int kBatchMaxSmem = 200 * 1024;

@@ -58,7 +58,7 @@ struct tl_session {
     uint64_t repermutes = 0;
     MatPin pin;                  // matrix path: L2 residency of part of a matrix larger than L2
 
-    DevBuf<unsigned char> tmp;     // Or-opt, Or-opt N: relocated range staging (npad records of 16 B)
+    DevBuf<unsigned char> tmp;     // Or-opt, Or-opt N, 3-opt N: relocated range staging (npad records of 16 B)
     DevBuf<unsigned char> rowinfo; // Or-opt: per-row removal gains (npad x 16 B)
     DevBuf<unsigned int> or_ticket; // Or-opt: work queue of the scan kernel
     int or_chunk = 0, or_items_per_cb = 0, or_item_begin = 0, or_item_end = 0;
@@ -78,13 +78,13 @@ struct tl_session {
     DevBuf<CachedDesc> cdesc;
     DevBuf<int> fullrows;
 
-    // candidate-list searches (TL_ALGO_TWO_OPT_NEIGHBOR, TL_ALGO_OR_OPT_NEIGHBOR): Pt records plus pos[]
-    // and the session's own copy of the problem's candidate lists
+    // candidate-list searches (TL_ALGO_TWO_OPT_NEIGHBOR, TL_ALGO_OR_OPT_NEIGHBOR, TL_ALGO_THREE_OPT_NEIGHBOR):
+    // Pt records plus pos[] and the session's own copy of the problem's candidate lists
     bool nl = false;
     DevBuf<uint32_t> pos;            // city -> position
     DevBuf<uint32_t> nl_cand;        // n x nl_k
     uint32_t nl_k = 0;
-    DevBuf<unsigned long long> nl_cnt; // Or-opt N: per-CTA counts of evaluated candidates
+    DevBuf<unsigned long long> nl_cnt; // Or-opt N, 3-opt N: per-CTA counts of evaluated candidates
 
     DevBuf<BestF> cand; // shard_count * grid records (BestF and BestI have the same layout)
     DevBuf<DevState> state;
@@ -104,6 +104,8 @@ struct tl_session {
     double device_ms = 0.0;
 
     bool matrix() const { return path_used == TL_PATH_MATRIX; }
+    // the candidate-list searches that relocate a span of positions (cyclic records, staging buffer, counts)
+    bool nl_relocating() const { return algo == TL_ALGO_OR_OPT_NEIGHBOR || algo == TL_ALGO_THREE_OPT_NEIGHBOR; }
     bool int_values() const { return metric_is_int(p->metric); }
     // the metric the persistent Mode R kernel recomputes distances in; none when the session reads f32
     // matrix entries (f32 matrix and EXPLICIT sessions)
@@ -237,7 +239,7 @@ tl_status upload_geometry(tl_session *s)
         if (const char *cap = getenv("TL_MAX_GRID")) s->grid = std::max(1, std::min(s->grid, atoi(cap)));
         TL_CUDA_TRY(s->cand.alloc((size_t)s->grid + 1));
         TL_CUDA_TRY(cudaMemsetAsync(s->cand.p, 0xff, ((size_t)s->grid + 1) * sizeof(BestF), s->c->stream)); // no move pending
-        if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR) TL_CUDA_TRY(s->nl_cnt.alloc((size_t)s->grid));
+        if (s->nl_relocating()) TL_CUDA_TRY(s->nl_cnt.alloc((size_t)s->grid));
         return TL_OK;
     }
     if (s->algo == TL_ALGO_OR_OPT) {
@@ -364,6 +366,10 @@ tl_status launch_scan(tl_session *s, bool fuse, bool exchange = true)
         launch_or_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->tmp.p, s->cand.p,
                           s->nl_cnt.p, s->state.p, s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
         s->c->launches++;
+    } else if (s->algo == TL_ALGO_THREE_OPT_NEIGHBOR) {
+        launch_three_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->tmp.p, s->cand.p,
+                             s->nl_cnt.p, s->state.p, s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
+        s->c->launches++;
     } else if (s->nl) {
         launch_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->cand.p, s->state.p,
                        s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
@@ -448,6 +454,12 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
         if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR) { // a long span left pending by the scan's last CTA
             launch_or_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->tmp.p, s->n, s->cand.p + s->grid, s->state.p,
                                s->ticket.p + 1, s->log.p, s->log_cap, apply_grid, st);
+            s->c->launches += 2;
+            continue;
+        }
+        if (s->algo == TL_ALGO_THREE_OPT_NEIGHBOR) { // as Or-opt N
+            launch_three_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->tmp.p, s->n, s->cand.p + s->grid, s->state.p,
+                                  s->ticket.p + 1, s->log.p, s->log_cap, apply_grid, st);
             s->c->launches += 2;
             continue;
         }
@@ -548,7 +560,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     if (cached) algo = TL_ALGO_TWO_OPT_BEST;
     if (algo != TL_ALGO_TWO_OPT_BEST && algo != TL_ALGO_TWO_OPT_BEST_CYCLIC && algo != TL_ALGO_TWO_OPT_REF &&
         algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT && algo != TL_ALGO_TWO_OPT_NEIGHBOR &&
-        algo != TL_ALGO_OR_OPT_NEIGHBOR) {
+        algo != TL_ALGO_OR_OPT_NEIGHBOR && algo != TL_ALGO_THREE_OPT_NEIGHBOR) {
         set_error("tl_session_create: unknown algo %d", algo);
         return TL_ERR_INVALID;
     }
@@ -556,7 +568,8 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         set_error("tl_session_create: unknown path %d", path);
         return TL_ERR_INVALID;
     }
-    const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR || algo == TL_ALGO_OR_OPT_NEIGHBOR;
+    const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR || algo == TL_ALGO_OR_OPT_NEIGHBOR ||
+                    algo == TL_ALGO_THREE_OPT_NEIGHBOR;
     if (nl && (path == TL_PATH_MATRIX || p->kind == PK_EXPLICIT)) {
         // candidate-list searches are for instances whose n^2 matrix is the problem; both metrics are recomputed
         set_error(p->kind == PK_EXPLICIT ? "candidate-list search needs coordinates (EXPLICIT problem)"
@@ -669,7 +682,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         set_error("tl_session_create: device allocation failed");
         return fail(TL_ERR_NOMEM);
     }
-    if (algo == TL_ALGO_OR_OPT_NEIGHBOR && s->tmp.alloc((size_t)s->npad * 16) != cudaSuccess) {
+    if (s->nl_relocating() && s->tmp.alloc((size_t)s->npad * 16) != cudaSuccess) {
         set_error("tl_session_create: device allocation failed");
         return fail(TL_ERR_NOMEM);
     }
@@ -686,8 +699,8 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         if (ce != cudaSuccess) { set_error("tl_session_create: %s", cudaGetErrorString(ce)); return fail(TL_ERR_CUDA); }
     }
     // or_opt::solve and three_opt::solve ignore the seed and return identity order when n < 4
-    // (or_opt.rs:31-34, three_opt.rs:25-28); so does Or-opt N
-    const bool or_like = algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT || algo == TL_ALGO_OR_OPT_NEIGHBOR;
+    // (or_opt.rs:31-34, three_opt.rs:25-28); so do Or-opt N and 3-opt N
+    const bool or_like = algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT || s->nl_relocating();
     std::vector<uint32_t> ident;
     if (or_like && s->trivial) {
         ident.resize(p->n);
@@ -736,8 +749,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         }
         s->src.kind = SRC_EUC_SAFE; // tl_session_tour reads the city fields only
         s->src.pts = s->pts.p;
-        launch_nl_init(p->metric, p->d_xy, d_tour.p, p->n, s->npad, algo == TL_ALGO_OR_OPT_NEIGHBOR, s->pts.p, s->pos.p,
-                       c->stream);
+        launch_nl_init(p->metric, p->d_xy, d_tour.p, p->n, s->npad, s->nl_relocating(), s->pts.p, s->pos.p, c->stream);
         c->launches++;
     } else {
         if (s->pts.alloc(s->npad) != cudaSuccess) { set_error("tl_session_create: device allocation failed"); return fail(TL_ERR_NOMEM); }
@@ -875,7 +887,7 @@ tl_status tl_session_scan(tl_session *s, tl_move *best, int32_t *found)
     TL_CUDA_TRY(cudaStreamSynchronize(s->c->stream));
     if (was_done) { s->h.done = was_done; rc = push_state(s); if (rc != TL_OK) return rc; }
     bool any;
-    const bool three = s->algo == TL_ALGO_THREE_OPT;
+    const bool three = s->algo == TL_ALGO_THREE_OPT || s->algo == TL_ALGO_THREE_OPT_NEIGHBOR;
     const bool or_opt = s->algo == TL_ALGO_OR_OPT || s->algo == TL_ALGO_OR_OPT_NEIGHBOR;
     if (s->int_values()) {
         std::vector<BestI> hi(hc.size());

@@ -459,7 +459,8 @@ Solution run_local_search(const TspProblem &problem, int algo, int path, const P
     // the candidate-list searches serve instances whose packed triangle cannot come to the host (2 TB at
     // 10^6 cities), and the per-move progress values of two_opt.rs and or_opt.rs need it: only the start
     // and the result are sent
-    const bool replay = tx && algo != TL_ALGO_TWO_OPT_NEIGHBOR && algo != TL_ALGO_OR_OPT_NEIGHBOR;
+    const bool replay = tx && algo != TL_ALGO_TWO_OPT_NEIGHBOR && algo != TL_ALGO_OR_OPT_NEIGHBOR &&
+                        algo != TL_ALGO_THREE_OPT_NEIGHBOR;
     std::vector<tl_move> log(replay ? (size_t)1 << 20 : 0);
     tl_stats st{};
     std::vector<uint32_t> before = tour;
@@ -567,13 +568,22 @@ Solution solve(const TspProblem &problem, const HeuristicOptions &, const Progre
 
 namespace three_opt {
 
+Solution solve_with(const TspProblem &problem, const std::string &mode, const ProgressSender *progress_tx,
+                    const std::vector<size_t> *init_tour, uint32_t candidates)
+{
+    const int algo = mode == "neighbor" ? TL_ALGO_THREE_OPT_NEIGHBOR : TL_ALGO_THREE_OPT;
+    // n < 4: identity order, seed ignored, no progress messages (three_opt.rs:25-28)
+    if (problem.cities.size() < 4) return Solution::from_parts(ids_of(problem.cities), problem.cities, problem.distances);
+    if (algo == TL_ALGO_THREE_OPT_NEIGHBOR && candidates)
+        check(tl_problem_set_candidates(problem.distances.impl->prob, candidates), "three_opt");
+    const std::vector<size_t> start = init_tour ? *init_tour : ids_of(problem.cities);
+    return run_local_search(problem, algo, TL_PATH_AUTO, progress_tx, start, "three_opt");
+}
+
 Solution solve(const TspProblem &problem, const HeuristicOptions &, const ProgressSender *progress_tx,
                const std::vector<size_t> *init_tour)
 {
-    // n < 4: identity order, seed ignored, no progress messages (three_opt.rs:25-28)
-    if (problem.cities.size() < 4) return Solution::from_parts(ids_of(problem.cities), problem.cities, problem.distances);
-    const std::vector<size_t> start = init_tour ? *init_tour : ids_of(problem.cities);
-    return run_local_search(problem, TL_ALGO_THREE_OPT, TL_PATH_AUTO, progress_tx, start, "three_opt");
+    return solve_with(problem, "", progress_tx, init_tour);
 }
 
 } // namespace three_opt
@@ -707,7 +717,10 @@ Result<Solution> solve_with_context(Solvers solver, const TspProblem &problem, c
         if (opts.cuda_mode == "neighbor")
             return Result<Solution>::ok(or_opt::solve_with(problem, "neighbor", tx, init_tour, opts.cuda_candidates));
         return Result<Solution>::ok(or_opt::solve(problem, h, tx, init_tour));
-    case Solvers::ThreeOpt: return Result<Solution>::ok(three_opt::solve(problem, h, tx, init_tour));
+    case Solvers::ThreeOpt:
+        if (opts.cuda_mode == "neighbor")
+            return Result<Solution>::ok(three_opt::solve_with(problem, "neighbor", tx, init_tour, opts.cuda_candidates));
+        return Result<Solution>::ok(three_opt::solve(problem, h, tx, init_tour));
     case Solvers::TwoOpt:
         if (opts.cuda_mode.empty() && opts.cuda_path.empty())
             return Result<Solution>::ok(two_opt::solve(problem, h, tx, init_tour));

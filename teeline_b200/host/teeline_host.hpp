@@ -209,10 +209,10 @@ struct AppOptions { // mod.rs:1586-1596; only the sub-tables this path consumes 
     std::optional<HeuristicOptions> heuristic;
     std::optional<AcoOptions> aco;
     std::optional<GAOptions> ga;
-    // extension table [stage.cuda] (never required): mode = "ref"|"best"|"best_cyclic"|"neighbor" (or_opt:
-    // "neighbor"), path = "auto"|"matrix"|"recompute",
+    // extension table [stage.cuda] (never required): mode = "ref"|"best"|"best_cyclic"|"neighbor" (or_opt,
+    // 3opt: "neighbor"), path = "auto"|"matrix"|"recompute",
     // seed = <integer> (the population solvers' Philox key; the reference's RNG is unseeded),
-    // candidates = <integer> (mode "neighbor" of 2opt and or_opt: k of the candidate lists, 1..32;
+    // candidates = <integer> (mode "neighbor" of 2opt, or_opt and 3opt: k of the candidate lists, 1..32;
     // 0 = TL_CANDIDATES_DEFAULT)
     std::string cuda_mode, cuda_path;
     uint64_t cuda_seed = 0;
@@ -240,6 +240,10 @@ Solution solve_with(const TspProblem &problem, const std::string &mode, const Pr
 namespace three_opt { // src/tsp/three_opt.rs:16-52
 Solution solve(const TspProblem &problem, const HeuristicOptions &opts, const ProgressSender *progress_tx,
                const std::vector<size_t> *init_tour);
+// extension: mode "neighbor" runs candidate-list 3-opt with k = candidates (0 = the library's default);
+// any other mode runs solve()'s 3-opt
+Solution solve_with(const TspProblem &problem, const std::string &mode, const ProgressSender *progress_tx,
+                    const std::vector<size_t> *init_tour, uint32_t candidates = 0);
 }
 namespace nearest_neighbor {
 Solution solve(const TspProblem &problem, const HeuristicOptions &opts, const ProgressSender *progress_tx,
