@@ -219,6 +219,21 @@ tl_status tl_problem_set_candidates(tl_problem *p, uint32_t k);
 /* nearest_neighbor::solve (nearest_neighbor.rs:22-70), start at position 0. */
 tl_status tl_nn_tour(tl_problem *p, uint32_t k, uint32_t *tour_out);
 
+/* greedy_edge::solve (src/tsp/greedy_edge.rs): the greedy-edge tour over ALL n(n-1)/2 edges, built on the
+ * device from the candidate lists (kernel K9).  Edge (a, b) with a < b (positions) has the key (d(a, b), a, b),
+ * d in the problem's metric as tl_knn compares it (f32; NINT_I32 values are exact there), compared
+ * lexicographically, so no two edges tie.  Taking the edges in key order, an edge is accepted when both
+ * endpoints have degree < 2 and lie in different fragments; after n-1 accepted edges the two endpoints of the
+ * Hamiltonian path are joined.  The result is this tour whatever the candidate lists are: k changes the speed
+ * only.  tour_out[0] = 0, tour_out[1] = the lower-positioned of city 0's two tour neighbours, then the cycle
+ * (n <= 3: the identity order).
+ * Uses the problem's candidate lists; without any, builds TL_CANDIDATES_DEFAULT lists and keeps them with the
+ * problem, as the first candidate-list session does.  Cities whose listed neighbours are all taken get lists
+ * rebuilt over the cities still free.  EXPLICIT problems: TL_ERR_UNSUPPORTED.  Nothing n^2 is allocated.
+ * stats (nullable): passes = device rounds, moves = accepted edges including the closing one, repermutes =
+ * list rebuilds, launches, device_ms, converged = 1. */
+tl_status tl_greedy_tour(tl_problem *p, uint32_t *tour_out, tl_stats *stats);
+
 /* DistanceMatrix::tour_length_by_pos for a batch (distance_matrix.rs:235-245; GA
  * fitness genetic_algorithm.rs:112-124; ACO ant_colony.rs:138,221).  tours is
  * batch x n positions, row-major.  out_f32[b] (F32 problems) / out_i64[b] (NINT). */

@@ -1,8 +1,10 @@
-"""ctypes loader for the CPU ORACLES of candidate-list 2-opt, Or-opt and 3-opt (oracle_nl/libteeline_oracle_nl.so).
+"""ctypes loader for the CPU ORACLES of candidate-list 2-opt, Or-opt and 3-opt and of the greedy-edge constructor
+(oracle_nl/libteeline_oracle_nl.so).
 
 TEST INFRASTRUCTURE ONLY, like `oracle`: tests and measurement scripts load it, the product package
 (teeline_b200/) never does.  Problems are `oracle.Problem` instances; the definitions are in
-two_opt_nl.h, or_opt_nl.h, three_opt_nl.h and include/teeline_cuda.h (tl_problem_set_candidates).
+two_opt_nl.h, or_opt_nl.h, three_opt_nl.h, greedy_nl.h and include/teeline_cuda.h (tl_problem_set_candidates,
+tl_greedy_tour).
 """
 from __future__ import annotations
 
@@ -22,7 +24,7 @@ _ORACLE_DIR = os.path.dirname(os.path.abspath(O.__file__))
 def build(force: bool = False) -> str:
     """Compile with gcc (oracle_nl/Makefile)."""
     srcs = [os.path.join(_DIR, f) for f in ("two_opt_nl.c", "two_opt_nl.h", "or_opt_nl.c", "or_opt_nl.h", "three_opt_nl.c",
-                                         "three_opt_nl.h", "Makefile")] + \
+                                         "three_opt_nl.h", "greedy_nl.c", "greedy_nl.h", "Makefile")] + \
         [os.path.join(_ORACLE_DIR, f) for f in ("teeline_oracle.c", "algos.inc", "teeline_oracle.h")]
     stale = not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in srcs)
     if force or stale:
@@ -126,3 +128,21 @@ def three_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 
                            C.byref(st), log, _p(ks), C.c_int64(log_cap))
     mv = [(log[m].delta, log[m].i, log[m].j, int(ks[m]), log[m].seg_len) for m in range(min(st.moves, log_cap))]
     return t, st, mv
+
+
+def _greedy(fn, x, y, metric):
+    x = np.ascontiguousarray(x, dtype=np.float32)
+    y = np.ascontiguousarray(y, dtype=np.float32)
+    out = np.empty(len(x), dtype=np.int32)
+    getattr(lib(), fn)(C.c_int32(len(x)), _p(x), _p(y), C.c_int(metric == "nint"), _p(out))
+    return out
+
+
+def greedy_brute(x, y, metric: str = "f32"):
+    """The greedy-edge tour by sorting all n(n-1)/2 edges (metric "f32" or "nint"); a few thousand cities."""
+    return _greedy("tlo_greedy_brute", x, y, metric)
+
+
+def greedy_lazy(x, y, metric: str = "f32"):
+    """The greedy-edge tour by Bentley's lazy greedy on a uniform grid; fast enough for 10^6 cities."""
+    return _greedy("tlo_greedy_lazy", x, y, metric)

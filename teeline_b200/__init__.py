@@ -137,6 +137,14 @@ class Problem:
         capi.check(self._lib.tl_nn_tour(self.h, k, capi.ptr(out)))
         return out
 
+    def greedy_tour(self):
+        """tl_greedy_tour: the greedy-edge tour, built on the device from the candidate lists (default lists
+        are built and kept when there are none).  Returns (tour, Stats)."""
+        out = np.empty(self.n, dtype=np.uint32)
+        st = Stats()
+        capi.check(self._lib.tl_greedy_tour(self.h, capi.ptr(out), C.byref(st)))
+        return out, st
+
     def tour_lengths(self, tours, mode: int = LEN_EXACT) -> np.ndarray:
         t = _u32(tours)
         if t.ndim == 1:

@@ -32,7 +32,7 @@ EXPORTS = [
     "tl_ctx_create", "tl_ctx_create_on_stream", "tl_ctx_destroy", "tl_ctx_sync", "tl_last_error",
     "tl_version", "tl_ctx_launch_count", "tl_nccl_unique_id", "tl_ctx_attach_nccl",
     "tl_problem_create_euc2d", "tl_problem_create_explicit", "tl_problem_destroy",
-    "tl_dist_matrix_packed", "tl_dist_matrix_packed_i32", "tl_knn", "tl_problem_set_candidates", "tl_nn_tour", "tl_tour_lengths",
+    "tl_dist_matrix_packed", "tl_dist_matrix_packed_i32", "tl_knn", "tl_problem_set_candidates", "tl_nn_tour", "tl_greedy_tour", "tl_tour_lengths",
     "tl_tour_lengths_i64", "tl_local_search", "tl_two_opt_batch", "tl_session_create",
     "tl_session_destroy", "tl_session_set_shard", "tl_session_scan", "tl_session_time_scans",
     "tl_session_enqueue",
@@ -111,6 +111,7 @@ def load():
     L.tl_knn.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
     L.tl_problem_set_candidates.argtypes = [C.c_void_p, C.c_uint32]
     L.tl_nn_tour.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
+    L.tl_greedy_tour.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Stats)]
     L.tl_tour_lengths.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]
     L.tl_tour_lengths_i64.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     L.tl_local_search.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64,

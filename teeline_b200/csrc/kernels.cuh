@@ -225,6 +225,38 @@ cudaError_t nn_tour_configure();
 void launch_nn_tour(const float2 *xy, const float *tri, uint32_t n, const uint32_t *knn, uint32_t kk,
                     Metric metric, uint32_t *tour, cudaStream_t st);
 
+// K9 greedy edge (k9_greedy.cu): a round is the best kernel and the accept kernel; the accept kernel's last
+// block ends the round in `status`, and later rounds of an enqueued batch return at once until the host acts
+enum : uint32_t { kGreedyRun = 0, kGreedyStalled = 1, kGreedyDone = 2 };
+struct GreedyState {
+    uint32_t status;    // kGreedyRun; kGreedyStalled: the last round accepted nothing; kGreedyDone: two free cities
+    uint32_t free;      // cities of degree < 2
+    uint32_t round_acc; // edges accepted by the running round
+    uint32_t ticket;
+    unsigned long long rounds, accepted;
+};
+struct GreedyBufs {
+    uint8_t *deg;
+    uint32_t *adj;   // 2n: the two tour neighbours of every city
+    uint32_t *other; // far endpoint of a free city's fragment
+    float *bd;       // per free city: key distance of its best edge or bound
+    uint32_t *bv;    // its partner, | kExhausted for a bound, UINT32_MAX for none
+    uint32_t *oth;   // other[] as the best kernel saw it
+    GreedyState *state;
+};
+constexpr uint32_t kGreedyRefreshK = 16; // width of the lists rebuilt over the free cities (>= 2)
+void launch_greedy_init(uint32_t n, uint8_t *deg, uint32_t *other, GreedyState *gs, cudaStream_t st);
+void launch_greedy_round(const float2 *xy, uint32_t n, Metric metric, const uint32_t *list, uint32_t k, GreedyBufs b,
+                         int grid, cudaStream_t st);
+size_t greedy_refresh_blocks(uint32_t n);
+// the free cities' coordinates and positions in position order (3 launches); blockcnt: greedy_refresh_blocks(n)
+void launch_greedy_compact(const float2 *xy, uint32_t n, const uint8_t *deg, uint32_t *blockcnt, float2 *cxy,
+                           uint32_t *cidx, cudaStream_t st);
+void launch_greedy_map(uint32_t F, uint32_t k, const uint32_t *cidx, const uint32_t *cknn, uint32_t *list, cudaStream_t st);
+// closes the path and writes the tour; succ and dist hold 4n entries each.  Returns the launch count.
+int launch_greedy_emit(uint32_t n, const uint8_t *deg, const uint32_t *other, uint32_t *adj, uint32_t *succ,
+                       uint32_t *dist, uint32_t *tour, cudaStream_t st);
+
 // K2 matrix path
 constexpr int kMatR = 8;                 // diagonals per lane (strided by 32 => coalesced rows)
 constexpr int kMatBW = 32 * kMatR;

@@ -252,6 +252,7 @@ int run_solvers()
 {
     std::printf("solvers on the accelerated (CUDA, sm_100a) path of this build:\n");
     std::printf("  nn | nearest_neighbor        nearest-neighbour constructor (nearest_neighbor.rs)\n");
+    std::printf("  gec | greedy_edge            greedy-edge constructor (greedy_edge.rs), --candidates K\n");
     std::printf("  2opt | two_opt               first-improvement 2-opt, bit-exact with two_opt.rs\n");
     std::printf("  2opt_best | two_opt_best     best-improvement 2-opt (extension)\n");
     std::printf("  2opt --mode neighbor         candidate-list best-improvement 2-opt, --candidates K (extension)\n");

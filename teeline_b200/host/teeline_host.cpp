@@ -142,7 +142,8 @@ bool auto_expand_with_shuffle(Solvers s)
 }
 bool is_accelerated(Solvers s)
 {
-    return s == Solvers::NearestNeighbor || s == Solvers::TwoOpt || s == Solvers::OrOpt || s == Solvers::TwoOptBest ||
+    return s == Solvers::NearestNeighbor || s == Solvers::GreedyEdge || s == Solvers::TwoOpt || s == Solvers::OrOpt ||
+           s == Solvers::TwoOptBest ||
            s == Solvers::ThreeOpt || s == Solvers::AntColony || s == Solvers::GeneticAlgorithm ||
            s == Solvers::RandomShuffle;
 }
@@ -676,6 +677,23 @@ Solution solve(const TspProblem &problem, const GAOptions &o, const ProgressSend
 
 } // namespace genetic_algorithm
 
+namespace greedy_edge {
+
+Solution solve(const TspProblem &problem, const AppOptions &opts, const ProgressSender *tx, const std::vector<size_t> *)
+{
+    // greedy_edge.rs builds its tour from the instance alone: the seed is ignored (stage_warnings says so)
+    const DistanceMatrix &dm = problem.distances;
+    if (opts.cuda_candidates) check(tl_problem_set_candidates(dm.impl->prob, opts.cuda_candidates), "greedy_edge");
+    std::vector<uint32_t> tour(dm.num_cities());
+    check(tl_greedy_tour(dm.impl->prob, tour.data(), nullptr), "greedy_edge");
+    const std::vector<size_t> route = to_ids(tour, dm);
+    Solution s = Solution::from_parts(route, problem.cities, dm);
+    send_final(tx, route, s.total);
+    return s;
+}
+
+} // namespace greedy_edge
+
 namespace random_shuffle {
 
 Solution solve(const TspProblem &problem, uint64_t seed)
@@ -713,6 +731,7 @@ Result<Solution> solve_with_context(Solvers solver, const TspProblem &problem, c
     if (v.is_err()) return Result<Solution>::err(v.error);
     switch (solver) {
     case Solvers::NearestNeighbor: return Result<Solution>::ok(nearest_neighbor::solve(problem, h, tx, init_tour));
+    case Solvers::GreedyEdge: return Result<Solution>::ok(greedy_edge::solve(problem, opts, tx, init_tour));
     case Solvers::OrOpt:
         if (opts.cuda_mode == "neighbor")
             return Result<Solution>::ok(or_opt::solve_with(problem, "neighbor", tx, init_tour, opts.cuda_candidates));
@@ -745,7 +764,7 @@ Result<Solution> solve_with_context(Solvers solver, const TspProblem &problem, c
     case Solvers::Unspecified: return Result<Solution>::err("solver not specified");
     default:
         return Result<Solution>::err(std::string("solver ") + solver_name(solver) +
-                                     " is outside the accelerated path of this build (nn, 2opt, or_opt, 3opt, aco, ga)");
+                                     " is outside the accelerated path of this build (nn, greedy_edge, 2opt, or_opt, 3opt, aco, ga)");
     }
 }
 

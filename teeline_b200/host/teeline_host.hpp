@@ -257,6 +257,11 @@ namespace genetic_algorithm { // src/tsp/genetic_algorithm.rs:16-44
 Solution solve(const TspProblem &problem, const GAOptions &opts, const ProgressSender *progress_tx,
                const std::vector<size_t> *init_tour, uint64_t seed = 0);
 }
+namespace greedy_edge { // src/tsp/greedy_edge.rs: the greedy-edge tour (tl_greedy_tour); the seed is ignored.
+// opts.cuda_candidates (1..32, 0 = keep the problem's lists) sets the width of the candidate lists first
+Solution solve(const TspProblem &problem, const AppOptions &opts, const ProgressSender *progress_tx,
+               const std::vector<size_t> *init_tour);
+}
 namespace random_shuffle { // src/tsp/random_shuffle.rs: a shuffled order of the city ids (splitmix64-seeded here)
 Solution solve(const TspProblem &problem, uint64_t seed = 0);
 }
