@@ -78,13 +78,24 @@ enum {
                                         costs O(n k) instead of O(n^2).  Same problems, paths and limits as
                                         Mode N; n < 4 returns the identity order with no scan, as
                                         TL_ALGO_OR_OPT does. */
-    TL_ALGO_THREE_OPT_NEIGHBOR = 8   /* "3-opt N": TL_ALGO_THREE_OPT's triples, costs, case choice and tie order
+    TL_ALGO_THREE_OPT_NEIGHBOR = 8,  /* "3-opt N": TL_ALGO_THREE_OPT's triples, costs, case choice and tie order
                                         over the triples that the first two candidate edges of a sequential
                                         3-exchange generate (see tl_problem_set_candidates): a step costs
                                         O(n k^2) instead of O(n^3).  Same problems, paths and limits as Or-opt N;
                                         n < 4 returns the identity order with no scan, as TL_ALGO_THREE_OPT
                                         does. */
+    TL_ALGO_TWO_OPT_NEIGHBOR_MULTI = 9 /* "Mode NM": Mode N's pairs, deltas and order, but a step also applies the
+                                        best improving pair of every block of TL_MULTI_BLOCK positions that is
+                                        disjoint from Mode N's move (see tl_problem_set_candidates): far fewer
+                                        steps to a Mode N local optimum.  Same problems, paths and limits as
+                                        Mode N; n < 4 returns the identity order with no scan. */
 };
+
+/* Mode NM's block size in positions (a power of two).  Among 256, 1024 and 4096, 4096 took the fewest steps and
+ * the least time to the optimum of 10^6-city greedy and NN tours on a B200 at a 1000 W power limit (5010 steps,
+ * 0.71 s from greedy; profiles/r05e_two_opt_neighbor_multi_timing.json, DESIGN.md section 5).  Instances of a
+ * few blocks (about 2*10^4 cities) take fewer steps with smaller blocks. */
+#define TL_MULTI_BLOCK 4096
 
 /* where distances come from during the scan */
 enum {
@@ -168,7 +179,7 @@ tl_status tl_dist_matrix_packed_i32(tl_problem *p, int32_t *out); /* NINT_I32 pr
  * ascending distance, ties by lower position, rows padded with UINT32_MAX. */
 tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
 
-/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR, TL_ALGO_OR_OPT_NEIGHBOR and TL_ALGO_THREE_OPT_NEIGHBOR, built
+/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR[_MULTI], TL_ALGO_OR_OPT_NEIGHBOR and TL_ALGO_THREE_OPT_NEIGHBOR, built
  * on the device by
  * tl_knn's kernel and kept with the problem (they depend on the instance only, like
  * lin_kernighan::build_candidates, lin_kernighan.rs:12-27).  K[c] = the first k entries of tl_knn(k)
@@ -209,6 +220,23 @@ tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
  * the largest savings > 0, ties to the lowest (i, j, k); duplicates carry the same key.  stats.evals
  * counts every counted triple, duplicates included.  With k >= n-1 every triple is generated (q = i+1,
  * b = p_j, e2 = j, t = p_j+1, b' = p_k, e1 = i, e3 = k), so the moves are TL_ALGO_THREE_OPT's.
+ *
+ * Mode NM: Mode N's generated pairs, deltas and (delta, i, j) order with strict '< 0'.  Step t (t = the steps
+ * the session has applied so far, 0 for the first step of a tl_local_search call) works on the tour as it stood
+ * at the start of the step:
+ *   1. G = Mode N's move, the argmin over all generated improving pairs; none: converged (Mode N's stop).
+ *   2. With B = TL_MULTI_BLOCK and o = (t mod 2) * B/2, position q lies in block floor((q + o) / B).  A pair
+ *      (i, j) is in-block when i and j+1 lie in the same block (so does every position it reads or writes);
+ *      a block's best is the argmin of (delta, i, j) over its in-block generated improving pairs.
+ *   3. The step applies G and every block best (i, j) other than G with j < i_G or i > j_G.  These share no
+ *      edge with G or with one another, so their start-of-step deltas are their real deltas.
+ *   4. They are logged G first, then by increasing i, each with its start-of-step delta.  stats.moves counts
+ *      logged moves, stats.passes scans and stats.evals generated pairs, as in Mode N.
+ *   5. max_moves >= 0: a step applies the first max_moves - moves of its moves in log order, and the search
+ *      stops with converged = 0.  A budget of m gives the first m moves of the unbudgeted log; a later
+ *      tl_session_run starts a new step with a fresh scan.
+ * With n <= B/2 every pair is in-block at both offsets and the moves are Mode N's; at convergence Mode N's scan
+ * finds no improving pair.  tl_session_scan and tl_session_time_scans scan for G as Mode N does.
  *
  * 1 <= k <= 32 (TL_ERR_INVALID otherwise); EXPLICIT problems: TL_ERR_UNSUPPORTED.  A session copies
  * the lists when it is created, so later calls do not affect it.  Without a call, the first session

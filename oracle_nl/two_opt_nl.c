@@ -6,6 +6,12 @@
 #include <stdlib.h>
 #include <string.h>
 
+/* Mode NM's per-block best: found = 0 for a block without an in-block improving pair */
+typedef struct {
+    int found;
+    tlo_move mv;
+} nl_block;
+
 typedef struct {
     const tlo_problem *p;
     const int32_t *tour, *pos, *cand;
@@ -13,6 +19,9 @@ typedef struct {
     int found;
     tlo_move mv;
     int64_t evals;
+    /* Mode NM only (blk non-null): position q lies in block (q + off) / block */
+    int32_t block, off;
+    nl_block *blk;
 } nl_job;
 
 static int better(double d1, int32_t i1, int32_t j1, double d2, int32_t i2, int32_t j2)
@@ -34,16 +43,25 @@ static double delta_of(const tlo_problem *p, const int32_t *t, int32_t i, int32_
     return (double)((float)(dac + dbd) - (float)(dab + dcd));
 }
 
+static void take(int *found, tlo_move *mv, double d, int32_t i, int32_t j)
+{
+    if (*found && !better(d, i, j, mv->delta, mv->i, mv->j)) return;
+    *found = 1;
+    memset(mv, 0, sizeof *mv);
+    mv->delta = d;
+    mv->i = i;
+    mv->j = j;
+}
+
 static void consider(nl_job *jb, int32_t i, int32_t j)
 {
     jb->evals++;
     const double d = delta_of(jb->p, jb->tour, i, j);
-    if (d < 0.0 && (!jb->found || better(d, i, j, jb->mv.delta, jb->mv.i, jb->mv.j))) {
-        jb->found = 1;
-        memset(&jb->mv, 0, sizeof jb->mv);
-        jb->mv.delta = d;
-        jb->mv.i = i;
-        jb->mv.j = j;
+    if (d >= 0.0) return;
+    take(&jb->found, &jb->mv, d, i, j);
+    if (jb->blk) {
+        const int32_t b = (i + jb->off) / jb->block;
+        if (b == (j + 1 + jb->off) / jb->block) take(&jb->blk[b].found, &jb->blk[b].mv, d, i, j); /* in-block pair */
     }
 }
 
@@ -65,8 +83,10 @@ static void *nl_worker(void *arg)
     return NULL;
 }
 
+/* blk (nullable, nblk entries): Mode NM's per-block bests for blocks of `block` positions shifted by off */
 static int scan_with_pos(const tlo_problem *p, const int32_t *tour, const int32_t *pos, const int32_t *cand,
-                         int32_t k, int nthreads, tlo_move *mv, int64_t *evals)
+                         int32_t k, int nthreads, tlo_move *mv, int64_t *evals, int32_t block, int32_t off,
+                         nl_block *blk, int32_t nblk)
 {
     const int32_t n = p->n;
     if (nthreads < 1) nthreads = 1;
@@ -79,6 +99,9 @@ static int scan_with_pos(const tlo_problem *p, const int32_t *tour, const int32_
         jobs[t].p = p; jobs[t].tour = tour; jobs[t].pos = pos; jobs[t].cand = cand; jobs[t].k = k;
         jobs[t].i0 = (int32_t)((int64_t)n * t / nthreads);
         jobs[t].i1 = (int32_t)((int64_t)n * (t + 1) / nthreads);
+        jobs[t].block = block;
+        jobs[t].off = off;
+        jobs[t].blk = blk ? (nl_block *)calloc((size_t)nblk, sizeof(nl_block)) : NULL;
         if (nthreads > 1)
             pthread_create(&th[t], NULL, nl_worker, &jobs[t]);
         else
@@ -93,6 +116,12 @@ static int scan_with_pos(const tlo_problem *p, const int32_t *tour, const int32_
             *mv = jobs[t].mv;
             found = 1;
         }
+        if (blk) { /* (delta, i, j) is a total order: the merge does not depend on the thread split */
+            for (int32_t b = 0; b < nblk; ++b)
+                if (jobs[t].blk[b].found) take(&blk[b].found, &blk[b].mv, jobs[t].blk[b].mv.delta, jobs[t].blk[b].mv.i,
+                                               jobs[t].blk[b].mv.j);
+            free(jobs[t].blk);
+        }
     }
     if (evals) *evals = ev;
     return found;
@@ -103,7 +132,7 @@ int tlo_two_opt_nl_scan(const tlo_problem *p, const int32_t *tour, const int32_t
 {
     int32_t *pos = (int32_t *)malloc((size_t)(p->n > 0 ? p->n : 1) * 4);
     for (int32_t q = 0; q < p->n; ++q) pos[tour[q]] = q;
-    const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, mv, evals);
+    const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, mv, evals, 0, 0, NULL, 0);
     free(pos);
     return found;
 }
@@ -118,7 +147,7 @@ void tlo_two_opt_nl(const tlo_problem *p, int32_t *tour, const int32_t *cand, in
         if (max_moves >= 0 && st->moves >= max_moves) break;
         tlo_move mv;
         int64_t ev = 0;
-        const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, &mv, &ev);
+        const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, &mv, &ev, 0, 0, NULL, 0);
         st->passes++;
         st->evals += ev;
         if (!found) break;
@@ -128,4 +157,50 @@ void tlo_two_opt_nl(const tlo_problem *p, int32_t *tour, const int32_t *cand, in
         st->moves++;
     }
     free(pos);
+}
+
+static void apply_logged(int32_t *tour, int32_t *pos, const tlo_move *mv, tlo_stats *st, tlo_move *log, int64_t log_cap)
+{
+    tlo_swap_2opt(tour, mv->i + 1, mv->j);
+    for (int32_t q = mv->i + 1; q <= mv->j; ++q) pos[tour[q]] = q;
+    if (log && st->moves < log_cap) log[st->moves] = *mv;
+    st->moves++;
+}
+
+int tlo_two_opt_nl_multi(const tlo_problem *p, int32_t *tour, const int32_t *cand, int32_t k, int32_t block,
+                         int64_t step0, int64_t max_moves, int nthreads, tlo_stats *st, tlo_move *log, int64_t log_cap)
+{
+    st->passes = st->moves = st->evals = 0;
+    const int32_t n = p->n;
+    const int32_t nblk = (n + block - 1) / block + 1;
+    int32_t *pos = (int32_t *)malloc((size_t)(n > 0 ? n : 1) * 4);
+    nl_block *blk = (nl_block *)malloc((size_t)nblk * sizeof(nl_block));
+    for (int32_t q = 0; q < n; ++q) pos[tour[q]] = q;
+    int converged = 0;
+    for (int64_t t = step0;; ++t) {
+        if (max_moves >= 0 && st->moves >= max_moves) break;
+        const int32_t off = (int32_t)(t & 1) * (block / 2);
+        memset(blk, 0, (size_t)nblk * sizeof(nl_block));
+        tlo_move g;
+        int64_t ev = 0;
+        const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, &g, &ev, block, off, blk, nblk);
+        st->passes++;
+        st->evals += ev;
+        if (!found) { converged = 1; break; }
+        /* every block best disjoint from G, in increasing i (blocks are in position order); all of them
+           are read before anything is applied, so the whole step works on the start-of-step tour */
+        int32_t na = 0;
+        for (int32_t b = 0; b < nblk; ++b) {
+            if (!blk[b].found) continue;
+            const tlo_move *m = &blk[b].mv;
+            if (m->i == g.i && m->j == g.j) continue;
+            if (m->j < g.i || m->i > g.j) blk[na++].mv = *m;
+        }
+        apply_logged(tour, pos, &g, st, log, log_cap);
+        for (int32_t a = 0; a < na && !(max_moves >= 0 && st->moves >= max_moves); ++a)
+            apply_logged(tour, pos, &blk[a].mv, st, log, log_cap);
+    }
+    free(blk);
+    free(pos);
+    return converged;
 }

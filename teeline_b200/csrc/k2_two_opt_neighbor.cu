@@ -17,6 +17,18 @@
 // there is none.  The grid size cannot depend on the move: the host queues steps without reading back.
 // The records, pos[] and the candidate lists (16 + 4 + 4k bytes per city) fit L2 up to about 10^6
 // cities, so the scan is a chain of dependent L2 gathers.
+//
+// Mode NM (multi-move, TL_ALGO_TWO_OPT_NEIGHBOR_MULTI; definition in include/teeline_cuda.h): the same
+// scan and G, and in step t (= DevState::scans) position q lies in block (q + o) >> bshift with
+// o = (t & 1) << (bshift - 1).  Every improving pair whose i and j+1 share a block does a 64-bit atomicMin
+// into that block's key: the order-preserving bits of its delta above the in-block offsets
+// (i - base) << bshift | (j - base), which orders a block's pairs by (delta, i, j).  The last CTA reduces G,
+// re-arms the keys while it compacts the block bests disjoint from G into a list in increasing i (a
+// block-wide scan; blocks are in position order), cuts the list at the move budget, writes the log and
+// ends the step.  It reverses a short G itself; the apply grid then reverses a long G cooperatively and
+// each listed block move (at most 2^bshift positions) with one CTA.  These moves touch disjoint edges: a
+// block move and G share at most an end position, whose entering-edge length one of them rewrites and the
+// other never reads (reverse_segment_inplace reads only the coordinates of the records at i and j+1).
 #include "apply.cuh"
 #include "kernels.cuh"
 
@@ -28,6 +40,35 @@ namespace {
 
 constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
+
+// Mode NM's block keys: 32 bits ordered as the delta (negative deltas only; no NaN)
+__device__ __forceinline__ uint32_t order_bits(float d)
+{
+    const uint32_t u = __float_as_uint(d);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ uint32_t order_bits(int32_t d) { return (uint32_t)d ^ 0x80000000u; }
+template <typename V>
+__device__ __forceinline__ V from_order_bits(uint32_t k);
+template <>
+__device__ __forceinline__ float from_order_bits<float>(uint32_t k)
+{
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+template <>
+__device__ __forceinline__ int32_t from_order_bits<int32_t>(uint32_t k) { return (int32_t)(k ^ 0x80000000u); }
+
+// an improving pair (i, j): offer it to its block when i and j+1 lie in the same block
+template <typename V>
+__device__ __forceinline__ void block_offer(const NlMulti &M, uint32_t off, V d, uint32_t i, uint32_t j)
+{
+    const uint32_t b = (i + off) >> M.bshift;
+    if (b != (j + 1 + off) >> M.bshift) return;
+    const uint32_t base = (b << M.bshift) - off; // wraps for block 0 at odd steps; the differences below do not
+    const unsigned long long key =
+        ((unsigned long long)order_bits(d) << 32) | (((i - base) << M.bshift) | (j - base));
+    atomicMin(M.keys + b, key);
+}
 
 // Tail of a fused step, run by the last CTA: reduce the per-CTA records, count the step's evaluated
 // pairs, then either reverse a short segment here and finish the step, or leave a long one pending.
@@ -70,11 +111,110 @@ __device__ __noinline__ void nl_tail(const Pol &P, uint32_t *pos, Best<typename 
     if (threadIdx.x == 0) finish_best_step(state, hdr, found, (float)v.delta, v.i, v.j, log, log_cap);
 }
 
+// Tail of a fused Mode NM step, run by the last CTA: nl_tail's G, then the accepted block bests.
 template <class Pol>
+__device__ __noinline__ void nlm_tail(const Pol &P, uint32_t *pos, Best<typename Pol::V> *blockbest, DevState *state,
+                                      unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap,
+                                      const NlMulti &M, uint32_t off)
+{
+    using V = typename Pol::V;
+    __shared__ Best<V> red[WARPS];
+    __shared__ unsigned long long red_cnt[WARPS];
+    __shared__ unsigned long long s_moves;
+    __shared__ long long s_max;
+    __shared__ uint32_t s_wcnt[WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    StateHeader hdr{};
+    if (threadIdx.x == 0) {
+        hdr = load_state_header(state);
+        s_moves = hdr.h0.x;
+        s_max = hdr.h1.x;
+    }
+    Best<V> v{(V)0, 0xffffffffu, 0xffffffffu, 0u};
+    unsigned long long cnt = 0;
+    for (int c = threadIdx.x; c < (int)gridDim.x; c += blockDim.x) {
+        const int4 raw = __ldcg(reinterpret_cast<const int4 *>(blockbest) + c);
+        const Best<V> o{Val<V>::from_bits(raw.x), (uint32_t)raw.y, (uint32_t)raw.z, (uint32_t)raw.w};
+        cnt += o.aux;
+        if (TwoOptOrder::better(o, v)) v = o;
+    }
+#pragma unroll
+    for (int off2 = 16; off2 > 0; off2 >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off2);
+    if (lane == 0) red_cnt[warp] = cnt;
+    v = block_argmin<WARPS, TwoOptOrder>(v, red); // its barrier publishes red_cnt, s_moves and s_max too
+    cnt = 0;
+#pragma unroll
+    for (int w = 0; w < WARPS; ++w) cnt += red_cnt[w];
+    const bool found = v.i != 0xffffffffu;
+    const unsigned long long m = s_moves;
+    // block moves this step may still apply after G (G always fits: the step runs only below the budget)
+    const unsigned long long allow = s_max < 0 ? ~0ull : (unsigned long long)s_max - m - 1;
+    // without G no pair improves, so no key was set
+    uint32_t taken = 0;
+    if (found) {
+        for (uint32_t c0 = 0; c0 < M.nslots; c0 += THREADS) {
+            const uint32_t b = c0 + threadIdx.x;
+            bool acc = false;
+            uint32_t mi = 0, mj = 0;
+            V d = (V)0;
+            if (b < M.nslots) {
+                const unsigned long long key = __ldcg(M.keys + b);
+                if (key != ~0ull) {
+                    M.keys[b] = ~0ull; // re-armed for the next step
+                    const uint32_t low = (uint32_t)key, base = (b << M.bshift) - off;
+                    mi = base + (low >> M.bshift);
+                    mj = base + (low & ((1u << M.bshift) - 1u));
+                    d = from_order_bits<V>((uint32_t)(key >> 32));
+                    acc = !(mi == v.i && mj == v.j) && (mj < v.i || mi > v.j);
+                }
+            }
+            const uint32_t bal = __ballot_sync(0xffffffffu, acc);
+            if (lane == 0) s_wcnt[warp] = __popc(bal);
+            __syncthreads();
+            uint32_t before = 0, total = 0;
+#pragma unroll
+            for (int w = 0; w < WARPS; ++w) {
+                before += w < warp ? s_wcnt[w] : 0u;
+                total += s_wcnt[w];
+            }
+            const uint32_t rank = taken + before + __popc(bal & ((1u << lane) - 1u));
+            if (acc && rank < allow) {
+                M.list[rank] = make_uint2(mi, mj);
+                const unsigned long long e = m + 1 + rank;
+                if (log && e < log_cap) log[e] = tl_move{(float)d, mi, mj, 0, 0, 0};
+            }
+            taken += total;
+            __syncthreads(); // s_wcnt is rewritten by the next round
+        }
+    }
+    const uint32_t napply = (uint32_t)min((unsigned long long)taken, allow);
+    const bool long_seg = found && (v.j - v.i) / 2 > (uint32_t)kNlCtaSwaps;
+    if (threadIdx.x == 0) {
+        state->computed += cnt;
+        M.desc[0] = napply;
+        M.desc[1] = long_seg ? v.i : 0xffffffffu;
+        M.desc[2] = v.j;
+        *ticket = 0u;
+        state->scans = hdr.h0.y + 1;
+        if (found) {
+            if (log && m < log_cap) log[m] = tl_move{(float)v.delta, v.i, v.j, 0, 0, 0};
+            const unsigned long long moves = m + 1 + napply;
+            state->moves = moves;
+            if (s_max >= 0 && (long long)moves >= s_max) state->done = 1;
+        } else {
+            state->done = 1;
+            state->converged = 1;
+        }
+    }
+    if (found && !long_seg) reverse_segment_inplace(P, v.i, v.j, nullptr, threadIdx.x, blockDim.x, false, V(), V(), pos);
+}
+
+// MULTI: Mode NM's fused step (block keys and nlm_tail); otherwise Mode N's scan
+template <bool MULTI, class Pol>
 __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     two_opt_nl_scan_kernel(Pol P, uint32_t *__restrict__ pos, const uint32_t *__restrict__ cand, uint32_t k,
                            uint32_t n, Best<typename Pol::V> *blockbest, DevState *state, unsigned int *ticket,
-                           tl_move *__restrict__ log, uint64_t log_cap, int fuse_apply)
+                           tl_move *__restrict__ log, uint64_t log_cap, int fuse_apply, NlMulti M)
 {
     using V = typename Pol::V;
     using Rec = typename Pol::Rec;
@@ -82,6 +222,9 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     griddep_wait(); // the previous step's move is applied and visible from here on
     // uniform across the grid: only a step's tail or apply grid writes it, after every CTA has finished
     if (*reinterpret_cast<const volatile int *>(&state->done)) return;
+    // Mode NM: this step's block offset (scans is only written by a step's tail, after every CTA has read it)
+    uint32_t off = 0;
+    if (MULTI) off = ((uint32_t)*reinterpret_cast<const volatile unsigned long long *>(&state->scans) & 1u) << (M.bshift - 1);
 
     V best = (V)0;
     uint32_t bi = 0xffffffffu, bj = 0xffffffffu, cnt = 0;
@@ -101,6 +244,7 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
             const Rec a = P.load(lo + 1), c = P.load(hi + 1);
             const V d = Val<V>::sub(Val<V>::add(shared, P.dist(a, c)), Val<V>::add(Pol::sp(a), Pol::sp(c)));
             ++cnt;
+            if (MULTI && d < (V)0) block_offer(M, off, d, lo, hi);
             if (d < (V)0 && better_2opt(d, lo, hi, best, bi, bj)) {
                 best = d;
                 bi = lo;
@@ -111,6 +255,7 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
             const Rec a = P.load(lo - 1), c = P.load(hi - 1);
             const V d = Val<V>::sub(Val<V>::add(P.dist(a, c), shared), Val<V>::add(Pol::sp(rlo), Pol::sp(rhi)));
             ++cnt;
+            if (MULTI && d < (V)0) block_offer(M, off, d, lo - 1, hi - 1);
             if (d < (V)0 && better_2opt(d, lo - 1, hi - 1, best, bi, bj)) {
                 best = d;
                 bi = lo - 1;
@@ -138,7 +283,36 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     if (threadIdx.x == 0) s_last = (ticket_take_acq_rel(ticket) == gridDim.x - 1) ? 1u : 0u; // thread 0 wrote blockbest
     __syncthreads();
     if (!s_last) return;
-    nl_tail(P, pos, blockbest, state, ticket, log, log_cap);
+    if (MULTI)
+        nlm_tail(P, pos, blockbest, state, ticket, log, log_cap, M, off);
+    else
+        nl_tail(P, pos, blockbest, state, ticket, log, log_cap);
+}
+
+// Mode NM's apply grid, launched after every step's scan: desc (written by nlm_tail) names a pending long G,
+// reversed by the whole grid, and the count of listed block moves, each reversed by one CTA.  The last CTA
+// to finish resets desc, so a later no-op step applies nothing.
+template <class Pol>
+__global__ void __launch_bounds__(256)
+    apply_multi_kernel(Pol P, uint32_t *pos, const uint2 *__restrict__ list, uint32_t *desc, unsigned int *ticket)
+{
+    using V = typename Pol::V;
+    griddep_wait(); // PDL: the step's scan has finished and its writes are visible
+    const uint32_t cnt = __ldcg(desc), gi = __ldcg(desc + 1), gj = __ldcg(desc + 2);
+    if (cnt == 0 && gi == 0xffffffffu) return; // uniform over the grid
+    if (gi != 0xffffffffu)
+        reverse_segment_inplace(P, gi, gj, nullptr, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x,
+                                false, V(), V(), pos);
+    for (uint32_t c = blockIdx.x; c < cnt; c += gridDim.x) {
+        const uint2 mv = list[c];
+        reverse_segment_inplace(P, mv.x, mv.y, nullptr, threadIdx.x, blockDim.x, false, V(), V(), pos);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && atomicAdd(ticket, 1u) == gridDim.x - 1) { // every CTA has read desc
+        *ticket = 0u;
+        desc[0] = 0u;
+        desc[1] = 0xffffffffu;
+    }
 }
 
 // tour-ordered records (entering-edge length in the policy's metric) and pos[city] = position.
@@ -186,16 +360,32 @@ void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint3
 
 void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
                     DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
-                    cudaStream_t st)
+                    cudaStream_t st, const NlMulti *multi)
 {
     cudaLaunchAttribute attr[1];
     const cudaLaunchConfig_t cfg = pdl_config(grid, THREADS, 0, attr, st);
     const int fuse = fuse_apply ? 1 : 0;
+    const NlMulti mm = multi ? *multi : NlMulti{};
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
-        cudaLaunchKernelEx(&cfg, two_opt_nl_scan_kernel<Pol>, Pol{pts}, pos, cand, k, n,
-                           reinterpret_cast<Best<typename Pol::V> *>(blockbest), state, ticket, log, (uint64_t)log_cap,
-                           fuse);
+        auto *bb = reinterpret_cast<Best<typename Pol::V> *>(blockbest);
+        if (multi && fuse_apply) // a scan without its step (tl_session_scan) leaves the block keys alone
+            cudaLaunchKernelEx(&cfg, two_opt_nl_scan_kernel<true, Pol>, Pol{pts}, pos, cand, k, n, bb, state, ticket, log,
+                               (uint64_t)log_cap, fuse, mm);
+        else
+            cudaLaunchKernelEx(&cfg, two_opt_nl_scan_kernel<false, Pol>, Pol{pts}, pos, cand, k, n, bb, state, ticket,
+                               log, (uint64_t)log_cap, fuse, mm);
+    });
+}
+
+void launch_nlm_apply(Metric metric, Pt *pts, uint32_t *pos, const NlMulti &multi, unsigned int *ticket, int grid,
+                      cudaStream_t st)
+{
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
+    with_metric(metric, [&](auto M) {
+        using Pol = NlPol<M>;
+        cudaLaunchKernelEx(&cfg, apply_multi_kernel<Pol>, Pol{pts}, pos, (const uint2 *)multi.list, multi.desc, ticket);
     });
 }
 

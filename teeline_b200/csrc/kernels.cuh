@@ -304,18 +304,32 @@ void launch_two_opt_cached_step(const Src &src, uint32_t n, int cyclic, unsigned
 
 // K2 candidate-list 2-opt, "Mode N" (k2_two_opt_neighbor.cu): distances recomputed in the problem's
 // metric.  blockbest holds grid + 1 records: one per CTA and, at [grid], the step's pending long move
-// for the apply grid.
+// for the apply grid (Mode N only).
 constexpr int kNlThreads = 256;
 constexpr int kNlMinBlocks = 2;
 constexpr int kNlCtaSwaps = 2048; // segments of up to this many swapped pairs are reversed by the reducing CTA
 // cyclic: Or-opt N's records (position 0 carries the closing edge, position n is the wrap copy)
 void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint32_t n, uint32_t npad, bool cyclic,
                     Pt *pts, uint32_t *pos, cudaStream_t st);
+// Multi-move candidate-list 2-opt, "Mode NM" (same file): Mode N's scan, plus one 64-bit key per block of
+// 2^bshift positions (order-preserving delta bits << 32 | in-block offsets of i and j), re-armed to ~0 by
+// the step's last CTA.  That CTA lists the accepted block moves (i, j) in `list` and leaves
+// desc = {block moves to apply, pending long G's i, its j} (i = ~0: none) for the apply grid, which resets it.
+struct NlMulti {
+    unsigned long long *keys; // nslots = ceil(n / 2^bshift) + 1
+    uint2 *list;              // nslots
+    uint32_t *desc;           // 3
+    uint32_t bshift, nslots;
+};
+// multi (nullable): a fused scan also keeps Mode NM's block bests and ends the step as Mode NM
 void launch_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *blockbest,
                     DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, bool fuse_apply, int grid,
-                    cudaStream_t st);
+                    cudaStream_t st, const NlMulti *multi = nullptr);
 void launch_nl_apply(Metric metric, Pt *pts, uint32_t *pos, const void *pending, DevState *state, unsigned int *ticket,
                      tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
+// Mode NM's apply grid: a pending long G cooperatively, each listed block move by one CTA
+void launch_nlm_apply(Metric metric, Pt *pts, uint32_t *pos, const NlMulti &multi, unsigned int *ticket, int grid,
+                      cudaStream_t st);
 
 // K3 candidate-list Or-opt, "Or-opt N" (k3_or_opt_neighbor.cu): Mode N's records (cyclic), pos[] and
 // lists.  blockbest holds grid + 1 records as in Mode N, blockcnt the grid per-CTA candidate counts;

@@ -85,6 +85,12 @@ struct tl_session {
     DevBuf<uint32_t> nl_cand;        // n x nl_k
     uint32_t nl_k = 0;
     DevBuf<unsigned long long> nl_cnt; // Or-opt N, 3-opt N: per-CTA counts of evaluated candidates
+    // Mode NM (TL_ALGO_TWO_OPT_NEIGHBOR_MULTI): per-block keys, the step's accepted block moves, apply descriptor
+    DevBuf<unsigned long long> nlm_keys;
+    DevBuf<uint2> nlm_list;
+    DevBuf<uint32_t> nlm_desc;
+    NlMulti nlm{};
+    int nlm_grid = 1; // the apply grid: fixed per session, since steps are queued without reading back
 
     DevBuf<BestF> cand; // shard_count * grid records (BestF and BestI have the same layout)
     DevBuf<DevState> state;
@@ -106,6 +112,7 @@ struct tl_session {
     bool matrix() const { return path_used == TL_PATH_MATRIX; }
     // the candidate-list searches that relocate a span of positions (cyclic records, staging buffer, counts)
     bool nl_relocating() const { return algo == TL_ALGO_OR_OPT_NEIGHBOR || algo == TL_ALGO_THREE_OPT_NEIGHBOR; }
+    bool nl_multi() const { return algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI; }
     bool int_values() const { return metric_is_int(p->metric); }
     // the metric the persistent Mode R kernel recomputes distances in; none when the session reads f32
     // matrix entries (f32 matrix and EXPLICIT sessions)
@@ -240,6 +247,24 @@ tl_status upload_geometry(tl_session *s)
         TL_CUDA_TRY(s->cand.alloc((size_t)s->grid + 1));
         TL_CUDA_TRY(cudaMemsetAsync(s->cand.p, 0xff, ((size_t)s->grid + 1) * sizeof(BestF), s->c->stream)); // no move pending
         if (s->nl_relocating()) TL_CUDA_TRY(s->nl_cnt.alloc((size_t)s->grid));
+        if (s->nl_multi()) {
+            NlMulti &m = s->nlm;
+            m.nslots = (uint32_t)((s->n + (1u << m.bshift) - 1) >> m.bshift) + 1;
+            TL_CUDA_TRY(s->nlm_keys.alloc(m.nslots));
+            TL_CUDA_TRY(s->nlm_list.alloc(m.nslots));
+            TL_CUDA_TRY(s->nlm_desc.alloc(3));
+            TL_CUDA_TRY(cudaMemsetAsync(s->nlm_keys.p, 0xff, (size_t)m.nslots * 8, s->c->stream)); // no key
+            TL_CUDA_TRY(cudaMemsetAsync(s->nlm_desc.p, 0xff, 12, s->c->stream));
+            TL_CUDA_TRY(cudaMemsetAsync(s->nlm_desc.p, 0, 4, s->c->stream)); // nothing to apply
+            m.keys = s->nlm_keys.p;
+            m.list = s->nlm_list.p;
+            m.desc = s->nlm_desc.p;
+            // one CTA per block move (up to two per SM), at least Mode N's apply grid for a long G
+            const uint32_t half_pairs = (s->n / 2 + 255) / 256;
+            s->nlm_grid = (int)std::max<uint32_t>(std::min<uint32_t>(half_pairs, (uint32_t)s->c->sm_count),
+                                                  std::min<uint32_t>(m.nslots, 2u * (uint32_t)s->c->sm_count));
+            s->nlm_grid = std::max(1, s->nlm_grid);
+        }
         return TL_OK;
     }
     if (s->algo == TL_ALGO_OR_OPT) {
@@ -372,7 +397,7 @@ tl_status launch_scan(tl_session *s, bool fuse, bool exchange = true)
         s->c->launches++;
     } else if (s->nl) {
         launch_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->cand.p, s->state.p,
-                       s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
+                       s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st, s->nl_multi() ? &s->nlm : nullptr);
         s->c->launches++;
     } else if (s->algo == TL_ALGO_THREE_OPT) {
         TL_CUDA_TRY(cudaMemsetAsync(s->or_ticket.p, 0, 4, st)); // re-arm the work queue
@@ -461,6 +486,11 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
             launch_three_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->tmp.p, s->n, s->cand.p + s->grid, s->state.p,
                                   s->ticket.p + 1, s->log.p, s->log_cap, apply_grid, st);
             s->c->launches += 2;
+            continue;
+        }
+        if (s->nl_multi()) { // the step's block moves and a pending long G (none: the grid leaves at once)
+            launch_nlm_apply(s->p->metric, s->pts.p, s->pos.p, s->nlm, s->ticket.p + 1, s->nlm_grid, st);
+            s->c->launches++;
             continue;
         }
         if (s->nl) { // a long segment left pending by the scan's last CTA (none: the grid leaves at once)
@@ -560,7 +590,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     if (cached) algo = TL_ALGO_TWO_OPT_BEST;
     if (algo != TL_ALGO_TWO_OPT_BEST && algo != TL_ALGO_TWO_OPT_BEST_CYCLIC && algo != TL_ALGO_TWO_OPT_REF &&
         algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT && algo != TL_ALGO_TWO_OPT_NEIGHBOR &&
-        algo != TL_ALGO_OR_OPT_NEIGHBOR && algo != TL_ALGO_THREE_OPT_NEIGHBOR) {
+        algo != TL_ALGO_OR_OPT_NEIGHBOR && algo != TL_ALGO_THREE_OPT_NEIGHBOR && algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI) {
         set_error("tl_session_create: unknown algo %d", algo);
         return TL_ERR_INVALID;
     }
@@ -569,7 +599,18 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         return TL_ERR_INVALID;
     }
     const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR || algo == TL_ALGO_OR_OPT_NEIGHBOR ||
-                    algo == TL_ALGO_THREE_OPT_NEIGHBOR;
+                    algo == TL_ALGO_THREE_OPT_NEIGHBOR || algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
+    // Mode NM's block size: TL_MULTI_BLOCK, or the TL_MULTI_BLOCK environment variable (a power of two in
+    // 2..65536) for measuring other sizes
+    uint32_t multi_block = TL_MULTI_BLOCK;
+    if (const char *ev = getenv("TL_MULTI_BLOCK"); ev && algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI) {
+        const long b = atol(ev);
+        if (b < 2 || b > 65536 || (b & (b - 1))) {
+            set_error("TL_MULTI_BLOCK=%s: must be a power of two in 2..65536", ev);
+            return TL_ERR_INVALID;
+        }
+        multi_block = (uint32_t)b;
+    }
     if (nl && (path == TL_PATH_MATRIX || p->kind == PK_EXPLICIT)) {
         // candidate-list searches are for instances whose n^2 matrix is the problem; both metrics are recomputed
         set_error(p->kind == PK_EXPLICIT ? "candidate-list search needs coordinates (EXPLICIT problem)"
@@ -596,6 +637,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     s->algo = algo;
     s->cached = cached;
     s->nl = nl;
+    while ((1u << s->nlm.bshift) < multi_block) ++s->nlm.bshift;
     s->path_used = want_matrix ? TL_PATH_MATRIX : TL_PATH_RECOMPUTE;
     s->n = p->n;
     s->cyclic = algo == TL_ALGO_TWO_OPT_BEST_CYCLIC || algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT;
@@ -700,7 +742,8 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     }
     // or_opt::solve and three_opt::solve ignore the seed and return identity order when n < 4
     // (or_opt.rs:31-34, three_opt.rs:25-28); so do Or-opt N and 3-opt N
-    const bool or_like = algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT || s->nl_relocating();
+    // (Mode NM too: a new mode, defined with no scan for n < 4)
+    const bool or_like = algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT || s->nl_relocating() || s->nl_multi();
     std::vector<uint32_t> ident;
     if (or_like && s->trivial) {
         ident.resize(p->n);
@@ -971,7 +1014,9 @@ tl_status tl_session_run(tl_session *s, int64_t max_moves)
     // past convergence (or past max_moves, which the device checks itself) are no-op launches.
     // with a move budget every step applies exactly one move (or finds none and stops), so the host
     // knows how many steps are still worth queueing without looking at the device
-    const bool budgeted = max_moves >= 0 && s->algo != TL_ALGO_TWO_OPT_REF;
+    // (not so for Mode R, whose persistent kernel stops by itself, and Mode NM, whose steps apply several
+    // moves: both get unbudgeted batches and the device stops at the budget)
+    const bool budgeted = max_moves >= 0 && s->algo != TL_ALGO_TWO_OPT_REF && s->algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
     int64_t budget = budgeted ? max_moves - (int64_t)s->h.moves : 0;
     auto issue = [&](int slot) -> tl_status {
         uint32_t batch = s->algo == TL_ALGO_TWO_OPT_REF ? 64 : 32;

@@ -461,7 +461,7 @@ Solution run_local_search(const TspProblem &problem, int algo, int path, const P
     // 10^6 cities), and the per-move progress values of two_opt.rs and or_opt.rs need it: only the start
     // and the result are sent
     const bool replay = tx && algo != TL_ALGO_TWO_OPT_NEIGHBOR && algo != TL_ALGO_OR_OPT_NEIGHBOR &&
-                        algo != TL_ALGO_THREE_OPT_NEIGHBOR;
+                        algo != TL_ALGO_THREE_OPT_NEIGHBOR && algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
     std::vector<tl_move> log(replay ? (size_t)1 << 20 : 0);
     tl_stats st{};
     std::vector<uint32_t> before = tour;
@@ -529,8 +529,9 @@ Solution solve_with(const TspProblem &problem, const std::string &mode, const st
     else if (mode == "best") algo = TL_ALGO_TWO_OPT_BEST;
     else if (mode == "best_cyclic") algo = TL_ALGO_TWO_OPT_BEST_CYCLIC;
     else if (mode == "neighbor") algo = TL_ALGO_TWO_OPT_NEIGHBOR;
-    else throw std::runtime_error("unknown 2-opt mode `" + mode + "` (ref | best | best_cyclic | neighbor)");
-    if (algo == TL_ALGO_TWO_OPT_NEIGHBOR && candidates)
+    else if (mode == "neighbor_multi") algo = TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
+    else throw std::runtime_error("unknown 2-opt mode `" + mode + "` (ref | best | best_cyclic | neighbor | neighbor_multi)");
+    if ((algo == TL_ALGO_TWO_OPT_NEIGHBOR || algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI) && candidates)
         check(tl_problem_set_candidates(problem.distances.impl->prob, candidates), "two_opt");
     const std::vector<size_t> start = init_tour ? *init_tour : ids_of(problem.cities); // two_opt.rs:18-20
     return run_local_search(problem, algo, path_code(path), progress_tx, start, "two_opt");

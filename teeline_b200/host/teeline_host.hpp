@@ -209,10 +209,10 @@ struct AppOptions { // mod.rs:1586-1596; only the sub-tables this path consumes 
     std::optional<HeuristicOptions> heuristic;
     std::optional<AcoOptions> aco;
     std::optional<GAOptions> ga;
-    // extension table [stage.cuda] (never required): mode = "ref"|"best"|"best_cyclic"|"neighbor" (or_opt,
-    // 3opt: "neighbor"), path = "auto"|"matrix"|"recompute",
+    // extension table [stage.cuda] (never required): mode = "ref"|"best"|"best_cyclic"|"neighbor"|"neighbor_multi"
+    // (or_opt, 3opt: "neighbor"), path = "auto"|"matrix"|"recompute",
     // seed = <integer> (the population solvers' Philox key; the reference's RNG is unseeded),
-    // candidates = <integer> (mode "neighbor" of 2opt, or_opt and 3opt: k of the candidate lists, 1..32;
+    // candidates = <integer> (modes "neighbor" and "neighbor_multi": k of the candidate lists, 1..32;
     // 0 = TL_CANDIDATES_DEFAULT)
     std::string cuda_mode, cuda_path;
     uint64_t cuda_seed = 0;
@@ -223,8 +223,8 @@ struct AppOptions { // mod.rs:1586-1596; only the sub-tables this path consumes 
 namespace two_opt {
 Solution solve(const TspProblem &problem, const HeuristicOptions &opts, const ProgressSender *progress_tx,
                const std::vector<size_t> *init_tour);
-// extension: best-improvement mode / explicit path selection ("ref"|"best"|"best_cyclic"|"neighbor",
-// "auto"|"matrix"|"recompute"); candidates: k of mode "neighbor" (0 = the library's default)
+// extension: best-improvement mode / explicit path selection ("ref"|"best"|"best_cyclic"|"neighbor"|"neighbor_multi",
+// "auto"|"matrix"|"recompute"); candidates: k of modes "neighbor" and "neighbor_multi" (0 = the library's default)
 Solution solve_with(const TspProblem &problem, const std::string &mode, const std::string &path,
                     const ProgressSender *progress_tx, const std::vector<size_t> *init_tour,
                     uint32_t candidates = 0);
