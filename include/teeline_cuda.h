@@ -84,11 +84,16 @@ enum {
                                         O(n k^2) instead of O(n^3).  Same problems, paths and limits as Or-opt N;
                                         n < 4 returns the identity order with no scan, as TL_ALGO_THREE_OPT
                                         does. */
-    TL_ALGO_TWO_OPT_NEIGHBOR_MULTI = 9 /* "Mode NM": Mode N's pairs, deltas and order, but a step also applies the
+    TL_ALGO_TWO_OPT_NEIGHBOR_MULTI = 9, /* "Mode NM": Mode N's pairs, deltas and order, but a step also applies the
                                         best improving pair of every block of TL_MULTI_BLOCK positions that is
                                         disjoint from Mode N's move (see tl_problem_set_candidates): far fewer
                                         steps to a Mode N local optimum.  Same problems, paths and limits as
                                         Mode N; n < 4 returns the identity order with no scan. */
+    TL_ALGO_OR_OPT_NEIGHBOR_MULTI = 10 /* "Or-opt NM": Or-opt N's moves, deltas, threshold and order, but a step also
+                                        applies the best move of every block of TL_OR_MULTI_BLOCK positions that does
+                                        not touch Or-opt N's move (see tl_problem_set_candidates): far fewer steps
+                                        to an Or-opt N local optimum.  Same problems, paths and limits as Or-opt N;
+                                        n < 4 returns the identity order with no scan. */
 };
 
 /* Mode NM's block size in positions (a power of two).  Among 256, 1024 and 4096, 4096 took the fewest steps and
@@ -96,6 +101,11 @@ enum {
  * 0.71 s from greedy; profiles/r05e_two_opt_neighbor_multi_timing.json, DESIGN.md section 5).  Instances of a
  * few blocks (about 2*10^4 cities) take fewer steps with smaller blocks. */
 #define TL_MULTI_BLOCK 4096
+/* Or-opt NM's block size in positions (a power of two, at most 16384).  Among 1024, 4096 and 16384, 16384 took the
+ * fewest steps and the least time from the Mode NM optima of 10^6-city greedy and NN tours on a B200 at a 1000 W
+ * power limit (1176 steps, 0.28 s from greedy against 0.37 s for 4096; profiles/r05f_or_opt_neighbor_multi_timing.json,
+ * DESIGN.md section 5).  At 10^5 cities 4096 took half the time of 16384. */
+#define TL_OR_MULTI_BLOCK 16384
 
 /* where distances come from during the scan */
 enum {
@@ -179,7 +189,8 @@ tl_status tl_dist_matrix_packed_i32(tl_problem *p, int32_t *out); /* NINT_I32 pr
  * ascending distance, ties by lower position, rows padded with UINT32_MAX. */
 tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
 
-/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR[_MULTI], TL_ALGO_OR_OPT_NEIGHBOR and TL_ALGO_THREE_OPT_NEIGHBOR, built
+/* Candidate lists for TL_ALGO_TWO_OPT_NEIGHBOR[_MULTI], TL_ALGO_OR_OPT_NEIGHBOR[_MULTI] and TL_ALGO_THREE_OPT_NEIGHBOR,
+ * built
  * on the device by
  * tl_knn's kernel and kept with the problem (they depend on the instance only, like
  * lin_kernighan::build_candidates, lin_kernighan.rs:12-27).  K[c] = the first k entries of tl_knn(k)
@@ -237,6 +248,31 @@ tl_status tl_knn(tl_problem *p, uint32_t k, uint32_t *out);
  *      tl_session_run starts a new step with a fresh scan.
  * With n <= B/2 every pair is in-block at both offsets and the moves are Mode N's; at convergence Mode N's scan
  * finds no improving pair.  tl_session_scan and tl_session_time_scans scan for G as Mode N does.
+ *
+ * Or-opt NM: Or-opt N's generated moves, legality, deltas, threshold and (delta, s, i, j, reversed) order.  Step t
+ * (t = the steps the session has applied so far) works on the tour as it stood at the start of the step:
+ *   1. G = Or-opt N's move, the minimum over all generated legal moves below the threshold; none: converged
+ *      (Or-opt N's stop).
+ *   2. The hull of a move (i, s, j, reversed) is [a0, a1] with a0 = min(i-1, j), a1 = max(i+s, j+1).  A move wraps
+ *      when it touches the closing edge: i = 0, i+s = n or j = n-1.  Every position its delta reads is in the hull,
+ *      and so is every position its relocation writes (the relocated span is [a0+1, a1-1], and a1 gets a new
+ *      entering edge); the cities at a0 and a1 do not move.
+ *   3. With B = TL_OR_MULTI_BLOCK and o = (t mod 2) * B/2, position q lies in block floor((q + o) / B).  A move that
+ *      does not wrap is in-block when a0 and a1 lie in the same block; a block's best is the minimum, in Or-opt N's
+ *      order, over its in-block generated legal moves below the threshold.
+ *   4. If G wraps, the step applies G alone.  Otherwise it applies G and every block best with a1 <= g0 or a0 >= g1,
+ *      [g0, g1] being G's hull.  Hulls of different blocks are disjoint, and a block best shares at most an end
+ *      position with G, which keeps its city and whose entering edge only one of the two rewrites: every
+ *      start-of-step delta is the move's real delta, and applying the moves one after another in log order gives
+ *      the same tour.
+ *   5. They are logged G first, then by increasing block (so by increasing i), each with its start-of-step delta.
+ *      stats.moves counts logged moves, stats.passes scans and stats.evals generated legal moves, as in Or-opt N.
+ *   6. max_moves >= 0: as in Mode NM, a step applies the first max_moves - moves of its moves in log order and the
+ *      search stops with converged = 0; a later tl_session_run starts a new step with a fresh scan.
+ * With n <= B/2 every move that does not wrap is in-block at both offsets, so the moves are Or-opt N's (and, with
+ * k >= n-1, TL_ALGO_OR_OPT's).  tl_session_scan and tl_session_time_scans scan for G as Or-opt N does.  Or-opt NM
+ * needs B <= 16384: the TL_MULTI_BLOCK environment variable, which also sets its block size, must then be a power of
+ * two in 2..16384 (TL_ERR_INVALID otherwise).
  *
  * 1 <= k <= 32 (TL_ERR_INVALID otherwise); EXPLICIT problems: TL_ERR_UNSUPPORTED.  A session copies
  * the lists when it is created, so later calls do not affect it.  Without a call, the first session

@@ -110,6 +110,19 @@ def or_opt_nl(p: O.Problem, tour, cand, max_moves: int = -1, nthreads: int = 1, 
     return t, st, [log[m].astuple() for m in range(min(st.moves, log_cap))]
 
 
+def or_opt_nl_multi(p: O.Problem, tour, cand, block: int, step0: int = 0, max_moves: int = -1, nthreads: int = 1,
+                    log_cap: int = 0):
+    """Or-opt NM (multi-move Or-opt N) with blocks of `block` positions, first step numbered step0, to its local
+    optimum (or max_moves).  Returns (tour, stats, moves, converged); moves as or_opt_nl's."""
+    assert block >= 2 and block & (block - 1) == 0, "block must be a power of two >= 2"
+    t = np.ascontiguousarray(tour, dtype=np.int32).copy()
+    c = _cand(cand)
+    st, log = O.Stats(), (O.Move * max(log_cap, 1))()
+    conv = lib().tlo_or_opt_nl_multi(p.ref, _p(t), _p(c), C.c_int32(c.shape[1]), C.c_int32(block), C.c_int64(step0),
+                                     C.c_int64(max_moves), C.c_int(nthreads), C.byref(st), log, C.c_int64(log_cap))
+    return t, st, [log[m].astuple() for m in range(min(st.moves, log_cap))], int(conv)
+
+
 def three_opt_nl_eval(p: O.Problem, tour, i: int, j: int, k: int):
     """The evaluation of the triple i < j < k on tour: (delta = -savings, case), or None when no case improves."""
     t = np.ascontiguousarray(tour, dtype=np.int32)

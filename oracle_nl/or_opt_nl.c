@@ -6,6 +6,12 @@
 #include <stdlib.h>
 #include <string.h>
 
+/* Or-opt NM's per-block best: found = 0 for a block without an in-block move below the threshold */
+typedef struct {
+    int found;
+    tlo_move mv;
+} or_block;
+
 typedef struct {
     const tlo_problem *p;
     const int32_t *tour, *pos, *cand;
@@ -13,6 +19,9 @@ typedef struct {
     int found;
     tlo_move mv;
     int64_t evals;
+    /* Or-opt NM only (blk non-null): position q lies in block (q + off) / block */
+    int32_t block, off;
+    or_block *blk;
 } or_job;
 
 /* (delta, seg_len, i, j, reversed) lexicographic */
@@ -47,6 +56,19 @@ static double delta_of(const tlo_problem *p, const int32_t *t, int32_t i, int32_
 #undef DF
 }
 
+/* the hull [a0, a1] of a move that does not wrap: every position its delta reads or its relocation writes */
+static void hull(const tlo_move *m, int32_t *a0, int32_t *a1)
+{
+    *a0 = m->i - 1 < m->j ? m->i - 1 : m->j;
+    *a1 = m->i + m->seg_len > m->j + 1 ? m->i + m->seg_len : m->j + 1;
+}
+
+/* the move touches the closing edge (p_n-1, p_0) */
+static int wraps(const tlo_move *m, int32_t n)
+{
+    return m->i == 0 || m->i + m->seg_len == n || m->j == n - 1;
+}
+
 static void consider(or_job *jb, int32_t i, int32_t s, int32_t j, int rev)
 {
     const int32_t n = jb->p->n;
@@ -62,9 +84,20 @@ static void consider(or_job *jb, int32_t i, int32_t s, int32_t j, int rev)
     o.seg_len = s;
     o.reversed = rev;
     const double thr = jb->p->kind == TLO_PACKED_I32 ? 0.0 : (double)(-1e-3f); /* or_opt.rs:86 */
-    if (o.delta < thr && (!jb->found || better(&o, &jb->mv))) {
+    if (!(o.delta < thr)) return;
+    if (!jb->found || better(&o, &jb->mv)) {
         jb->found = 1;
         jb->mv = o;
+    }
+    if (jb->blk && !wraps(&o, n)) {
+        int32_t a0, a1;
+        hull(&o, &a0, &a1);
+        const int32_t b = (a0 + jb->off) / jb->block;
+        or_block *B = &jb->blk[b];
+        if (b == (a1 + jb->off) / jb->block && (!B->found || better(&o, &B->mv))) { /* in-block move */
+            B->found = 1;
+            B->mv = o;
+        }
     }
 }
 
@@ -90,8 +123,10 @@ static void *or_worker(void *arg)
     return NULL;
 }
 
+/* blk (nullable, nblk entries): Or-opt NM's per-block bests for blocks of `block` positions shifted by off */
 static int scan_with_pos(const tlo_problem *p, const int32_t *tour, const int32_t *pos, const int32_t *cand,
-                         int32_t k, int nthreads, tlo_move *mv, int64_t *evals)
+                         int32_t k, int nthreads, tlo_move *mv, int64_t *evals, int32_t block, int32_t off,
+                         or_block *blk, int32_t nblk)
 {
     const int32_t n = p->n;
     if (nthreads < 1) nthreads = 1;
@@ -104,6 +139,9 @@ static int scan_with_pos(const tlo_problem *p, const int32_t *tour, const int32_
         jobs[t].p = p; jobs[t].tour = tour; jobs[t].pos = pos; jobs[t].cand = cand; jobs[t].k = k;
         jobs[t].q0 = (int32_t)((int64_t)n * t / nthreads);
         jobs[t].q1 = (int32_t)((int64_t)n * (t + 1) / nthreads);
+        jobs[t].block = block;
+        jobs[t].off = off;
+        jobs[t].blk = blk ? (or_block *)calloc((size_t)nblk, sizeof(or_block)) : NULL;
         if (nthreads > 1)
             pthread_create(&th[t], NULL, or_worker, &jobs[t]);
         else
@@ -118,6 +156,13 @@ static int scan_with_pos(const tlo_problem *p, const int32_t *tour, const int32_
             *mv = jobs[t].mv;
             found = 1;
         }
+        if (blk) { /* (delta, s, i, j, reversed) is a total order: the merge does not depend on the thread split */
+            for (int32_t b = 0; b < nblk; ++b) {
+                const or_block *J = &jobs[t].blk[b];
+                if (J->found && (!blk[b].found || better(&J->mv, &blk[b].mv))) blk[b] = *J;
+            }
+            free(jobs[t].blk);
+        }
     }
     if (evals) *evals = ev;
     return found;
@@ -128,7 +173,7 @@ int tlo_or_opt_nl_scan(const tlo_problem *p, const int32_t *tour, const int32_t 
 {
     int32_t *pos = (int32_t *)malloc((size_t)(p->n > 0 ? p->n : 1) * 4);
     for (int32_t q = 0; q < p->n; ++q) pos[tour[q]] = q;
-    const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, mv, evals);
+    const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, mv, evals, 0, 0, NULL, 0);
     free(pos);
     return found;
 }
@@ -144,7 +189,7 @@ void tlo_or_opt_nl(const tlo_problem *p, int32_t *tour, const int32_t *cand, int
         if (max_moves >= 0 && st->moves >= max_moves) break;
         tlo_move mv;
         int64_t ev = 0;
-        const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, &mv, &ev);
+        const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, &mv, &ev, 0, 0, NULL, 0);
         st->passes++;
         st->evals += ev;
         if (!found) break;
@@ -157,4 +202,58 @@ void tlo_or_opt_nl(const tlo_problem *p, int32_t *tour, const int32_t *cand, int
         st->moves++;
     }
     free(pos);
+}
+
+static void apply_logged(int32_t *tour, int32_t *pos, int32_t n, const tlo_move *mv, tlo_stats *st, tlo_move *log,
+                         int64_t log_cap)
+{
+    tlo_or_opt_apply(tour, n, mv->i, mv->seg_len, mv->j, mv->reversed);
+    const int32_t lo = mv->j >= mv->i + mv->seg_len ? mv->i : mv->j + 1;
+    const int32_t hi = mv->j >= mv->i + mv->seg_len ? mv->j : mv->i + mv->seg_len - 1;
+    for (int32_t q = lo; q <= hi; ++q) pos[tour[q]] = q;
+    if (log && st->moves < log_cap) log[st->moves] = *mv;
+    st->moves++;
+}
+
+int tlo_or_opt_nl_multi(const tlo_problem *p, int32_t *tour, const int32_t *cand, int32_t k, int32_t block,
+                        int64_t step0, int64_t max_moves, int nthreads, tlo_stats *st, tlo_move *log, int64_t log_cap)
+{
+    st->passes = st->moves = st->evals = 0;
+    const int32_t n = p->n;
+    if (n < 4) return 1; /* as tlo_or_opt_nl: no scan */
+    const int32_t nblk = (n + block - 1) / block + 1;
+    int32_t *pos = (int32_t *)malloc((size_t)n * 4);
+    or_block *blk = (or_block *)malloc((size_t)nblk * sizeof(or_block));
+    for (int32_t q = 0; q < n; ++q) pos[tour[q]] = q;
+    int converged = 0;
+    for (int64_t t = step0;; ++t) {
+        if (max_moves >= 0 && st->moves >= max_moves) break;
+        const int32_t off = (int32_t)(t & 1) * (block / 2);
+        memset(blk, 0, (size_t)nblk * sizeof(or_block));
+        tlo_move g;
+        int64_t ev = 0;
+        const int found = scan_with_pos(p, tour, pos, cand, k, nthreads, &g, &ev, block, off, blk, nblk);
+        st->passes++;
+        st->evals += ev;
+        if (!found) { converged = 1; break; }
+        /* G alone when it wraps; otherwise every block best whose hull lies on either side of G's, in block order.
+           All of them are read before anything is applied, so the whole step works on the start-of-step tour. */
+        int32_t na = 0;
+        if (!wraps(&g, n)) {
+            int32_t g0, g1;
+            hull(&g, &g0, &g1);
+            for (int32_t b = 0; b < nblk; ++b) {
+                if (!blk[b].found) continue;
+                int32_t a0, a1;
+                hull(&blk[b].mv, &a0, &a1);
+                if (a1 <= g0 || a0 >= g1) blk[na++].mv = blk[b].mv;
+            }
+        }
+        apply_logged(tour, pos, n, &g, st, log, log_cap);
+        for (int32_t a = 0; a < na && !(max_moves >= 0 && st->moves >= max_moves); ++a)
+            apply_logged(tour, pos, n, &blk[a].mv, st, log, log_cap);
+    }
+    free(blk);
+    free(pos);
+    return converged;
 }

@@ -14,9 +14,9 @@ import weakref
 import numpy as np
 
 from . import _capi as capi
-from ._capi import (ALGO_OR_OPT, ALGO_OR_OPT_NEIGHBOR, ALGO_THREE_OPT, ALGO_TWO_OPT_BEST, ALGO_TWO_OPT_BEST_CACHED, ALGO_TWO_OPT_BEST_CYCLIC,
+from ._capi import (ALGO_OR_OPT, ALGO_OR_OPT_NEIGHBOR, ALGO_OR_OPT_NEIGHBOR_MULTI, ALGO_THREE_OPT, ALGO_TWO_OPT_BEST, ALGO_TWO_OPT_BEST_CACHED, ALGO_TWO_OPT_BEST_CYCLIC,
                     ALGO_THREE_OPT_NEIGHBOR, ALGO_TWO_OPT_NEIGHBOR, ALGO_TWO_OPT_NEIGHBOR_MULTI, ALGO_TWO_OPT_REF,
-                    CANDIDATES_DEFAULT, MULTI_BLOCK,
+                    CANDIDATES_DEFAULT, MULTI_BLOCK, OR_MULTI_BLOCK,
                     DIST_F32_EXACT, DIST_NINT_I32, LEN_EXACT, LEN_FAST, PATH_AUTO, PATH_MATRIX,
                     PATH_RECOMPUTE, Move, Stats, TeelineError)
 
@@ -130,7 +130,7 @@ class Problem:
 
     def set_candidates(self, k: int = CANDIDATES_DEFAULT):
         """tl_problem_set_candidates: the k-nearest candidate lists that later ALGO_TWO_OPT_NEIGHBOR[_MULTI],
-        ALGO_OR_OPT_NEIGHBOR and ALGO_THREE_OPT_NEIGHBOR sessions of this problem search (1 <= k <= 32)."""
+        ALGO_OR_OPT_NEIGHBOR[_MULTI] and ALGO_THREE_OPT_NEIGHBOR sessions of this problem search (1 <= k <= 32)."""
         capi.check(self._lib.tl_problem_set_candidates(self.h, k))
 
     def nn_tour(self, k: int = 3) -> np.ndarray:

@@ -24,7 +24,9 @@ ALGO_TWO_OPT_NEIGHBOR = 6
 ALGO_OR_OPT_NEIGHBOR = 7
 ALGO_THREE_OPT_NEIGHBOR = 8
 ALGO_TWO_OPT_NEIGHBOR_MULTI = 9
+ALGO_OR_OPT_NEIGHBOR_MULTI = 10
 MULTI_BLOCK = 4096
+OR_MULTI_BLOCK = 16384
 CANDIDATES_DEFAULT = 8
 PATH_AUTO, PATH_MATRIX, PATH_RECOMPUTE = 0, 1, 2
 LEN_EXACT, LEN_FAST = 0, 1

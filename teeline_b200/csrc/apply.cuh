@@ -292,23 +292,16 @@ __device__ __forceinline__ void relocate_scatter(const Pol &P, const typename Po
     }
 }
 
-// Tail of a fused candidate-list relocation step (Or-opt N, 3-opt N), run by the scan's last CTA of
-// WARPS warps: reduce the per-CTA records blockbest[0 .. grid) in Move's order, add the per-CTA counts of
-// evaluated candidates to state->computed, then either relocate a span of at most kOrNlCtaSpan positions
-// here through tmp and finish the step, or leave a longer one pending in blockbest[grid] for the apply
-// grids (relocate_gather_kernel / relocate_scatter_kernel with pending_only).
-template <int WARPS, class Move, class Pol>
-__device__ __noinline__ void relocate_step_tail(const Pol &P, uint32_t n, uint32_t *pos, typename Pol::Rec *tmp,
-                                                Best<typename Pol::V> *blockbest, const unsigned long long *blockcnt,
-                                                DevState *state, unsigned int *ticket, tl_move *__restrict__ log,
-                                                uint64_t log_cap)
+// The records reduction of a fused candidate-list relocation step's tail, run by the scan's last CTA of WARPS
+// warps: every thread gets the best of blockbest[0 .. grid) in Move's order and the sum of the per-CTA counts of
+// evaluated candidates (cnt_out).  Contains a barrier, which also publishes the caller's earlier shared writes.
+template <int WARPS, class Move, typename V>
+__device__ __forceinline__ Best<V> reduce_step_records(const Best<V> *blockbest, const unsigned long long *blockcnt,
+                                                       unsigned long long &cnt_out)
 {
-    using V = typename Pol::V;
     __shared__ Best<V> red[WARPS];
     __shared__ unsigned long long red_cnt[WARPS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    StateHeader hdr{};
-    if (threadIdx.x == 0) hdr = load_state_header(state);
     Best<V> v{(V)0, 0xffffffffu, 0xffffffffu, 0u};
     unsigned long long cnt = 0;
     for (int c = threadIdx.x; c < (int)gridDim.x; c += blockDim.x) {
@@ -325,6 +318,26 @@ __device__ __noinline__ void relocate_step_tail(const Pol &P, uint32_t n, uint32
     cnt = 0;
 #pragma unroll
     for (int w = 0; w < WARPS; ++w) cnt += red_cnt[w];
+    cnt_out = cnt;
+    return v;
+}
+
+// Tail of a fused candidate-list relocation step (Or-opt N, 3-opt N), run by the scan's last CTA of
+// WARPS warps: reduce the per-CTA records blockbest[0 .. grid) in Move's order, add the per-CTA counts of
+// evaluated candidates to state->computed, then either relocate a span of at most kOrNlCtaSpan positions
+// here through tmp and finish the step, or leave a longer one pending in blockbest[grid] for the apply
+// grids (relocate_gather_kernel / relocate_scatter_kernel with pending_only).
+template <int WARPS, class Move, class Pol>
+__device__ __noinline__ void relocate_step_tail(const Pol &P, uint32_t n, uint32_t *pos, typename Pol::Rec *tmp,
+                                                Best<typename Pol::V> *blockbest, const unsigned long long *blockcnt,
+                                                DevState *state, unsigned int *ticket, tl_move *__restrict__ log,
+                                                uint64_t log_cap)
+{
+    using V = typename Pol::V;
+    StateHeader hdr{};
+    if (threadIdx.x == 0) hdr = load_state_header(state);
+    unsigned long long cnt;
+    const Best<V> v = reduce_step_records<WARPS, Move>(blockbest, blockcnt, cnt);
     const Move m = Move::of(v);
     const bool long_span = m.found && m.hi - m.lo + 1 > (uint32_t)kOrNlCtaSpan;
     if (threadIdx.x == 0) {

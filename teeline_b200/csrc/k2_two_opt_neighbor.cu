@@ -30,6 +30,7 @@
 // block move and G share at most an end position, whose entering-edge length one of them rewrites and the
 // other never reads (reverse_segment_inplace reads only the coordinates of the records at i and j+1).
 #include "apply.cuh"
+#include "block_keys.cuh"
 #include "kernels.cuh"
 
 #include <math_constants.h>
@@ -40,23 +41,6 @@ namespace {
 
 constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
-
-// Mode NM's block keys: 32 bits ordered as the delta (negative deltas only; no NaN)
-__device__ __forceinline__ uint32_t order_bits(float d)
-{
-    const uint32_t u = __float_as_uint(d);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ uint32_t order_bits(int32_t d) { return (uint32_t)d ^ 0x80000000u; }
-template <typename V>
-__device__ __forceinline__ V from_order_bits(uint32_t k);
-template <>
-__device__ __forceinline__ float from_order_bits<float>(uint32_t k)
-{
-    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
-}
-template <>
-__device__ __forceinline__ int32_t from_order_bits<int32_t>(uint32_t k) { return (int32_t)(k ^ 0x80000000u); }
 
 // an improving pair (i, j): offer it to its block when i and j+1 lie in the same block
 template <typename V>
@@ -152,40 +136,25 @@ __device__ __noinline__ void nlm_tail(const Pol &P, uint32_t *pos, Best<typename
     // without G no pair improves, so no key was set
     uint32_t taken = 0;
     if (found) {
-        for (uint32_t c0 = 0; c0 < M.nslots; c0 += THREADS) {
-            const uint32_t b = c0 + threadIdx.x;
-            bool acc = false;
-            uint32_t mi = 0, mj = 0;
-            V d = (V)0;
-            if (b < M.nslots) {
-                const unsigned long long key = __ldcg(M.keys + b);
-                if (key != ~0ull) {
-                    M.keys[b] = ~0ull; // re-armed for the next step
-                    const uint32_t low = (uint32_t)key, base = (b << M.bshift) - off;
-                    mi = base + (low >> M.bshift);
-                    mj = base + (low & ((1u << M.bshift) - 1u));
-                    d = from_order_bits<V>((uint32_t)(key >> 32));
-                    acc = !(mi == v.i && mj == v.j) && (mj < v.i || mi > v.j);
-                }
-            }
-            const uint32_t bal = __ballot_sync(0xffffffffu, acc);
-            if (lane == 0) s_wcnt[warp] = __popc(bal);
-            __syncthreads();
-            uint32_t before = 0, total = 0;
-#pragma unroll
-            for (int w = 0; w < WARPS; ++w) {
-                before += w < warp ? s_wcnt[w] : 0u;
-                total += s_wcnt[w];
-            }
-            const uint32_t rank = taken + before + __popc(bal & ((1u << lane) - 1u));
-            if (acc && rank < allow) {
-                M.list[rank] = make_uint2(mi, mj);
+        uint2 *list = static_cast<uint2 *>(M.list);
+        struct Mv {
+            uint32_t i, j;
+            V d;
+        };
+        taken = compact_block_keys<WARPS, Mv>(
+            M, allow, s_wcnt,
+            [&](uint32_t b, unsigned long long key, Mv &mv) {
+                const uint32_t low = (uint32_t)key, base = (b << M.bshift) - off;
+                mv.i = base + (low >> M.bshift);
+                mv.j = base + (low & ((1u << M.bshift) - 1u));
+                mv.d = from_order_bits<V>((uint32_t)(key >> 32));
+                return !(mv.i == v.i && mv.j == v.j) && (mv.j < v.i || mv.i > v.j);
+            },
+            [&](uint32_t rank, const Mv &mv) {
+                list[rank] = make_uint2(mv.i, mv.j);
                 const unsigned long long e = m + 1 + rank;
-                if (log && e < log_cap) log[e] = tl_move{(float)d, mi, mj, 0, 0, 0};
-            }
-            taken += total;
-            __syncthreads(); // s_wcnt is rewritten by the next round
-        }
+                if (log && e < log_cap) log[e] = tl_move{(float)mv.d, mv.i, mv.j, 0, 0, 0};
+            });
     }
     const uint32_t napply = (uint32_t)min((unsigned long long)taken, allow);
     const bool long_seg = found && (v.j - v.i) / 2 > (uint32_t)kNlCtaSwaps;
@@ -385,7 +354,8 @@ void launch_nlm_apply(Metric metric, Pt *pts, uint32_t *pos, const NlMulti &mult
     const cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
-        cudaLaunchKernelEx(&cfg, apply_multi_kernel<Pol>, Pol{pts}, pos, (const uint2 *)multi.list, multi.desc, ticket);
+        cudaLaunchKernelEx(&cfg, apply_multi_kernel<Pol>, Pol{pts}, pos, static_cast<const uint2 *>(multi.list), multi.desc,
+                           ticket);
     });
 }
 

@@ -34,7 +34,22 @@
 // barrier, scatter); a longer one is left pending for the gather and scatter grids that every step
 // launches, which leave at once when nothing is pending.  The grid size cannot depend on the move: the
 // host queues steps without reading back.
+//
+// Or-opt NM (multi-move, TL_ALGO_OR_OPT_NEIGHBOR_MULTI; definition in include/teeline_cuda.h): the same scan and
+// G.  A move's hull is [a0, a1] = [min(i-1, j), max(i+s, j+1)]: every position its delta reads, and its relocated
+// span is [a0+1, a1-1] with a1's entering edge rewritten.  In step t (= DevState::scans) position q lies in block
+// (q + o) >> bshift with o = (t & 1) << (bshift - 1); every move below the threshold that does not wrap (i = 0,
+// i+s = n or j = n-1 touch the closing edge) and whose a0 and a1 share a block does a 64-bit atomicMin into that
+// block's key: the order-preserving delta bits above (s-1, i - base, j - base, rev), which orders a block's moves
+// as better_or does (bshift <= 14 keeps the fields in 31 bits).  The last CTA reduces G, re-arms the keys while it
+// compacts the block bests whose hull lies on either side of G's (none when G wraps) into a list in block order,
+// cuts the list at the move budget, writes the log and ends the step.  It relocates a short G itself; the apply
+// grids relocate a long G cooperatively and each listed block move with one CTA.  Every move is staged in tmp at
+// its own positions, so the disjoint spans share the buffer.  A block move and G share at most a hull end, whose
+// city neither moves and whose entering edge only one of them rewrites (the other reads that record's
+// coordinates only).
 #include "apply.cuh"
+#include "block_keys.cuh"
 #include "kernels.cuh"
 #include "or_opt_rank.cuh"
 
@@ -46,11 +61,102 @@ constexpr int THREADS = kNlThreads;
 constexpr int WARPS = THREADS / 32;
 constexpr uint32_t kNone = 0xffffffffu;
 
+// a legal move below the threshold: offer it to its block when it does not wrap and its hull lies in one block
+template <typename V>
+__device__ __forceinline__ void block_offer(const NlMulti &M, uint32_t off, uint32_t n, V d, uint32_t i, uint32_t j,
+                                            uint32_t s, uint32_t rev)
+{
+    if (i == 0 || i + s == n || j == n - 1) return;
+    const uint32_t a0 = min(i - 1, j), a1 = max(i + s, j + 1);
+    const uint32_t b = (a0 + off) >> M.bshift;
+    if (b != (a1 + off) >> M.bshift) return;
+    const uint32_t base = (b << M.bshift) - off; // wraps for block 0 at odd steps; the differences below do not
+    const uint32_t low =
+        ((s - 1) << (2 * M.bshift + 1)) | ((i - base) << (M.bshift + 1)) | ((j - base) << 1) | rev;
+    atomicMin(M.keys + b, ((unsigned long long)order_bits(d) << 32) | low);
+}
+
+// Tail of a fused Or-opt NM step, run by the last CTA: G as relocate_step_tail reduces it, then the accepted
+// block bests (see the file comment).
 template <class Pol>
+__device__ __noinline__ void or_nlm_tail(const Pol &P, uint32_t n, uint32_t *pos, Pt *tmp,
+                                         Best<typename Pol::V> *blockbest, const unsigned long long *blockcnt,
+                                         DevState *state, unsigned int *ticket, tl_move *__restrict__ log,
+                                         uint64_t log_cap, const NlMulti &M, uint32_t off)
+{
+    using V = typename Pol::V;
+    __shared__ unsigned long long s_moves;
+    __shared__ long long s_max;
+    __shared__ uint32_t s_wcnt[WARPS];
+    StateHeader hdr{};
+    if (threadIdx.x == 0) {
+        hdr = load_state_header(state);
+        s_moves = hdr.h0.x;
+        s_max = hdr.h1.x;
+    }
+    unsigned long long cnt;
+    const Best<V> v = reduce_step_records<WARPS, OrMove>(blockbest, blockcnt, cnt); // publishes s_moves, s_max
+    const OrMove g = OrMove::of(v);
+    const unsigned long long m = s_moves;
+    // block moves this step may still apply after G (G always fits: the step runs only below the budget)
+    const unsigned long long allow = s_max < 0 ? ~0ull : (unsigned long long)s_max - m - 1;
+    const bool wraps = g.i == 0 || g.i + g.s == n || g.j == n - 1; // G alone
+    const uint32_t g0 = min(g.i - 1, g.j), g1 = max(g.i + g.s, g.j + 1);
+    // without G no move is below the threshold, so no key was set
+    uint32_t taken = 0;
+    if (g.found) {
+        Best<V> *list = static_cast<Best<V> *>(M.list);
+        const uint32_t mask = (1u << M.bshift) - 1u;
+        taken = compact_block_keys<WARPS, Best<V>>(
+            M, allow, s_wcnt,
+            [&](uint32_t b, unsigned long long key, Best<V> &mv) {
+                const uint32_t low = (uint32_t)key, base = (b << M.bshift) - off;
+                mv.delta = from_order_bits<V>((uint32_t)(key >> 32));
+                mv.i = base + ((low >> (M.bshift + 1)) & mask);
+                mv.j = base + ((low >> 1) & mask);
+                mv.aux = ((low >> (2 * M.bshift + 1)) << 1) | (low & 1u); // (s-1)*2 + rev
+                const uint32_t a0 = min(mv.i - 1, mv.j), a1 = max(mv.i + (mv.aux >> 1) + 1, mv.j + 1);
+                return !wraps && (a1 <= g0 || a0 >= g1);
+            },
+            [&](uint32_t rank, const Best<V> &mv) {
+                list[rank] = mv;
+                const unsigned long long e = m + 1 + rank;
+                if (log && e < log_cap) log[e] = OrMove::of(mv).entry();
+            });
+    }
+    const uint32_t napply = (uint32_t)min((unsigned long long)taken, allow);
+    const bool long_span = g.found && g.hi - g.lo + 1 > (uint32_t)kOrNlCtaSpan;
+    if (threadIdx.x == 0) {
+        state->computed += cnt;
+        M.desc[0] = napply;
+        M.desc[1] = long_span ? v.i : kNone;
+        M.desc[2] = v.j;
+        M.desc[3] = v.aux;
+        *ticket = 0u;
+        state->scans = hdr.h0.y + 1;
+        if (g.found) {
+            if (log && m < log_cap) log[m] = g.entry();
+            const unsigned long long moves = m + 1 + napply;
+            state->moves = moves;
+            if (s_max >= 0 && (long long)moves >= s_max) state->done = 1;
+        } else {
+            state->done = 1;
+            state->converged = 1;
+        }
+    }
+    if (g.found && !long_span) {
+        relocate_gather(P, tmp + g.lo, g, threadIdx.x, blockDim.x);
+        __syncthreads();
+        relocate_scatter(P, tmp + g.lo, n, g, pos, threadIdx.x, blockDim.x);
+    }
+}
+
+// MULTI: Or-opt NM's fused step (block keys and or_nlm_tail); otherwise Or-opt N's scan
+template <bool MULTI, class Pol>
 __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     or_nl_scan_kernel(Pol P, uint32_t *__restrict__ pos, const uint32_t *__restrict__ cand, uint32_t k, uint32_t n,
                       Pt *tmp, Best<typename Pol::V> *blockbest, unsigned long long *blockcnt, DevState *state,
-                      unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap, int fuse_apply)
+                      unsigned int *ticket, tl_move *__restrict__ log, uint64_t log_cap, int fuse_apply, NlMulti M)
 {
     using V = typename Pol::V;
     using Rec = typename Pol::Rec;
@@ -58,6 +164,9 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     griddep_wait(); // the previous step's move is applied and visible from here on
     // uniform across the grid: only a step's tail or apply grid writes it, after every CTA has finished
     if (*reinterpret_cast<const volatile int *>(&state->done)) return;
+    // Or-opt NM: this step's block offset (scans is only written by a step's tail, after every CTA has read it)
+    uint32_t off = 0;
+    if (MULTI) off = ((uint32_t)*reinterpret_cast<const volatile unsigned long long *>(&state->scans) & 1u) << (M.bshift - 1);
 
     Best<V> best{(V)0, kNone, kNone, 0u};
     uint32_t cnt = 0;
@@ -68,6 +177,7 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
         if (!legal) return;
         ++cnt;
         const Best<V> o{d, i, j, (s - 1) * 2 + rev};
+        if (MULTI && d < thr) block_offer(M, off, n, d, i, j, s, rev);
         if (d < thr && better_or(o, best)) best = o;
     };
     // j is a legal insertion edge of the segment [i, i+s-1] (the caller checks n > s+1, 0 <= i, i+s <= n)
@@ -149,23 +259,95 @@ __global__ void __launch_bounds__(THREADS, kNlMinBlocks)
     if (threadIdx.x == 0) s_last = (ticket_take_acq_rel(ticket) == gridDim.x - 1) ? 1u : 0u; // thread 0 wrote blockbest
     __syncthreads();
     if (!s_last) return;
-    relocate_step_tail<WARPS, OrMove>(P, n, pos, tmp, blockbest, blockcnt, state, ticket, log, log_cap);
+    if (MULTI)
+        or_nlm_tail(P, n, pos, tmp, blockbest, blockcnt, state, ticket, log, log_cap, M, off);
+    else
+        relocate_step_tail<WARPS, OrMove>(P, n, pos, tmp, blockbest, blockcnt, state, ticket, log, log_cap);
+}
+
+// Or-opt NM's apply grids, launched after every step's scan.  desc (written by or_nlm_tail) names a pending long G
+// and the count of listed block moves.  The gather grid stages G cooperatively and relocates each block move with
+// one CTA (gather, barrier, scatter); G's positions are disjoint from every block move's, so the two run together.
+// The scatter grid then writes G back, and its last CTA resets desc, so a later no-op step applies nothing.
+template <class Pol>
+__device__ __forceinline__ OrMove pending_g(const uint32_t *desc, uint32_t gi)
+{
+    return OrMove::of(Best<typename Pol::V>{(typename Pol::V)0, gi, __ldcg(desc + 2), __ldcg(desc + 3)});
+}
+
+template <class Pol>
+__global__ void __launch_bounds__(256)
+    or_nlm_gather_kernel(Pol P, Pt *tmp, uint32_t n, const Best<typename Pol::V> *__restrict__ list,
+                         const uint32_t *desc, uint32_t *pos)
+{
+    griddep_wait(); // PDL: the step's scan has finished and its writes are visible
+    const uint32_t cnt = __ldcg(desc), gi = __ldcg(desc + 1);
+    if (cnt == 0 && gi == kNone) return; // uniform over the grid
+    if (gi != kNone) {
+        const OrMove g = pending_g<Pol>(desc, gi);
+        relocate_gather(P, tmp + g.lo, g, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
+    }
+    for (uint32_t c = blockIdx.x; c < cnt; c += gridDim.x) {
+        const OrMove m = OrMove::of(list[c]);
+        relocate_gather(P, tmp + m.lo, m, threadIdx.x, blockDim.x);
+        __syncthreads();
+        relocate_scatter(P, tmp + m.lo, n, m, pos, threadIdx.x, blockDim.x);
+    }
+}
+
+template <class Pol>
+__global__ void __launch_bounds__(256)
+    or_nlm_scatter_kernel(Pol P, const Pt *tmp, uint32_t n, uint32_t *desc, unsigned int *ticket, uint32_t *pos)
+{
+    griddep_wait(); // PDL: the gather grid has finished
+    const uint32_t cnt = __ldcg(desc), gi = __ldcg(desc + 1);
+    if (cnt == 0 && gi == kNone) return; // uniform over the grid
+    if (gi != kNone) {
+        const OrMove g = pending_g<Pol>(desc, gi);
+        relocate_scatter(P, tmp + g.lo, n, g, pos, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && atomicAdd(ticket, 1u) == gridDim.x - 1) { // every CTA has read desc
+        *ticket = 0u;
+        desc[0] = 0u;
+        desc[1] = kNone;
+    }
 }
 
 } // namespace
 
 void launch_or_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *tmp,
                        void *blockbest, unsigned long long *blockcnt, DevState *state, unsigned int *ticket, tl_move *log,
-                       uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st)
+                       uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st, const NlMulti *multi)
 {
     cudaLaunchAttribute attr[1];
     const cudaLaunchConfig_t cfg = pdl_config(grid, THREADS, 0, attr, st);
     const int fuse = fuse_apply ? 1 : 0;
+    const NlMulti mm = multi ? *multi : NlMulti{};
     with_metric(metric, [&](auto M) {
         using Pol = NlPol<M>;
-        cudaLaunchKernelEx(&cfg, or_nl_scan_kernel<Pol>, Pol{pts}, pos, cand, k, n, reinterpret_cast<Pt *>(tmp),
-                           reinterpret_cast<Best<typename Pol::V> *>(blockbest), blockcnt, state, ticket, log,
-                           (uint64_t)log_cap, fuse);
+        auto *bb = reinterpret_cast<Best<typename Pol::V> *>(blockbest);
+        auto *t = reinterpret_cast<Pt *>(tmp);
+        if (multi && fuse_apply) // a scan without its step (tl_session_scan) leaves the block keys alone
+            cudaLaunchKernelEx(&cfg, or_nl_scan_kernel<true, Pol>, Pol{pts}, pos, cand, k, n, t, bb, blockcnt, state,
+                               ticket, log, (uint64_t)log_cap, fuse, mm);
+        else
+            cudaLaunchKernelEx(&cfg, or_nl_scan_kernel<false, Pol>, Pol{pts}, pos, cand, k, n, t, bb, blockcnt, state,
+                               ticket, log, (uint64_t)log_cap, fuse, mm);
+    });
+}
+
+void launch_or_nlm_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32_t n, const NlMulti &multi,
+                         unsigned int *ticket, int grid, cudaStream_t st)
+{
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = pdl_config(grid, 256, 0, attr, st);
+    with_metric(metric, [&](auto M) {
+        using Pol = NlPol<M>;
+        auto *t = reinterpret_cast<Pt *>(tmp);
+        cudaLaunchKernelEx(&cfg, or_nlm_gather_kernel<Pol>, Pol{pts}, t, n,
+                           static_cast<const Best<typename Pol::V> *>(multi.list), (const uint32_t *)multi.desc, pos);
+        cudaLaunchKernelEx(&cfg, or_nlm_scatter_kernel<Pol>, Pol{pts}, (const Pt *)t, n, multi.desc, ticket, pos);
     });
 }
 

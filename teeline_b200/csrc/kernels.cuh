@@ -315,10 +315,13 @@ void launch_nl_init(Metric metric, const float2 *xy, const uint32_t *tour, uint3
 // 2^bshift positions (order-preserving delta bits << 32 | in-block offsets of i and j), re-armed to ~0 by
 // the step's last CTA.  That CTA lists the accepted block moves (i, j) in `list` and leaves
 // desc = {block moves to apply, pending long G's i, its j} (i = ~0: none) for the apply grid, which resets it.
+// Multi-move Or-opt N, "Or-opt NM" (k3_or_opt_neighbor.cu), keeps the same buffers: its keys hold (s, i, j, rev)
+// below the delta bits, `list` holds the accepted moves as Or-opt records (Best<V>) and
+// desc = {block moves to apply, pending long G's i, j, aux}.
 struct NlMulti {
     unsigned long long *keys; // nslots = ceil(n / 2^bshift) + 1
-    uint2 *list;              // nslots
-    uint32_t *desc;           // 3
+    void *list;               // nslots entries: uint2 (Mode NM) or 16-byte Or-opt records (Or-opt NM)
+    uint32_t *desc;           // 4
     uint32_t bshift, nslots;
 };
 // multi (nullable): a fused scan also keeps Mode NM's block bests and ends the step as Mode NM
@@ -335,11 +338,16 @@ void launch_nlm_apply(Metric metric, Pt *pts, uint32_t *pos, const NlMulti &mult
 // lists.  blockbest holds grid + 1 records as in Mode N, blockcnt the grid per-CTA candidate counts;
 // tmp stages the relocated span (npad records).
 constexpr int kOrNlCtaSpan = 4096; // relocated spans of up to this many positions are moved by the reducing CTA
+// multi (nullable): a fused scan also keeps Or-opt NM's block bests and ends the step as Or-opt NM
 void launch_or_nl_scan(Metric metric, Pt *pts, uint32_t *pos, const uint32_t *cand, uint32_t k, uint32_t n, void *tmp,
                        void *blockbest, unsigned long long *blockcnt, DevState *state, unsigned int *ticket, tl_move *log,
-                       uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st);
+                       uint64_t log_cap, bool fuse_apply, int grid, cudaStream_t st, const NlMulti *multi = nullptr);
 void launch_or_nl_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32_t n, const void *pending,
                         DevState *state, unsigned int *ticket, tl_move *log, uint64_t log_cap, int grid, cudaStream_t st);
+// Or-opt NM's apply grids (same file): a pending long G cooperatively and each listed block move by one CTA, every
+// move staged in tmp from its first relocated position on; the last CTA resets multi.desc
+void launch_or_nlm_apply(Metric metric, Pt *pts, uint32_t *pos, void *tmp, uint32_t n, const NlMulti &multi,
+                         unsigned int *ticket, int grid, cudaStream_t st);
 
 // K6 candidate-list 3-opt, "3-opt N" (k6_three_opt_neighbor.cu): Or-opt N's records, pos[], lists,
 // buffers and relocation routes; its records carry the savings, as K6's do.

@@ -85,9 +85,10 @@ struct tl_session {
     DevBuf<uint32_t> nl_cand;        // n x nl_k
     uint32_t nl_k = 0;
     DevBuf<unsigned long long> nl_cnt; // Or-opt N, 3-opt N: per-CTA counts of evaluated candidates
-    // Mode NM (TL_ALGO_TWO_OPT_NEIGHBOR_MULTI): per-block keys, the step's accepted block moves, apply descriptor
+    // Mode NM and Or-opt NM (TL_ALGO_TWO_OPT_NEIGHBOR_MULTI, TL_ALGO_OR_OPT_NEIGHBOR_MULTI): per-block keys, the
+    // step's accepted block moves, apply descriptor
     DevBuf<unsigned long long> nlm_keys;
-    DevBuf<uint2> nlm_list;
+    DevBuf<uint4> nlm_list;
     DevBuf<uint32_t> nlm_desc;
     NlMulti nlm{};
     int nlm_grid = 1; // the apply grid: fixed per session, since steps are queued without reading back
@@ -111,8 +112,12 @@ struct tl_session {
 
     bool matrix() const { return path_used == TL_PATH_MATRIX; }
     // the candidate-list searches that relocate a span of positions (cyclic records, staging buffer, counts)
-    bool nl_relocating() const { return algo == TL_ALGO_OR_OPT_NEIGHBOR || algo == TL_ALGO_THREE_OPT_NEIGHBOR; }
-    bool nl_multi() const { return algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI; }
+    bool nl_relocating() const
+    {
+        return algo == TL_ALGO_OR_OPT_NEIGHBOR || algo == TL_ALGO_THREE_OPT_NEIGHBOR || algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI;
+    }
+    // the multi-move candidate-list searches (block keys, list and descriptor)
+    bool nl_multi() const { return algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI || algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI; }
     bool int_values() const { return metric_is_int(p->metric); }
     // the metric the persistent Mode R kernel recomputes distances in; none when the session reads f32
     // matrix entries (f32 matrix and EXPLICIT sessions)
@@ -252,14 +257,14 @@ tl_status upload_geometry(tl_session *s)
             m.nslots = (uint32_t)((s->n + (1u << m.bshift) - 1) >> m.bshift) + 1;
             TL_CUDA_TRY(s->nlm_keys.alloc(m.nslots));
             TL_CUDA_TRY(s->nlm_list.alloc(m.nslots));
-            TL_CUDA_TRY(s->nlm_desc.alloc(3));
+            TL_CUDA_TRY(s->nlm_desc.alloc(4));
             TL_CUDA_TRY(cudaMemsetAsync(s->nlm_keys.p, 0xff, (size_t)m.nslots * 8, s->c->stream)); // no key
-            TL_CUDA_TRY(cudaMemsetAsync(s->nlm_desc.p, 0xff, 12, s->c->stream));
+            TL_CUDA_TRY(cudaMemsetAsync(s->nlm_desc.p, 0xff, 16, s->c->stream));
             TL_CUDA_TRY(cudaMemsetAsync(s->nlm_desc.p, 0, 4, s->c->stream)); // nothing to apply
             m.keys = s->nlm_keys.p;
             m.list = s->nlm_list.p;
             m.desc = s->nlm_desc.p;
-            // one CTA per block move (up to two per SM), at least Mode N's apply grid for a long G
+            // one CTA per block move (up to two per SM), at least Mode N's (Or-opt N's) apply grid for a long G
             const uint32_t half_pairs = (s->n / 2 + 255) / 256;
             s->nlm_grid = (int)std::max<uint32_t>(std::min<uint32_t>(half_pairs, (uint32_t)s->c->sm_count),
                                                   std::min<uint32_t>(m.nslots, 2u * (uint32_t)s->c->sm_count));
@@ -387,9 +392,10 @@ tl_status launch_scan(tl_session *s, bool fuse, bool exchange = true)
     const ShardComm *comm = (fused && s->shard_count > 1) ? &s->comm : nullptr;
     BestF *mine = s->cand.p + (size_t)s->shard_index * s->grid;
     cudaStream_t st = s->c->stream;
-    if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR) {
+    if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR || s->algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI) {
         launch_or_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->tmp.p, s->cand.p,
-                          s->nl_cnt.p, s->state.p, s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st);
+                          s->nl_cnt.p, s->state.p, s->ticket.p, s->log.p, s->log_cap, fuse, s->grid, st,
+                          s->nl_multi() ? &s->nlm : nullptr);
         s->c->launches++;
     } else if (s->algo == TL_ALGO_THREE_OPT_NEIGHBOR) {
         launch_three_nl_scan(s->p->metric, s->pts.p, s->pos.p, s->nl_cand.p, s->nl_k, s->n, s->tmp.p, s->cand.p,
@@ -485,6 +491,11 @@ tl_status enqueue_steps(tl_session *s, uint32_t steps)
         if (s->algo == TL_ALGO_THREE_OPT_NEIGHBOR) { // as Or-opt N
             launch_three_nl_apply(s->p->metric, s->pts.p, s->pos.p, s->tmp.p, s->n, s->cand.p + s->grid, s->state.p,
                                   s->ticket.p + 1, s->log.p, s->log_cap, apply_grid, st);
+            s->c->launches += 2;
+            continue;
+        }
+        if (s->algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI) { // as Mode NM, with Or-opt N's two apply grids
+            launch_or_nlm_apply(s->p->metric, s->pts.p, s->pos.p, s->tmp.p, s->n, s->nlm, s->ticket.p + 1, s->nlm_grid, st);
             s->c->launches += 2;
             continue;
         }
@@ -590,7 +601,8 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     if (cached) algo = TL_ALGO_TWO_OPT_BEST;
     if (algo != TL_ALGO_TWO_OPT_BEST && algo != TL_ALGO_TWO_OPT_BEST_CYCLIC && algo != TL_ALGO_TWO_OPT_REF &&
         algo != TL_ALGO_OR_OPT && algo != TL_ALGO_THREE_OPT && algo != TL_ALGO_TWO_OPT_NEIGHBOR &&
-        algo != TL_ALGO_OR_OPT_NEIGHBOR && algo != TL_ALGO_THREE_OPT_NEIGHBOR && algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI) {
+        algo != TL_ALGO_OR_OPT_NEIGHBOR && algo != TL_ALGO_THREE_OPT_NEIGHBOR && algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI &&
+        algo != TL_ALGO_OR_OPT_NEIGHBOR_MULTI) {
         set_error("tl_session_create: unknown algo %d", algo);
         return TL_ERR_INVALID;
     }
@@ -599,14 +611,17 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
         return TL_ERR_INVALID;
     }
     const bool nl = algo == TL_ALGO_TWO_OPT_NEIGHBOR || algo == TL_ALGO_OR_OPT_NEIGHBOR ||
-                    algo == TL_ALGO_THREE_OPT_NEIGHBOR || algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
-    // Mode NM's block size: TL_MULTI_BLOCK, or the TL_MULTI_BLOCK environment variable (a power of two in
-    // 2..65536) for measuring other sizes
-    uint32_t multi_block = TL_MULTI_BLOCK;
-    if (const char *ev = getenv("TL_MULTI_BLOCK"); ev && algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI) {
-        const long b = atol(ev);
-        if (b < 2 || b > 65536 || (b & (b - 1))) {
-            set_error("TL_MULTI_BLOCK=%s: must be a power of two in 2..65536", ev);
+                    algo == TL_ALGO_THREE_OPT_NEIGHBOR || algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI ||
+                    algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI;
+    // Mode NM's and Or-opt NM's block size: TL_MULTI_BLOCK / TL_OR_MULTI_BLOCK, or the TL_MULTI_BLOCK environment
+    // variable (a power of two in 2..65536, 2..16384 for Or-opt NM, whose keys hold s, i, j and rev in 31 bits) for
+    // measuring other sizes
+    uint32_t multi_block = algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI ? TL_OR_MULTI_BLOCK : TL_MULTI_BLOCK;
+    if (const char *ev = getenv("TL_MULTI_BLOCK");
+        ev && (algo == TL_ALGO_TWO_OPT_NEIGHBOR_MULTI || algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI)) {
+        const long b = atol(ev), bmax = algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI ? 16384 : 65536;
+        if (b < 2 || b > bmax || (b & (b - 1))) {
+            set_error("TL_MULTI_BLOCK=%s: must be a power of two in 2..%ld", ev, bmax);
             return TL_ERR_INVALID;
         }
         multi_block = (uint32_t)b;
@@ -742,7 +757,7 @@ tl_status tl_session_create(tl_problem *p, int32_t algo, int32_t path, const uin
     }
     // or_opt::solve and three_opt::solve ignore the seed and return identity order when n < 4
     // (or_opt.rs:31-34, three_opt.rs:25-28); so do Or-opt N and 3-opt N
-    // (Mode NM too: a new mode, defined with no scan for n < 4)
+    // (Mode NM and Or-opt NM too: new modes, defined with no scan for n < 4)
     const bool or_like = algo == TL_ALGO_OR_OPT || algo == TL_ALGO_THREE_OPT || s->nl_relocating() || s->nl_multi();
     std::vector<uint32_t> ident;
     if (or_like && s->trivial) {
@@ -931,7 +946,8 @@ tl_status tl_session_scan(tl_session *s, tl_move *best, int32_t *found)
     if (was_done) { s->h.done = was_done; rc = push_state(s); if (rc != TL_OK) return rc; }
     bool any;
     const bool three = s->algo == TL_ALGO_THREE_OPT || s->algo == TL_ALGO_THREE_OPT_NEIGHBOR;
-    const bool or_opt = s->algo == TL_ALGO_OR_OPT || s->algo == TL_ALGO_OR_OPT_NEIGHBOR;
+    const bool or_opt =
+        s->algo == TL_ALGO_OR_OPT || s->algo == TL_ALGO_OR_OPT_NEIGHBOR || s->algo == TL_ALGO_OR_OPT_NEIGHBOR_MULTI;
     if (s->int_values()) {
         std::vector<BestI> hi(hc.size());
         memcpy(hi.data(), hc.data(), hc.size() * sizeof(BestF));
@@ -1014,9 +1030,9 @@ tl_status tl_session_run(tl_session *s, int64_t max_moves)
     // past convergence (or past max_moves, which the device checks itself) are no-op launches.
     // with a move budget every step applies exactly one move (or finds none and stops), so the host
     // knows how many steps are still worth queueing without looking at the device
-    // (not so for Mode R, whose persistent kernel stops by itself, and Mode NM, whose steps apply several
-    // moves: both get unbudgeted batches and the device stops at the budget)
-    const bool budgeted = max_moves >= 0 && s->algo != TL_ALGO_TWO_OPT_REF && s->algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
+    // (not so for Mode R, whose persistent kernel stops by itself, and Mode NM and Or-opt NM, whose steps apply
+    // several moves: they get unbudgeted batches and the device stops at the budget)
+    const bool budgeted = max_moves >= 0 && s->algo != TL_ALGO_TWO_OPT_REF && !s->nl_multi();
     int64_t budget = budgeted ? max_moves - (int64_t)s->h.moves : 0;
     auto issue = [&](int slot) -> tl_status {
         uint32_t batch = s->algo == TL_ALGO_TWO_OPT_REF ? 64 : 32;

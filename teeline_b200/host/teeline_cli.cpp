@@ -73,7 +73,7 @@ Args parse_args(int argc, char **argv)
         else if (s == "--evaporation-rate") a.evaporation_rate = std::strtof(next("--evaporation-rate").c_str(), nullptr);
         else if (s == "--num-ants") a.num_ants = std::strtoull(next("--num-ants").c_str(), nullptr, 10);
         else if (s == "--seed") a.seed = std::strtoull(next("--seed").c_str(), nullptr, 10);
-        else if (s == "--mode") a.mode = next("--mode");  // extension: ref | best | best_cyclic | neighbor | neighbor_multi (or_opt, 3opt: neighbor)
+        else if (s == "--mode") a.mode = next("--mode");  // extension: ref | best | best_cyclic | neighbor | neighbor_multi (or_opt: neighbor | neighbor_multi, 3opt: neighbor)
         else if (s == "--candidates") { // extension: k nearest candidates of --mode neighbor, 1..32
             const std::string v = next("--candidates");
             char *end = nullptr;
@@ -259,6 +259,7 @@ int run_solvers()
     std::printf("  2opt --mode neighbor_multi   candidate-list 2-opt, many disjoint moves per step, --candidates K (extension)\n");
     std::printf("  or_opt | or-opt              Or-opt, bit-exact with or_opt.rs\n");
     std::printf("  or_opt --mode neighbor       candidate-list best-improvement Or-opt, --candidates K (extension)\n");
+    std::printf("  or_opt --mode neighbor_multi candidate-list Or-opt, many disjoint moves per step, --candidates K (extension)\n");
     std::printf("  3opt | three_opt             best-improvement 3-opt, bit-exact with three_opt.rs\n");
     std::printf("  3opt --mode neighbor         candidate-list best-improvement 3-opt, --candidates K (extension)\n");
     std::printf("presets: fast (nn,2opt)\n");

@@ -461,7 +461,8 @@ Solution run_local_search(const TspProblem &problem, int algo, int path, const P
     // 10^6 cities), and the per-move progress values of two_opt.rs and or_opt.rs need it: only the start
     // and the result are sent
     const bool replay = tx && algo != TL_ALGO_TWO_OPT_NEIGHBOR && algo != TL_ALGO_OR_OPT_NEIGHBOR &&
-                        algo != TL_ALGO_THREE_OPT_NEIGHBOR && algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI;
+                        algo != TL_ALGO_THREE_OPT_NEIGHBOR && algo != TL_ALGO_TWO_OPT_NEIGHBOR_MULTI &&
+                        algo != TL_ALGO_OR_OPT_NEIGHBOR_MULTI;
     std::vector<tl_move> log(replay ? (size_t)1 << 20 : 0);
     tl_stats st{};
     std::vector<uint32_t> before = tour;
@@ -551,10 +552,12 @@ namespace or_opt {
 Solution solve_with(const TspProblem &problem, const std::string &mode, const ProgressSender *progress_tx,
                     const std::vector<size_t> *init_tour, uint32_t candidates)
 {
-    const int algo = mode == "neighbor" ? TL_ALGO_OR_OPT_NEIGHBOR : TL_ALGO_OR_OPT;
+    const int algo = mode == "neighbor"         ? TL_ALGO_OR_OPT_NEIGHBOR
+                     : mode == "neighbor_multi" ? TL_ALGO_OR_OPT_NEIGHBOR_MULTI
+                                                : TL_ALGO_OR_OPT;
     // n < 4: identity order, seed ignored, no progress messages (or_opt.rs:31-34)
     if (problem.cities.size() < 4) return Solution::from_parts(ids_of(problem.cities), problem.cities, problem.distances);
-    if (algo == TL_ALGO_OR_OPT_NEIGHBOR && candidates)
+    if (algo != TL_ALGO_OR_OPT && candidates)
         check(tl_problem_set_candidates(problem.distances.impl->prob, candidates), "or_opt");
     const std::vector<size_t> start = init_tour ? *init_tour : ids_of(problem.cities);
     return run_local_search(problem, algo, TL_PATH_AUTO, progress_tx, start, "or_opt");
@@ -734,8 +737,8 @@ Result<Solution> solve_with_context(Solvers solver, const TspProblem &problem, c
     case Solvers::NearestNeighbor: return Result<Solution>::ok(nearest_neighbor::solve(problem, h, tx, init_tour));
     case Solvers::GreedyEdge: return Result<Solution>::ok(greedy_edge::solve(problem, opts, tx, init_tour));
     case Solvers::OrOpt:
-        if (opts.cuda_mode == "neighbor")
-            return Result<Solution>::ok(or_opt::solve_with(problem, "neighbor", tx, init_tour, opts.cuda_candidates));
+        if (opts.cuda_mode == "neighbor" || opts.cuda_mode == "neighbor_multi")
+            return Result<Solution>::ok(or_opt::solve_with(problem, opts.cuda_mode, tx, init_tour, opts.cuda_candidates));
         return Result<Solution>::ok(or_opt::solve(problem, h, tx, init_tour));
     case Solvers::ThreeOpt:
         if (opts.cuda_mode == "neighbor")

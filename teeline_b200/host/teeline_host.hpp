@@ -210,7 +210,7 @@ struct AppOptions { // mod.rs:1586-1596; only the sub-tables this path consumes 
     std::optional<AcoOptions> aco;
     std::optional<GAOptions> ga;
     // extension table [stage.cuda] (never required): mode = "ref"|"best"|"best_cyclic"|"neighbor"|"neighbor_multi"
-    // (or_opt, 3opt: "neighbor"), path = "auto"|"matrix"|"recompute",
+    // (or_opt: "neighbor"|"neighbor_multi", 3opt: "neighbor"), path = "auto"|"matrix"|"recompute",
     // seed = <integer> (the population solvers' Philox key; the reference's RNG is unseeded),
     // candidates = <integer> (modes "neighbor" and "neighbor_multi": k of the candidate lists, 1..32;
     // 0 = TL_CANDIDATES_DEFAULT)
@@ -232,8 +232,8 @@ Solution solve_with(const TspProblem &problem, const std::string &mode, const st
 namespace or_opt {
 Solution solve(const TspProblem &problem, const HeuristicOptions &opts, const ProgressSender *progress_tx,
                const std::vector<size_t> *init_tour);
-// extension: mode "neighbor" runs candidate-list Or-opt with k = candidates (0 = the library's default);
-// any other mode runs solve()'s Or-opt
+// extension: mode "neighbor" runs candidate-list Or-opt and mode "neighbor_multi" its multi-move form, with
+// k = candidates (0 = the library's default); any other mode runs solve()'s Or-opt
 Solution solve_with(const TspProblem &problem, const std::string &mode, const ProgressSender *progress_tx,
                     const std::vector<size_t> *init_tour, uint32_t candidates = 0);
 }
